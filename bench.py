@@ -76,7 +76,14 @@ def parse_args():
     ap.add_argument("--gp-n", type=int, default=8192, help="GP training-set size (BASELINE configs[3]: n = 8192)")
     ap.add_argument("--graph", action="store_true", help="replay each micro-batch forward as a CUDA graph")
     ap.add_argument("--profile-json", default=None, help="write the per-op CUDA-event profile of one micro-batch here")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the score table of the last timed step as DIR/<name>.npy (float32)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the GPU path computed: it needs --impl ours")
+    return args
 
 
 NCU_CAPTURES = ("r02_ncu_all_launches_one_forward.csv", "r01_ncu_all_launches_one_forward_v6_mb256.csv")
@@ -275,6 +282,25 @@ def run_reference(args):
 
 
 # ---- our arm ---------------------------------------------------------------------------------------------
+DUMP_MAX_ROWS = 1 << 21      # 16 bytes per row with the row index: 32 MiB, under the 64 MB a dump may take
+
+
+def dump_outputs(out_dir, table, np):
+    """The [N, 2] score table of a step as PerturbationEngine.score_masks hands it out: target_prob.npy and top1.npy,
+    float32, one entry per mask in job order.  Inputs are seeded, so two builds can be compared file for file.  A table
+    of more than DUMP_MAX_ROWS masks is written as a fixed seeded sample of its rows, with their indices in row.npy
+    (float64)."""
+    t = table.float().cpu().numpy()
+    arrays = {"target_prob": t[:, 0].copy(), "top1": t[:, 1].copy()}
+    if t.shape[0] > DUMP_MAX_ROWS:
+        rows = np.sort(np.random.default_rng(0).choice(t.shape[0], DUMP_MAX_ROWS, replace=False))
+        arrays = {k: v[rows] for k, v in arrays.items()}
+        arrays["row"] = rows.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
 def run_ours(args):
     import numpy as np
     import torch
@@ -392,8 +418,15 @@ def run_ours(args):
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
-    ms = timed(lambda: device_step(bits_dev), args.steps)
+    last = [None]
+
+    def timed_step():
+        last[0] = device_step(bits_dev)
+
+    ms = timed(timed_step, args.steps)
     clocks = sampler.stop() if rank == 0 else None
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, last[0], np)     # before the e2e steps below overwrite the table
     l1, t1 = all_launches()
     ties1 = eng.tie_stats()
     # + per score_local call: score kernel (+ compact, fp32 score, scatter with the tie policy); + one all-gather per step

@@ -1,7 +1,7 @@
-"""Generates tests/golden/*.npz by EXECUTING THE REFERENCE'S OWN CODE in the build container.
+"""Generates tests/golden/*.npz by EXECUTING THE REFERENCE'S OWN CODE from a checkout of it.
 
-Run once here (`python tests/golden/make_golden.py`); /root/reference does not exist on the GPU box, so the
-tests only ever read the committed .npz files.  Nothing from the reference is copied into the repo: the hot
+Run once with that checkout (`python tests/golden/make_golden.py <reference checkout>`); the tests only ever read
+the committed .npz files.  Nothing from the reference is copied into the repo: the hot
 loops cannot be imported on Python 3.12 (`async=True` SyntaxError, argparse/downloads at import time), so the
 loop-body statements are located in the reference files by content, dedented and exec'd in a namespace that
 supplies the loop's free variables (`segments`, `org_img`, `input`, ...) — i.e. the fixtures are outputs of
@@ -30,7 +30,7 @@ import sys
 import numpy as np
 import torch
 
-REF = "/root/reference"
+REF = None   # the reference checkout, from the command line
 OUT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.dirname(os.path.dirname(OUT)))
 
@@ -308,8 +308,9 @@ def make_localize():
 
 
 if __name__ == "__main__":
-    if not os.path.isdir(REF):
-        raise SystemExit("the reference tree is only present in the build container")
+    if len(sys.argv) != 2 or not os.path.isdir(sys.argv[1]):
+        raise SystemExit("usage: python tests/golden/make_golden.py <checkout of LiliMeng/network_interpretation_imagenet>")
+    REF = os.path.abspath(sys.argv[1])
     make_masks_imagenet()
     make_masks_cifar()
     make_masks_mnist()

@@ -39,3 +39,10 @@ def test_committed_gpu_line_has_every_contract_key():
     cb = d["cpu_baseline"]
     assert cb["kind"] in ("port", "reference") and cb["cores"] >= 1 and cb["value"] > 0
     assert "workload" in d["config"] and "model" not in d["config"]
+
+
+def test_rejects_no_timed_steps_and_dumps_without_the_gpu_path():
+    for extra in (["--steps", "0"], ["--warmup", "-1"], ["--impl", "reference", "--dump-outputs", "out"]):
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *extra], capture_output=True, text=True,
+                           timeout=120, cwd=ROOT)
+        assert r.returncode == 2 and "error:" in r.stderr, (extra, r.stderr[-800:])

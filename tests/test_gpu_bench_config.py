@@ -9,6 +9,11 @@ Tolerances (north_star): logits within 1e-2 relative in bf16, stated here elemen
 |a - b| <= 1e-2 * max_k |b[n, k]| for every element of every row (stricter than one max-norm over the batch); identical
 top-1 on EVERY mask; target-class probability within the bound the logit tolerance implies,
 |d ln p| <= 2 * 1e-2 * max|logit|  (p = exp(l_t - lse(l)); both terms move by at most the logit error)."""
+import json
+import os
+import subprocess
+import sys
+
 import numpy as np
 import pytest
 import torch
@@ -19,6 +24,7 @@ from oracle import scoring as oscore
 from oracle import synthetic
 
 pytestmark = pytest.mark.gpu
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 TOL_BF16 = 1e-2
 N_MASKS = 768
@@ -137,3 +143,24 @@ def test_tie_policy_is_device_side_and_bounded(bench_setup):
     out0 = eng0.score_masks(bits)
     assert eng0.tie_stats()["near_ties"] == 0
     assert torch.equal(out0["target_prob"], s16["target_prob"]) and torch.equal(out0["top1"], s16["top1"])
+
+
+def test_bench_dump_outputs_are_the_scores_of_the_last_timed_step(nib, tmp_path):
+    """bench.py --dump-outputs writes the score table its timed path produced: the scores the engine gives for the same
+    seeded job (the first N masks of seed 1, the seeded ResNet-101, micro-batch and stream copies as passed)."""
+    n, mb = 96, 48
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "2", "--warmup", "1", "--masks-per-step",
+                        str(n), "--micro-batch", str(mb), "--no-cpu-baseline", "--no-library-bar", "--no-gp",
+                        "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=900, cwd=ROOT)
+    assert r.returncode == 0, r.stderr[-3000:]
+    line = json.loads([l for l in r.stdout.splitlines() if l.startswith("{")][-1])
+    assert line["steps"] == 2 and line["config"]["masks_per_step_total"] == n
+    assert sorted(os.listdir(tmp_path)) == ["target_prob.npy", "top1.npy"]
+    prob, top1 = np.load(tmp_path / "target_prob.npy"), np.load(tmp_path / "top1.npy")
+    assert prob.dtype == top1.dtype == np.float32 and prob.shape == top1.shape == (n,)
+    eng = nib.PerturbationEngine(ocls.build_imagenet_model("resnet101"), synthetic.synthetic_image("imagenet"),
+                                 synthetic.voronoi_labels(224, 224, 50), target=0, mode=nib.KEEP_MUL, precision="bf16",
+                                 max_batch=mb, S=50, streams=STREAMS)
+    out = eng.score_masks(nib.selection_bits(nib.draw_selections("subset_keep", 50, n, seed=1), 50))
+    assert np.array_equal(top1, out["top1"].cpu().numpy().astype(np.float32))
+    np.testing.assert_allclose(prob, out["target_prob"].cpu().numpy(), rtol=1e-5, atol=0)
