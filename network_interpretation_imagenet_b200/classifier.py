@@ -13,6 +13,7 @@ Recognised structures (by attributes, not class identity, so the reference's own
   * models/resnet.py ResNetCifar (BasicBlockWithDeathRate + DownsampleB, eval path :26-42, :71-76)
   * mnist Classification_Net (conv1..conv6 + fc1, returns (x0, x1, x2, pred0), mnist :97-105)
   * torchvision DenseNet and the CIFAR DenseNet(-BC) of models/densenet.py:44-99
+  * torchvision VGG (vgg11/13/16/19, with or without BN) and AlexNet: `features / avgpool / classifier`
 """
 from __future__ import annotations
 
@@ -165,9 +166,12 @@ class Classifier:
         m = module.module if isinstance(module, nn.DataParallel) else module  # cifar :75 wraps in DataParallel
         if hasattr(m, "layer4") and hasattr(m, "fc") and hasattr(m, "maxpool"):
             return _lower_tv_resnet(m, input_hw or (224, 224), prec, precision, max_batch)
+        if _is_plain_cnn(m):
+            return _lower_tv_plain(m, input_hw or (224, 224), prec, precision, max_batch)
         if precision == "split":
             raise TypeError("precision 'split' (split-bf16 tensors on the tcgen05 pair kernel) is lowered for torchvision "
-                            "ResNets only (every body conv needs Cin % 64 == 0 and Cout % 64 == 0); use 'x3' for this network")
+                            "ResNets, VGGs and AlexNet only (every body conv needs Cin % 64 == 0 and Cout % 64 == 0); use "
+                            "'x3' for this network")
         if hasattr(m, "layer3") and hasattr(m, "fc") and not hasattr(m, "layer4"):
             return _lower_resnet_cifar(m, input_hw or (32, 32), prec, precision, max_batch)
         if hasattr(m, "conv6") and hasattr(m, "fc1"):
@@ -542,3 +546,165 @@ def _lower_densenet_cifar(m, hw, prec, precision, max_batch):
             b.pool(_lib.POOL_AVG, buf, Ctot, feat, 8, 8, 0, pre=bn_affine(m.norm5))
             b.fc(feat, Ctot, m.classifier.out_features, m.classifier.weight, m.classifier.bias)
     return Classifier(b, x_in, (3, H, W), m.classifier.out_features, precision, max_batch, arch="densenet_cifar")
+
+
+# ---- torchvision VGG / AlexNet: features (conv [BN] ReLU, max pool) / avgpool / classifier (Linear ReLU Dropout) ----------
+def _is_plain_cnn(m) -> bool:
+    return (isinstance(getattr(m, "features", None), nn.Sequential) and isinstance(getattr(m, "classifier", None), nn.Sequential)
+            and not hasattr(m.features, "denseblock1"))
+
+
+def _pair(v):
+    return tuple(v) if isinstance(v, (tuple, list)) else (v, v)
+
+
+def _plain_cnn_layers(m, hw, precision):
+    """Checks the whole module and returns (feature ops, (C, H, W) of the final map, [(Linear, relu)]) without touching the
+    library: feature ops are ("conv", Conv2d, BatchNorm2d | None, relu) and ("pool", k, stride, pad).  TypeError names a
+    module this lowering does not take, ValueError an input size it cannot serve."""
+    H, W = hw
+    C = None
+    ops = []
+    mods = list(m.features.children())
+    i = 0
+    while i < len(mods):
+        mod = mods[i]
+        if isinstance(mod, nn.Conv2d):
+            k, s, p, d = _pair(mod.kernel_size), _pair(mod.stride), _pair(mod.padding), _pair(mod.dilation)
+            if (mod.groups != 1 or d != (1, 1) or k[0] != k[1] or s[0] != s[1] or isinstance(mod.padding, str) or p[0] != p[1]
+                    or mod.padding_mode != "zeros"):
+                raise TypeError(f"unsupported Conv2d in features[{i}]: {mod} (needs groups 1, dilation 1, square kernel, "
+                                "stride and zero padding)")
+            if C is not None and mod.in_channels != C:
+                raise TypeError(f"features[{i}]: {mod} takes {mod.in_channels} channels, the map has {C}")
+            bn = None
+            if i + 1 < len(mods) and isinstance(mods[i + 1], nn.BatchNorm2d):
+                bn = mods[i + 1]
+                i += 1
+            relu = i + 1 < len(mods) and isinstance(mods[i + 1], nn.ReLU)
+            if relu:
+                i += 1
+            H, W = _out_hw(H, k[0], s[0], p[0]), _out_hw(W, k[0], s[0], p[0])
+            if H < 1 or W < 1:
+                raise ValueError(f"input {hw} is too small for features[{i}]")
+            C = mod.out_channels
+            ops.append(("conv", mod, bn, relu))
+        elif isinstance(mod, nn.MaxPool2d):
+            k, s, p, d = _pair(mod.kernel_size), _pair(mod.stride), _pair(mod.padding), _pair(mod.dilation)
+            if k[0] != k[1] or s[0] != s[1] or p[0] != p[1] or d != (1, 1) or mod.ceil_mode or mod.return_indices:
+                raise TypeError(f"unsupported MaxPool2d in features[{i}]: {mod} (needs a square window, dilation 1, "
+                                "ceil_mode=False)")
+            if C is None:
+                raise TypeError("features must start with a Conv2d")
+            H, W = _out_hw(H, k[0], s[0], p[0]), _out_hw(W, k[0], s[0], p[0])
+            if H < 1 or W < 1:
+                raise ValueError(f"input {hw} is too small for features[{i}]")
+            ops.append(("pool", k[0], s[0], p[0]))
+        else:
+            raise TypeError(f"unsupported module in features[{i}]: {type(mod).__name__}")
+        i += 1
+    if C is None:
+        raise TypeError("features holds no Conv2d")
+    ap = getattr(m, "avgpool", None)
+    if ap is not None and not isinstance(ap, nn.Identity):
+        if not isinstance(ap, nn.AdaptiveAvgPool2d):
+            raise TypeError(f"unsupported avgpool: {type(ap).__name__}")
+        oh, ow = _pair(ap.output_size)
+        if (oh is not None and oh != H) or (ow is not None and ow != W):
+            # only the identity case is lowered (every 224^2 drop-in); a general adaptive pool is not
+            raise ValueError(f"input {hw} gives a {H}x{W} feature map; avgpool wants {ap.output_size} and is lowered "
+                             "only where it is an identity")
+    lins = []
+    for j, mod in enumerate(m.classifier.children()):
+        if isinstance(mod, nn.Linear):
+            lins.append([mod, False])
+        elif isinstance(mod, nn.ReLU):
+            if not lins or lins[-1][1]:
+                raise TypeError(f"classifier[{j}]: a ReLU must follow a Linear")
+            lins[-1][1] = True
+        elif not isinstance(mod, nn.Dropout):     # Dropout: identity in eval
+            raise TypeError(f"unsupported module in classifier[{j}]: {type(mod).__name__}")
+    if len(lins) < 2 or lins[-1][1]:
+        raise TypeError("classifier must hold at least two Linear layers and end in a Linear without ReLU")
+    if H != W:
+        raise ValueError(f"input {hw} gives a non-square {H}x{W} feature map")
+    if lins[0][0].in_features != C * H * W:
+        raise ValueError(f"input {hw} gives {C}x{H}x{W} features; classifier[0] takes {lins[0][0].in_features}")
+    for a, b in zip(lins, lins[1:]):
+        if b[0].in_features != a[0].out_features:
+            raise TypeError(f"{b[0]} does not take the {a[0].out_features} outputs of {a[0]}")
+    if precision == "split":
+        body = [op[1] for op in ops[1:] if op[0] == "conv"]
+        widths = [(c.in_channels, c.out_channels) for c in body] + [(C, lins[0][0].out_features)]
+        widths += [(l.in_features, l.out_features) for l, _ in lins[1:-1]]
+        if any(a % 64 or b % 64 for a, b in widths):
+            raise TypeError("precision 'split' needs Cin % 64 == 0 and Cout % 64 == 0 for every conv after the first and "
+                            "every Linear but the last; use 'x3' for this network")
+    return ops, (C, H, W), [(l, r) for l, r in lins]
+
+
+# Longest reduction an fp32-grade lowering puts on split-bf16 tensor-core products (net.cu NIB_X3_MAX_K): the tensor cores'
+# fp32 accumulation drifts with K, so split networks run VGG's fc6 (K = 25088) on fp32 buffers on the CUDA cores.
+_FP32_GRADE_TC_MAX_K = 16384
+
+
+def _lower_tv_plain(m, hw, prec, precision, max_batch):
+    """Convs (BN folded) and max pools as they come; the first Linear as a valid KxK conv over the KxK final map (its
+    weight viewed [out][C][K][K]: nib_net_add_conv's KRSC repack then matches the NHWC order of the map, so no flatten op
+    is needed), the middle Linears as 1x1 convs on 1x1 maps, the last Linear as the fc op.  bf16: a 3x3/1 first conv
+    reads 8-channel pixels in a 1-pixel zero halo (the tcgen05 raw-row mode, conv_tc.cu tc_conv_is_raw3x3).  split: the
+    first conv, the pools and a Linear longer than _FP32_GRADE_TC_MAX_K run on fp32 buffers, everything else on split-bf16
+    tensors, with converts between."""
+    ops, (C, Hf, Wf), lins = _plain_cnn_layers(m, hw, precision)   # everything is checked before the library is touched
+    H, W = hw
+    b = _Builder(prec, max_batch)
+    split = precision == "split"
+    c1 = ops[0][1]
+    cin = c1.in_channels
+    raw3 = (precision == "bf16" and _pair(c1.kernel_size) == (3, 3) and _pair(c1.stride) == (1, 1)
+            and _pair(c1.padding) == (1, 1) and cin <= 8)
+    x_in = b.buffer(H, W, 8, pad=1, pooled=False) if raw3 else b.buffer(H, W, _in_cpad(cin), pooled=False, f32=split)
+    x, Cx, Hx, Wx, x_split = x_in, cin, H, W, False
+
+    def to_split(want):
+        nonlocal x, x_split
+        if split and want != x_split:
+            y = b.buffer(Hx, Wx, Cx, f32=not want)
+            b.convert(x, y)
+            b.release(x)
+            x, x_split = y, want
+
+    for op in ops:
+        if op[0] == "conv":
+            _, cv, bn, relu = op
+            if x != x_in:
+                to_split(True)
+            k, s, p = cv.kernel_size[0], _pair(cv.stride)[0], _pair(cv.padding)[0]
+            Ho, Wo = _out_hw(Hx, k, s, p), _out_hw(Wx, k, s, p)
+            o = b.buffer(Ho, Wo, cv.out_channels, f32=split and not x_split)
+            w, bias = fold_bn(cv.weight, cv.bias, bn)
+            b.conv(x, Cx, o, cv.out_channels, w, bias, k, s, p, relu=relu)
+            if x != x_in:
+                b.release(x)
+            x, Cx, Hx, Wx = o, cv.out_channels, Ho, Wo
+        else:
+            _, k, s, p = op
+            to_split(False)
+            Ho, Wo = _out_hw(Hx, k, s, p), _out_hw(Wx, k, s, p)
+            o = b.buffer(Ho, Wo, Cx, f32=split)
+            b.pool(_lib.POOL_MAX, x, Cx, o, k, s, p)
+            b.release(x)
+            x, Hx, Wx = o, Ho, Wo
+    for j, (lin, relu) in enumerate(lins[:-1]):
+        K = Hx if j == 0 else 1
+        tc = Cx * K * K <= _FP32_GRADE_TC_MAX_K
+        to_split(tc)
+        wc = lin.weight.detach().reshape(lin.out_features, Cx, K, K)
+        o = b.buffer(1, 1, lin.out_features, f32=split and not tc)
+        b.conv(x, Cx, o, lin.out_features, wc, lin.bias, K, 1, 0, relu=relu)
+        b.release(x)
+        x, Cx, Hx, Wx = o, lin.out_features, 1, 1
+    to_split(False)
+    last = lins[-1][0]
+    b.fc(x, Cx, last.out_features, last.weight, last.bias)
+    return Classifier(b, x_in, (cin, H, W), last.out_features, precision, max_batch, arch="tv_plain")

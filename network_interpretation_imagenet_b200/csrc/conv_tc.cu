@@ -15,7 +15,8 @@
 //     tile (whole image rows in the raster of the padded width); tap (dy, dx) is the same swizzled operand started
 //     (dy * Wp + dx) rows further on (descriptor base offset 0: the swizzle phase is address-based);
 //   * mode 5: the 7x7 stride-2 stem reads the raw padded input rows through an UNSWIZZLED descriptor whose rows
-//     overlap (row pitch 16 B = the stride-2 window over 8-byte pixels);
+//     overlap (row pitch 16 B = the stride-2 window over 8-byte pixels); a 3x3 stride-1 first conv on 16-byte pixels
+//     (VGG's conv1_1) reads its three rows the same way (row pitch 16 B = one pixel);
 //   * pre-activation 1x1 convs (DenseNet): four extra warps apply relu(x * scale + shift) to every A tile in shared
 //     memory between its TMA completion and the MMA, instead of a separate pack pass.
 //
@@ -88,6 +89,11 @@ struct TcKernelParams {
   const float* xf_scale;
   const float* xf_shift;
   int halo_swap;                   // im2col == 5 diagnostics: swap the LBO / SBO roles of the unswizzled descriptor
+  // im2col == 5 (raw input rows): filter rows per tile (7: the 7x7/2 stem, 3: a 3x3/1 first conv) and column tiles per
+  // output row (1 unless the row is wider than the 128-row M tile).  Pair tile mp holds output rows 2 (mp / col_tiles) and
+  // 2 (mp / col_tiles) + 1 (one per CTA) in the SAME column tile mp % col_tiles, so both CTAs' A operands start at the same
+  // shared-memory offset: the leader's descriptor addresses both.
+  int raw_rows, col_tiles;
 };
 
 // ---- PTX wrappers -------------------------------------------------------------------------------
@@ -688,6 +694,13 @@ conv_tc3_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
     asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tmem_slot), "r"(TMEM_COLS) : "memory");
     asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
   }
+  if (p.im2col == 5 && p.stride == 1) {
+    // 3x3 raw rows: the last output pixel's zero-weight filler tap reads the 16 bytes just past the third row, which no
+    // TMA load ever writes.  Zero the ring once so that 0 * (whatever the SM held before) cannot inject a NaN.
+    for (uint32_t off = 16u * threadIdx.x; off < (uint32_t)(STAGES * SM::STAGE_BYTES); off += 16u * blockDim.x)
+      sts_v4(smem_base + off, make_uint4(0u, 0u, 0u, 0u));
+    fence_async_smem();
+  }
   tc_fence_before();
   __syncthreads();
   cluster_sync_all();   // the peer's barriers exist before anything arrives on them
@@ -755,8 +768,9 @@ conv_tc3_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
     for (int tile = pair; tile < total_tiles; tile += npairs, ++it) {
       const int n_tile = tile % p.n_tiles;
       const int mp = tile / p.n_tiles;
-      const int m_tile = mp * 2 + (int)rank;
-      const int m0 = m_tile * p.tile_rows;
+      // raw rows: m_tile is the output row (image-major); the tile covers column tile mp % col_tiles of it
+      const int m_tile = p.im2col == 5 ? (mp / p.col_tiles) * 2 + (int)rank : mp * 2 + (int)rank;
+      const int m0 = p.im2col == 5 ? (m_tile * p.col_tiles + mp % p.col_tiles) * p.tile_rows : m_tile * p.tile_rows;
       const int n0 = n_tile * BLOCK_N;
       int w0 = 0, h0 = 0, img = 0;
       if (p.im2col == 1) {
@@ -788,7 +802,7 @@ conv_tc3_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
         continue;
       }
       if (BRES && !HAS_RES && p.im2col == 5) {
-        // stem: the seven padded input rows under one output row, raw (7 x row bytes), one ring stage per tile
+        // the padded input rows under one output row (7 for the stem, 3 for a 3x3 conv), raw, one ring stage per tile
         TC3_TIMED(0, mbar_wait(empty_bar(stage), phase ^ 1u, p.err_flag, 1));
         if (elect_one()) {
           if (rank == 0) mbar_arrive_expect_tx(full_bar(stage), (uint32_t)(2 * p.a_bytes));
@@ -895,13 +909,17 @@ conv_tc3_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
           // pixel 2q of input row 2p + r, i.e. 16 q bytes into that row - an unswizzled K-major operand whose rows
           // OVERLAP (row pitch 16 B, K chunk pitch 16 B).  Each input byte crosses L2 -> SM once per output row instead
           // of once per tap: 12.9 KB per tile instead of 56 KB of 64-byte rows.
+          // The 3x3 stride-1 form is the same operand over 16-byte pixels: 3 taps x 8 channels + one filler tap per filter
+          // row, row pitch 16 B = one pixel; column tile c starts 16 (c * tile_rows) bytes into the rows (both CTAs of the
+          // pair are in the same column tile).
           TC3_TIMED(0, mbar_wait(full_bar(stage), phase, p.err_flag, 2));
           tc_fence_after();
           if (elect_one()) {
-            const uint32_t a_addr = smem_base + stage * SM::STAGE_BYTES;
+            const int q0 = ((tile / p.n_tiles) % p.col_tiles) * p.tile_rows;
+            const uint32_t a_addr = smem_base + stage * SM::STAGE_BYTES + 16u * (uint32_t)q0;
             const uint32_t lbo = p.halo_swap ? 128u : 16u, sbo = p.halo_swap ? 16u : 128u;
 #pragma unroll 1
-            for (int r = 0; r < 7; ++r) {
+            for (int r = 0; r < p.raw_rows; ++r) {
               const uint32_t b_addr = smem_base + SM::BRES_OFFSET + (r >> 1) * SM::BH_BYTES + (r & 1) * (SM::BH_BYTES / 2);
 #pragma unroll
               for (int ks = 0; ks < 2; ++ks) {
@@ -1041,8 +1059,8 @@ conv_tc3_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
     for (; tile < total_tiles; tile += step, it += (SM::SPLIT_COLS ? 1 : 2), ++lt) {
       const int n_tile = tile % p.n_tiles;
       const int mp = tile / p.n_tiles;
-      const int m_tile = mp * 2 + (int)rank;
-      const int m0 = m_tile * p.tile_rows;
+      const int m_tile = p.im2col == 5 ? (mp / p.col_tiles) * 2 + (int)rank : mp * 2 + (int)rank;
+      const int m0 = p.im2col == 5 ? (m_tile * p.col_tiles + mp % p.col_tiles) * p.tile_rows : m_tile * p.tile_rows;
       const int n0 = n_tile * BLOCK_N;
       const int ab = it & 1;
       TC3_TIMED(0, mbar_wait(tmem_full_bar(ab), (uint32_t)((it >> 1) & 1), p.err_flag, 3));
@@ -1675,6 +1693,7 @@ struct TcConvPlan {
   int tile_rows;
   int num_k_blocks, cblocks;
   int halo_wp, halo_r, halo_tpi, halo_cb, halo_n;   // im2col == 4
+  int raw_rows, col_tiles;                          // im2col == 5
   unsigned int* err_flag;
 };
 
@@ -1722,6 +1741,45 @@ bool tc_conv_is_stem4(const ConvParams& p) {
          (p.Hin + 2 * p.in_halo) >= 2 * (p.P - 1) + 8;
 }
 
+// Raw-row TMA box of a padded row of row_el elements: {inner, row_el / inner} with a legal inner extent (a multiple of 8
+// elements = 16 B, at most 256, dividing the row, at most 256 chunks); 0 if there is none.
+static int raw_row_inner(int row_el) {
+  for (int c = 256; c >= 8; c -= 8)
+    if (row_el % c == 0 && row_el / c <= 256) return c;
+  return 0;
+}
+
+// 3x3 raw rows: column tiles per output row.  One tile when the row fits the 128-row M tile; otherwise the smallest
+// split into equal tiles of at most 128 columns, provided a tile keeps at least half of the MMA's rows busy.  0: no split.
+static int raw3x3_col_tiles(int Q) {
+  if (Q <= TC_BLOCK_M) return 1;
+  for (int t = 2; Q / t >= TC_BLOCK_M / 2; ++t)
+    if (Q % t == 0 && Q / t <= TC_BLOCK_M) return t;
+  return 0;
+}
+
+// 3x3 stride-1 pad-1 first conv (VGG conv1_1) on 8-channel-padded pixels (16 B) inside a 1-pixel zero halo, im2col mode 5:
+// output pixel q of filter row r reads 3 taps x 8 channels starting at pixel q of padded row p + r, so each filter row is
+// one 32-element K atom (3 taps + a zero-weight filler tap) of the overlapping-row operand the stem uses; K = 3 x 32, six
+// MMAs per tile.  Weights [Cout][4][32] (row 3 zero), resident; Cout 64 or 128 (the resident-weight pair kernel holds one
+// N tile).  The three rows of one image row (plus the filler's 16 B) must fit one 16 KB ring stage.
+bool tc_conv_is_raw3x3(const ConvParams& p) {
+  static const bool off = getenv("NIB_TC_NO_HALO") != nullptr;
+  if (off || p.split) return false;
+  if (!(p.R == 3 && p.S == 3 && p.stride == 1 && p.pad == 1 && p.Cin <= 8 && p.in_cstride == 8 && p.in_coff == 0 &&
+        p.in_halo == 1))
+    return false;
+  if (!(p.Cout == 64 || p.Cout == 128) || p.out_halo != 0 || p.out_cstride % 8 != 0 || p.out_coff % 8 != 0) return false;
+  if (p.pre_scale != nullptr || p.res != nullptr || p.w_alt == nullptr || p.P != p.Hin || p.Q != p.Win) return false;
+  const int t = raw3x3_col_tiles(p.Q);
+  if (t == 0) return false;
+  const int Wp = p.Win + 2, row_bytes = Wp * 16;
+  if (3 * row_bytes + 16 > TC_BLOCK_M * TC_BLOCK_K * 2) return false;
+  // the last MMA row of the last column tile reads 2 rows + 127 pixels + 64 B past the tile's first pixel
+  if (2 * row_bytes + 16 * (p.Q - p.Q / t + TC_BLOCK_M - 1) + 64 > TC_BLOCK_M * TC_BLOCK_K * 2) return false;
+  return raw_row_inner(Wp * 8) > 0;
+}
+
 // 3x3 stride-1 pad-1 convolution, 64 -> 64 channels, on the CTA-pair kernel with resident weights: the im2col path reads
 // every input pixel nine times from L2 (16 KB per K block per SM against a ~43 B/clk/SM L2 port: 385 cycles per K block
 // for 128 cycles of MMA), this one loads each tile's input patch once.  Whole image rows per tile, in the raster of the
@@ -1758,7 +1816,7 @@ bool tc_conv_supported(const ConvParams& p) {
       return false;
     return true;
   }
-  if (tc_conv_is_stem(p) || tc_conv_is_stem4(p)) return true;
+  if (tc_conv_is_stem(p) || tc_conv_is_stem4(p) || tc_conv_is_raw3x3(p)) return true;
   if (p.Cin % TC_BLOCK_K != 0) return false;
   if (p.in_cstride % 8 != 0 || p.in_coff % 8 != 0) return false;   // 16 B TMA alignment
   if (p.Cout % 32 != 0) return false;
@@ -1835,13 +1893,12 @@ int tc_conv_plan_create(const ConvParams& p, int max_batch, TcConvPlan** out) {
     int inner = 0;
     {
       static const bool off = getenv("NIB_TC_NO_HALO") != nullptr;
-      const int row_el = Wp * 4;
-      if (!off && 6 * Wp * 8 + 16 * 127 + 64 <= 16384)
-        for (int c = 256; c >= 8; c -= 8)
-          if (row_el % c == 0 && row_el / c <= 256) { inner = c; break; }
+      if (!off && 6 * Wp * 8 + 16 * 127 + 64 <= 16384) inner = raw_row_inner(Wp * 4);
     }
     if (inner > 0) {
       plan->im2col = 5;
+      plan->raw_rows = 7;
+      plan->col_tiles = 1;
       plan->halo_wp = Wp * 8;
       cuuint64_t dims[4] = {(cuuint64_t)inner, (cuuint64_t)(Wp * 4 / inner), (cuuint64_t)Hp, (cuuint64_t)max_batch};
       cuuint64_t strides[3] = {(cuuint64_t)inner * 2, (cuuint64_t)Wp * 8, (cuuint64_t)Hp * Wp * 8};
@@ -1883,6 +1940,52 @@ int tc_conv_plan_create(const ConvParams& p, int max_batch, TcConvPlan** out) {
                                  CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
       if (r != CUDA_SUCCESS) {
         set_error("cuTensorMapEncodeTiled (stem weights, 64B swizzle) failed (%d)", (int)r);
+        delete plan;
+        return NIB_ECUDA;
+      }
+    }
+    plan->tmB = plan->tmBh;
+    *out = plan;
+    return NIB_OK;
+  }
+  if (tc_conv_is_raw3x3(p)) {
+    const int Hp = p.Hin + 2, Wp = p.Win + 2, row_el = Wp * 8, inner = raw_row_inner(row_el);
+    plan->im2col = 5;
+    plan->raw_rows = 3;
+    plan->col_tiles = raw3x3_col_tiles(p.Q);
+    plan->cblocks = 1;
+    plan->num_k_blocks = 2;                 // resident weights: filter rows (0, 1) and (2, zero row)
+    plan->tile_rows = p.Q / plan->col_tiles;
+    plan->halo_wp = Wp * 16;
+    {
+      // three padded rows of one image as {inner, chunk, row, image}
+      cuuint64_t dims[4] = {(cuuint64_t)inner, (cuuint64_t)(row_el / inner), (cuuint64_t)Hp, (cuuint64_t)max_batch};
+      cuuint64_t strides[3] = {(cuuint64_t)inner * 2, (cuuint64_t)Wp * 16, (cuuint64_t)Hp * Wp * 16};
+      cuuint32_t box[4] = {(cuuint32_t)inner, (cuuint32_t)(row_el / inner), 3, 1};
+      cuuint32_t es[4] = {1, 1, 1, 1};
+      CUresult r = g_encodeTiled(&plan->tmA, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(p.in), dims, strides,
+                                 box, es, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
+                                 CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+      if (r != CUDA_SUCCESS) {
+        set_error("cuTensorMapEncodeTiled (3x3, raw rows) failed (%d)", (int)r);
+        delete plan;
+        return NIB_ECUDA;
+      }
+    }
+    rc = finish_plan(plan, p, max_batch, p.w_alt, 2 * 64);
+    if (rc != NIB_OK) { delete plan; return rc; }
+    if (!plan->v3) { set_error("tc_conv_plan_create: the 3x3 raw-row mode needs the CTA-pair kernel"); delete plan; return NIB_EINVAL; }
+    {
+      // weights [Cout][128] as 64B-swizzled K atoms of 32 elements, BLOCK_N/2 rows per CTA (overrides finish_plan's map)
+      cuuint64_t dims[2] = {128, (cuuint64_t)p.Cout};
+      cuuint64_t strides[1] = {128 * 2};
+      cuuint32_t box[2] = {32, (cuuint32_t)(plan->block_n / 2)};
+      cuuint32_t es[2] = {1, 1};
+      CUresult r = g_encodeTiled(&plan->tmBh, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(p.w_alt), dims, strides,
+                                 box, es, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B,
+                                 CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+      if (r != CUDA_SUCCESS) {
+        set_error("cuTensorMapEncodeTiled (3x3 raw-row weights, 64B swizzle) failed (%d)", (int)r);
         delete plan;
         return NIB_ECUDA;
       }
@@ -2221,6 +2324,7 @@ static int tc_dispatch(const TcConvPlan* plan, const TcKernelParams& kp, int til
     // CTA-pair kernel; stage counts fill the 227 KB of each SM (ring + output/residual boxes)
     const bool res = kp.res != nullptr;
     if (plan->im2col == 4) return launch_tc3<64, 9, false, true>(plan, kp, st);   // resident patch + resident weights
+    if (plan->im2col == 5 && plan->block_n == 128) return launch_tc3<128, 6, false, true>(plan, kp, st);   // raw rows, 128 out
     if (plan->block_n == 256) return res ? launch_tc3<256, 5, true>(plan, kp, st) : launch_tc3<256, 6, false>(plan, kp, st);
     if (plan->block_n == 128) return res ? launch_tc3<128, 6, true>(plan, kp, st) : launch_tc3<128, 8, false>(plan, kp, st);
     if (plan->block_n == 64 && !res && kp.n_tiles == 1 && kp.num_k_blocks <= TC3_BRES_KBLOCKS)
@@ -2340,7 +2444,12 @@ int tc_conv_launch(const TcConvPlan* plan, const ConvParams& p, cudaStream_t st)
     static const bool swap = getenv("NIB_TC_STEM_SWAP") != nullptr;
     kp.halo_wp = plan->halo_wp;          // bytes of one padded input row
     kp.halo_swap = swap ? 1 : 0;
-    kp.a_bytes = 7 * plan->halo_wp;
+    kp.raw_rows = plan->raw_rows;
+    kp.col_tiles = plan->col_tiles;
+    kp.a_bytes = plan->raw_rows * plan->halo_wp;
+    // pair tiles = output-row pairs x column tiles (an odd last row pairs with a row past the batch, as any odd tile count)
+    const int rows = p.M / p.Q;
+    kp.m_tiles = (rows + 1) / 2 * 2 * plan->col_tiles;
   }
   const int tiles = kp.m_tiles * kp.n_tiles;
   static const bool dbg = getenv("NIB_TC_DBG") != nullptr;

@@ -13,6 +13,9 @@
 
 using namespace nib;
 
+// longest reduction (R * S * Cin) an fp32-grade net puts on split-bf16 tensor-core products; classifier.py mirrors it
+static constexpr size_t NIB_X3_MAX_K = 16384;
+
 enum BufKind { BUF_F32 = 0, BUF_BF16 = 1, BUF_SPLIT = 2 };   // BUF_SPLIT: bf16 [hi(C) | lo(C)] per pixel, x = hi + lo
 
 struct NetBuffer {
@@ -262,7 +265,10 @@ int nib_net_add_conv(nib_net* net, const nib_conv_desc* d, const float* h_weight
   } else {
     NIB_CUDA(cudaMalloc(&op.d_w, nel * 4 + 256));
     NIB_CUDA(cudaMemcpy(op.d_w, krsc.data(), nel * 4, cudaMemcpyHostToDevice));
-    if (net->x3 && d->Cin % 16 == 0) {   // w = hi + lo with hi = bf16(w), lo = bf16(w - hi)
+    // w = hi + lo with hi = bf16(w), lo = bf16(w - hi).  Not for reductions longer than NIB_X3_MAX_K: the tensor cores'
+    // fp32 accumulation drifts with K (VGG's fc6, K = 25088, measured 1.6e-4 .. 1.9e-4 of the logits' scale against 1e-4
+    // for fp32 grade), so those run on the CUDA cores
+    if (net->x3 && d->Cin % 16 == 0 && K <= NIB_X3_MAX_K) {
       std::vector<uint16_t> hi(nel), lo(nel);
       for (size_t i = 0; i < nel; ++i) {
         hi[i] = f32_to_bf16_rn(krsc[i]);
@@ -297,6 +303,19 @@ int nib_net_add_conv(nib_net* net, const nib_conv_desc* d, const float* h_weight
           for (int c = 0; c < d->Cin; ++c)
             hb[(((size_t)co * 7 + r) * 8 + s) * 8 + c] =
                 f32_to_bf16_rn(h_weight[(((size_t)co * d->Cin + c) * 7 + r) * 7 + s]);
+    NIB_CUDA(cudaMalloc(&op.d_w_alt, hb.size() * 2 + 256));
+    NIB_CUDA(cudaMemcpy(op.d_w_alt, hb.data(), hb.size() * 2, cudaMemcpyHostToDevice));
+  }
+  if (net->bf16 && d->R == 3 && d->S == 3 && d->stride == 1 && d->pad == 1 && d->Cin <= 8 && bi.C == 8 && bi.pad == 1) {
+    // 3x3 first conv on raw input rows (conv_tc.cu tc_conv_is_raw3x3): filter row r = one 32-element K atom of
+    // 3 taps x 8 channels + a zero filler tap; row 3 is zero so the weights are two whole 64-element K blocks
+    std::vector<uint16_t> hb((size_t)d->Cout * 4 * 32, 0);
+    for (int co = 0; co < d->Cout; ++co)
+      for (int r = 0; r < 3; ++r)
+        for (int s = 0; s < 3; ++s)
+          for (int c = 0; c < d->Cin; ++c)
+            hb[((size_t)co * 4 + r) * 32 + s * 8 + c] =
+                f32_to_bf16_rn(h_weight[(((size_t)co * d->Cin + c) * 3 + r) * 3 + s]);
     NIB_CUDA(cudaMalloc(&op.d_w_alt, hb.size() * 2 + 256));
     NIB_CUDA(cudaMemcpy(op.d_w_alt, hb.data(), hb.size() * 2, cudaMemcpyHostToDevice));
   }

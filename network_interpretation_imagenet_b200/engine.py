@@ -34,6 +34,13 @@ from .scoring import score
 # literally (band 2e-2) would send 99.6 % of the masks of this near-tied random-init network to fp32.  Trained networks
 # have top-2 margins far outside any of these bands and the policy costs them one empty launch sequence (~0.6 ms).
 DEFAULT_TIE_BAND = 4.5e-3
+# Arch-keyed bands (Classifier.arch) where a network's flip study puts the numbers above DEFAULT_TIE_BAND.
+# torchvision VGG / AlexNet ("tv_plain"): flip study on the bench workload (tools/r02_diag2.py 16384 <arch>, bf16 at micro-batch
+# 384 x 2 streams against the fp32 lowering; profiles/vgg_flip_study_vgg16.json, profiles/vgg_flip_study_vgg16_bn.json): error
+# of (top1 - j) over the classes within 2e-2 of the top-1 <= 1.38e-2 (vgg16) / 1.15e-2 (vgg16_bn); 318 / 217 of 16384 arg-maxes
+# differ, at bf16 margins <= 7.4e-3 / 8.8e-3; row-wise logit error <= 1.35e-2 / 1.12e-2.  The band sits above the
+# near-class error and every flip margin; 17.8 % of vgg16's masks have a bf16 margin below 1.25e-2, 27.5 % below 2e-2.
+TIE_BANDS = {"tv_plain": 1.5e-2}
 DEFAULT_TIE_CAPACITY = 1024     # rows of the re-score buffer per window of masks
 DEFAULT_TIE_WINDOW = 4096       # masks scored per tie-policy pass (capacity = 25 % of a window: the seeded DenseNet-121,
                                 # the most tied of the networks here, has 13 % of its masks inside the band on average and
@@ -102,10 +109,10 @@ class ScoreComm:
 class PerturbationEngine:
     """refine_ties: relative top-2 margin (top1 - runner-up) / max|logit| below which a bf16-scored mask is re-scored by
     an fp32-grade copy of the classifier (`tie_precision`: "split" = the tcgen05 pair kernel over split-bf16 tensors,
-    torchvision ResNets only; "x3" = fp32 activations with split-bf16 mma.sync products; both within ~3e-5 of the fp32
+    torchvision ResNets, VGGs and AlexNet; "x3" = fp32 activations with split-bf16 mma.sync products; both within ~3e-5 of the fp32
     lowering; "fp32" = the CUDA-core lowering itself; "auto" picks "split" where it applies, else "x3"), so that top-1
     equals the reference's on every mask outside numerical noise.
-    "auto" (default) = DEFAULT_TIE_BAND for bf16 classifiers lowered from a torch module, off otherwise; None/0 = off.
+    "auto" (default) = TIE_BANDS[arch] (else DEFAULT_TIE_BAND) for bf16 classifiers lowered from a torch module, off otherwise; None/0 = off.
     The policy runs entirely on the device (no host synchronisation): near-tie rows are compacted into a buffer of
     `tie_capacity` rows (per window of `tie_window` masks), the fp32 network runs on that buffer with the device-side
     count as its live batch size, and the refined scores are scattered back.  `tie_stats()` reads the counters (near-ties
@@ -127,16 +134,17 @@ class PerturbationEngine:
         if isinstance(refine_ties, str):
             if refine_ties != "auto":
                 raise ValueError("refine_ties must be 'auto', None or a float")
-            refine_ties = DEFAULT_TIE_BAND if (self.classifier.precision == "bf16" and self._model_src is not None) else None
+            band = TIE_BANDS.get(self.classifier.arch, DEFAULT_TIE_BAND)
+            refine_ties = band if (self.classifier.precision == "bf16" and self._model_src is not None) else None
         self.refine_ties = float(refine_ties) if (refine_ties and self.classifier.precision == "bf16") else None
         if self.refine_ties is not None and self._model_src is None:
             raise ValueError("refine_ties needs the torch module (to lower an fp32 copy), not a lowered Classifier")
         self.tie_capacity = int(tie_capacity)
         self.tie_window = max(1, int(tie_window))
         if tie_precision == "auto":
-            # torchvision ResNets (every body conv a multiple of 64 channels wide) re-score on the tcgen05 pair kernel over
-            # split-bf16 tensors; everything else on the mma.sync split-bf16 kernel over fp32 tensors
-            tie_precision = "split" if self.classifier.arch == "tv_resnet" else "x3"
+            # torchvision ResNets, VGGs and AlexNet (every body conv a multiple of 64 channels wide) re-score on the tcgen05
+            # pair kernel over split-bf16 tensors; everything else on the mma.sync split-bf16 kernel over fp32 tensors
+            tie_precision = "split" if self.classifier.arch in ("tv_resnet", "tv_plain") else "x3"
         if tie_precision not in ("split", "x3", "fp32"):
             raise ValueError("tie_precision must be 'auto', 'split' (split-bf16 tensors, tcgen05), 'x3' (split-bf16 products on "
                              "fp32 tensors, mma.sync) or 'fp32' (CUDA cores)")
