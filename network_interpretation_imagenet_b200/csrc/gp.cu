@@ -187,7 +187,8 @@ dgemm_sub_kernel(DgemmArgs g) {
   // C -= acc.  Each thread owns column pairs (2fk, 2fk+1): one 16-byte access per pair, so the four lanes of a fragment
   // row cover a whole 64 B (two full sectors) — 8-byte accesses wrote every sector in four partial pieces and the
   // read-modify-write of C ran at ~1 TB/s.  Loads are gathered in batches before any store of the batch (a store may
-  // alias the next load as far as the compiler knows, which would serialise the L2 round trips).
+  // alias the next load as far as the compiler knows, which would serialise the L2 round trips).  Row offsets are
+  // 64-bit like the operand pointers': C may span more than 2^31 elements.
   const bool vec_ok = ((g.ldc & 1) == 0) && ((reinterpret_cast<uintptr_t>(g.C) & 15) == 0);
 #pragma unroll
   for (int mb = 0; mb < MT; mb += 2) {
@@ -200,10 +201,10 @@ dgemm_sub_kernel(DgemmArgs g) {
         const int j = j0 + wn * 32 + nt * 8 + 2 * fk;
         const bool ok0 = i < g.M && j < g.N && !(g.lower_only && j > i);
         const bool ok1 = i < g.M && j + 1 < g.N && !(g.lower_only && j + 1 > i);
-        if (vec_ok && ok0 && ok1) cv[m2][nt] = *reinterpret_cast<const double2*>(g.C + i * g.ldc + j);
+        if (vec_ok && ok0 && ok1) cv[m2][nt] = *reinterpret_cast<const double2*>(g.C + (long long)i * g.ldc + j);
         else {
-          cv[m2][nt].x = ok0 ? g.C[i * g.ldc + j] : 0.0;
-          cv[m2][nt].y = ok1 ? g.C[i * g.ldc + j + 1] : 0.0;
+          cv[m2][nt].x = ok0 ? g.C[(long long)i * g.ldc + j] : 0.0;
+          cv[m2][nt].y = ok1 ? g.C[(long long)i * g.ldc + j + 1] : 0.0;
         }
       }
     }
@@ -216,10 +217,10 @@ dgemm_sub_kernel(DgemmArgs g) {
         const bool ok0 = i < g.M && j < g.N && !(g.lower_only && j > i);
         const bool ok1 = i < g.M && j + 1 < g.N && !(g.lower_only && j + 1 > i);
         const double2 o = make_double2(cv[m2][nt].x - acc[mb + m2][nt][0], cv[m2][nt].y - acc[mb + m2][nt][1]);
-        if (vec_ok && ok0 && ok1) *reinterpret_cast<double2*>(g.C + i * g.ldc + j) = o;
+        if (vec_ok && ok0 && ok1) *reinterpret_cast<double2*>(g.C + (long long)i * g.ldc + j) = o;
         else {
-          if (ok0) g.C[i * g.ldc + j] = o.x;
-          if (ok1) g.C[i * g.ldc + j + 1] = o.y;
+          if (ok0) g.C[(long long)i * g.ldc + j] = o.x;
+          if (ok1) g.C[(long long)i * g.ldc + j + 1] = o.y;
         }
       }
     }
@@ -1141,7 +1142,7 @@ __global__ void transpose_kernel(const double* __restrict__ in, int rows, int co
 __global__ void __launch_bounds__(256)
 gemv_mean_kernel(const double* __restrict__ Ks, int m, int n, int ldks, const double* __restrict__ alpha, double y_mean,
                  double y_std, double* __restrict__ mu) {
-  const int q = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int q = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);   // one warp per query
   const int lane = threadIdx.x & 31;
   if (q >= m) return;
   double acc = 0.0;
@@ -1494,7 +1495,7 @@ int nib_gp_posterior(const double* d_L, int n, int ldl, const double* d_alpha, c
   NIB_REQUIRE(d_L && d_alpha && d_Ks && n > 0 && m > 0 && ldl >= n && ldks >= n, "nib_gp_posterior: bad arguments");
   cudaStream_t st = (cudaStream_t)stream;
   if (d_mu) {
-    gemv_mean_kernel<<<ceil_div(m * 32, 256), 256, 0, st>>>(d_Ks, m, n, ldks, d_alpha, y_mean, y_std, d_mu);
+    gemv_mean_kernel<<<ceil_div(m, 8), 256, 0, st>>>(d_Ks, m, n, ldks, d_alpha, y_mean, y_std, d_mu);
     NIB_LAUNCH_CHECK();
   }
   if (d_var || d_std) {
