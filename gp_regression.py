@@ -4,14 +4,19 @@ Same entry points and on-disk contract as the reference (file:line are the refer
   load_images_from_folder(folder)        :63-72    ./masks/mask_{i}_{label}.png, label parsed from the file name
   prepare_training_data()                :74-156   heat map H[p] = sum of labels of the masks whose pixel p is 255; train_x = the
                                                    covered pixel coordinates (i, j), train_y = H there
-  GPRegressionModel(train_x, train_y, likelihood)  :160-176  KISS-GP: RBF on a 30 x 30 interpolation grid over [0, n]^2 + outputscale
+  GPRegressionModel(train_x, train_y, likelihood, grid_size=30)  :160-176  KISS-GP: RBF on a grid_size x grid_size interpolation
+                                                   grid over [0, n]^2 + outputscale (grid_size=300 as the reference's
+                                                   gp_superpixel_data_imagenet.py uses: the Kronecker solver, see below)
   train(...)                             :179-229  evaluates the marginal likelihood 20 times WITHOUT stepping the optimiser in the
                                                    branch it runs, then saves the (initial) parameters
   eval_superpixels(model, likelihood)    :232-281  posterior of `likelihood(model(x))` at all n x n pixels
   plot_result(predictions)               :284-372  heat maps (written to ./weighted_mask/ here instead of cv2.imshow / matplotlib)
 
 What changed underneath: the O(N * n^2) Python dictionary loop is one HBM-bound kernel (`nib_heatmap_pixels`), and the GP is
-solved exactly in its inducing-weight form on the device (network_interpretation_imagenet_b200/ski.py, csrc/ski.cu + gp.cu).
+solved exactly in its inducing-weight form on the device (network_interpretation_imagenet_b200/ski.py, csrc/ski.cu + gp.cu):
+with dense G x G factors (G = grid_size^2) up to grid_size 100, and above that, where they no longer fit, matrix-free by
+preconditioned conjugate gradients on the Kronecker structure of the grid kernel (csrc/ski_kron.cu).  The checkpoint
+keeps grid_size, so eval_superpixels predicts on the grid the model was trained with.
 gpytorch is not needed (and absent here): the checkpoint is a small dict of the model's hyper-parameters.
 """
 from __future__ import annotations
@@ -102,8 +107,9 @@ class GaussianLikelihood:
 
 
 class GPRegressionModel:
-    """KISS-GP regression with the reference's structure: near-zero constant mean, RBF base kernel on a grid_size = 30
-    interpolation grid over [0, n]^2, trainable log_outputscale (all initial values 0, as gpytorch's parameters)."""
+    """KISS-GP regression with the reference's structure: near-zero constant mean, RBF base kernel on a grid_size x
+    grid_size interpolation grid over [0, n]^2 (30 by default, as the reference's gp_regression.py; 300 as its
+    gp_superpixel_data_imagenet.py), trainable log_outputscale (all initial values 0, as gpytorch's parameters)."""
 
     def __init__(self, train_x, train_y, likelihood, grid_size=30):
         self.train_x, self.train_y, self.likelihood = train_x, train_y, likelihood

@@ -28,7 +28,8 @@
 extern "C" {
 #endif
 
-#define NIB_ABI_VERSION 2   /* 2: + tie policy, device-side batch size, NCCL score all-gather, threshold/bbox helpers */
+#define NIB_ABI_VERSION 3   /* 2: + tie policy, device-side batch size, NCCL score all-gather, threshold/bbox helpers
+                               3: + Kronecker-structured SKI (nib_ski_kron_*, nib_ski_band_*) */
 
 enum nib_status {
   NIB_OK = 0,
@@ -398,6 +399,38 @@ int nib_ski_accumulate(const double* d_X, const double* d_y, int n, double grid0
 int nib_ski_predict(const double* d_Xq, int m, double grid0, double spacing, int grid_size,
                     double const_mean, const double* d_mean_u, const double* d_Gm, double noise,
                     int add_noise, double* d_mean, double* d_var, void* stream);
+
+/* The same SKI model on grids too large for dense G x G factors (grid_size 300: G = 90 000), csrc/ski_kron.cu.
+ * K = os K1 (x) K1 has the square root S = M_R (x) M_C with gs x gs factors built on the host (ski.py), and
+ *   mean_U = S B^-1 S^T b,   var(x*) = noise (S^T w*)^T B^-1 (S^T w*) (+ noise),   B = noise I + S^T A S,
+ * solved by preconditioned CG with the diagonal D = noise + coef * thetaR[i] * thetaC[j] (exact for a lattice of pixels).
+ * Vectors over the grid are G = gs^2 doubles, row-major (index i0 * gs + i1); r right-hand sides are r such vectors
+ * back to back.  r <= 65535, grid_size <= 46340.
+ *   nib_ski_kron_apply        Y[:, c] = (M_R (x) M_C) X[:, c] (trans 0) or (M_R (x) M_C)^T X[:, c] (trans 1), i.e.
+ *                             M_R X_c M_C^T / M_R^T X_c M_C per gs x gs block; d_MR, d_MC [gs][gs]; d_work r*G doubles
+ *   nib_ski_band_accumulate   A = W^T W in band form d_A [G][7][7] (A[g][(d0+3)*7 + d1+3] couples g with g + (d0, d1),
+ *                             zero where that leaves the grid) and d_b = W^T (y - const_mean) [G], without floating-point
+ *                             atomics (bitwise reproducible).  d_work: 4 * (2n + 3G + 2) + 72 n bytes
+ *   nib_ski_band_spmv         Y[:, c] = A X[:, c] for the band A above
+ *   nib_ski_kron_pcg          solves B x = rhs for r columns (d_rhs, d_x [r][G]) to relative residual <= tol per column;
+ *                             d_thetaR, d_thetaC [gs]; d_work 8 * (5 r G + 5 r + 4) bytes.  The host reads the state every
+ *                             check_every iterations; on return *h_iters = most iterations taken by a column and
+ *                             *h_relres = largest relative residual reached (> tol: not converged within max_iter)
+ *   nib_ski_kron_var_rhs      d_rhs[q] = (M_R^T w0_q) (x) (M_C^T w1_q) for m queries d_Xq [m, 2] (grid_size <= 3072)
+ *   nib_ski_kron_var_reduce   d_var[q] = noise * d_rhs[q] . d_x[q] (+ noise when add_noise) */
+int nib_ski_kron_apply(const double* d_X, double* d_Y, int r, int grid_size, const double* d_MR, const double* d_MC,
+                       int trans, double* d_work, void* stream);
+int nib_ski_band_accumulate(const double* d_X, const double* d_y, int n, double grid0, double spacing, int grid_size,
+                            double const_mean, double* d_A, double* d_b, void* d_work, void* stream);
+int nib_ski_band_spmv(const double* d_A, int grid_size, const double* d_X, double* d_Y, int r, void* stream);
+int nib_ski_kron_pcg(const double* d_A, int grid_size, const double* d_MR, const double* d_MC, const double* d_thetaR,
+                     const double* d_thetaC, double coef, double noise, const double* d_rhs, double* d_x, int r,
+                     double tol, int max_iter, int check_every, double* d_work, int* h_iters, double* h_relres,
+                     void* stream);
+int nib_ski_kron_var_rhs(const double* d_Xq, int m, double grid0, double spacing, int grid_size, const double* d_MR,
+                         const double* d_MC, double* d_rhs, void* stream);
+int nib_ski_kron_var_reduce(const double* d_rhs, const double* d_x, int m, int grid_size, double noise, int add_noise,
+                            double* d_var, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * Variational GP classification on the inducing grid: the O(n) part of one optimiser step of

@@ -13,7 +13,7 @@ PKG_DIR = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(PKG_DIR, "libnib.so")
 
 NIB_OK = 0
-ABI_VERSION = 2
+ABI_VERSION = 3
 MASK_KEEP_MUL, MASK_REMOVE_MINMAX = 0, 1
 F32, BF16 = 0, 1
 NCHW, NHWC = 0, 1
@@ -106,6 +106,13 @@ _PROTOTYPES = {
     "nib_heatmap_pixels": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp]),
     "nib_ski_accumulate": (_i, [_vp, _vp, _i, _d, _d, _i, _d, _vp, _vp, _vp]),
     "nib_ski_predict": (_i, [_vp, _i, _d, _d, _i, _d, _vp, _vp, _d, _i, _vp, _vp, _vp]),
+    "nib_ski_kron_apply": (_i, [_vp, _vp, _i, _i, _vp, _vp, _i, _vp, _vp]),
+    "nib_ski_band_accumulate": (_i, [_vp, _vp, _i, _d, _d, _i, _d, _vp, _vp, _vp, _vp]),
+    "nib_ski_band_spmv": (_i, [_vp, _i, _vp, _vp, _i, _vp]),
+    "nib_ski_kron_pcg": (_i, [_vp, _i, _vp, _vp, _vp, _vp, _d, _d, _vp, _vp, _i, _d, _i, _i, _vp, C.POINTER(_i),
+                              C.POINTER(_d), _vp]),
+    "nib_ski_kron_var_rhs": (_i, [_vp, _i, _d, _d, _i, _vp, _vp, _vp, _vp]),
+    "nib_ski_kron_var_reduce": (_i, [_vp, _vp, _i, _i, _d, _i, _vp, _vp]),
     "nib_segment_weights": (_i, [_vp, _i, _vp, _i, _i, _vp, _vp, _vp]),
     "nib_heat_normalize_u8": (_i, [_vp, _i, _vp, _vp, _vp]),
     "nib_threshold_bbox": (_i, [_vp, _i, _i, _i, _vp, _vp]),

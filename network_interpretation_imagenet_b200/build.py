@@ -15,7 +15,7 @@ PKG_DIR = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(PKG_DIR, "csrc")
 LIB_PATH = os.path.join(PKG_DIR, "libnib.so")
 BUILD_DIR = os.path.join(PKG_DIR, "build")
-SOURCES = ["api.cu", "mask_synth.cu", "score.cu", "conv_simt.cu", "conv_x3.cu", "conv_tc.cu", "net.cu", "gp.cu", "segment.cu", "ski.cu", "comm.cu", "localize.cu"]
+SOURCES = ["api.cu", "mask_synth.cu", "score.cu", "conv_simt.cu", "conv_x3.cu", "conv_tc.cu", "net.cu", "gp.cu", "segment.cu", "ski.cu", "ski_kron.cu", "comm.cu", "localize.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-O3", "-lineinfo", "-std=c++17",
