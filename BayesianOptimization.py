@@ -11,7 +11,8 @@ integer in [lo, hi) and ignores `n_restarts` (:84-90); duplicates are replaced b
 
 `bayesian_optimisation_masks` is the scaled-up form BASELINE.json's config 4 names: the GP input is the mask
 itself (selection bit-vector, Hamming-RBF kernel) and each round scores all m candidate masks on the device
-(fit -> posterior on m candidates -> EI arg-max -> one new evaluation -> append)."""
+(fit -> posterior on m candidates -> EI arg-max -> one new evaluation -> append), or with `batch_size` q > 1 q
+Kriging-believer picks per round, scored in one batched forward."""
 from __future__ import annotations
 
 from random import randint
@@ -91,19 +92,47 @@ def bayesian_optimisation(n_iters, sample_loss, val_loader, nn_model, criterion,
 
 
 def bayesian_optimisation_masks(n_iters, score_masks, train_bits, train_scores, candidate_bits, alpha=1e-5,
-                                length_scale=None, n_restarts_optimizer=0, refit_every=0, random_state=0):
+                                length_scale=None, n_restarts_optimizer=0, refit_every=0, random_state=0, batch_size=1):
     """Active learning over masks (BASELINE config 4: `n_iters` rounds on n training masks, m candidates).
 
     score_masks(bits[k, words]) -> np.ndarray[k] target-class probabilities, e.g.
     `lambda b: engine.score_masks(b)["target_prob"].cpu().numpy()` (PerturbationEngine.score_masks itself returns a dict
     of device tensors).
     Each round: GP fit on (train_bits, train_scores) -> posterior mean/std on every remaining candidate -> EI
-    (greater_is_better, as reference :175) -> arg-max candidate is evaluated and appended."""
+    (greater_is_better, as reference :175) -> arg-max candidate is evaluated and appended.
+
+    batch_size = q > 1 evaluates q masks per round: ActiveMaskGP.select_batch picks them by greedy Kriging believer on
+    the device, one score_masks call scores them together, and set_batch_values enters the scores.  It needs the fixed
+    length scale (`length_scale` given, refit_every = 0).  The history has one entry per evaluated mask."""
     import torch
     Z = np.ascontiguousarray(train_bits, dtype=np.uint64).copy()
     y = np.asarray(train_scores, dtype=np.float64).copy()
     cand = np.ascontiguousarray(candidate_bits, dtype=np.uint64)
     history = []
+    q = int(batch_size)
+    if q < 1:
+        raise ValueError("batch_size must be >= 1")
+    if q > 1:
+        if length_scale is None or refit_every:
+            raise ValueError("batch_size > 1 needs a fixed length_scale and refit_every=0: batch selection extends the "
+                             "resident factor, which a length-scale search would rebuild")
+        gp = _gp.ActiveMaskGP(cand, alpha=alpha, length_scale=length_scale, normalize_y=True,
+                              capacity=n_iters * q).fit(Z, y)
+        for it in range(n_iters):
+            picks, ei = gp.select_batch(q, greater_is_better=True)
+            if len(picks) == 0:   # every EI is NaN (all sigma == 0): one random candidate like reference :178-180
+                alive = np.nonzero(gp.alive.cpu().numpy())[0]
+                j = int(alive[np.random.RandomState(random_state + it).randint(len(alive))])
+                s = float(np.asarray(score_masks(cand[j:j + 1]))[0])
+                history.append({"round": it, "candidate": j, "ei": float("nan"), "score": s, "length_scale": length_scale})
+                gp.append(j, s)
+                continue
+            scores = np.asarray(score_masks(cand[picks]), dtype=np.float64).reshape(-1)
+            gp.set_batch_values(scores)
+            for j, e, s in zip(picks, ei, scores):
+                history.append({"round": it, "candidate": int(j), "ei": float(e), "score": float(s),
+                                "length_scale": length_scale})
+        return np.concatenate([Z, cand[[h["candidate"] for h in history]]], 0), np.asarray(gp.y_host), history
     if length_scale is not None and not refit_every:
         # fixed length scale: the Gram matrix of the points already seen never changes, so each round is a rank-one update
         # of the factor and of the posterior workspace (ActiveMaskGP) instead of an O(n^3 + m n^2) refit

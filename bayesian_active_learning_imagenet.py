@@ -13,7 +13,9 @@ bbox_threshold = 180) sums the labels of the evaluated masks into a heat map, bo
 IOU with the ground-truth box - heat map, 8-bit view and bounding box are device kernels here (localize.py).
 
 `--masks` switches to the scaled-up form of BASELINE.json config 4: the GP input is the mask itself, n training
-masks, `--rounds` acquisition rounds over m candidate masks scored by EI on the device."""
+masks, `--rounds` acquisition rounds over m candidate masks scored by EI on the device.  `--acq-batch Q` (default 1)
+evaluates Q masks per round: Kriging-believer picks on the device, scored in one batched forward (Q * `--rounds` masks in
+all; `-b/--batch-size` stays the forward's micro-batch)."""
 from __future__ import annotations
 
 import argparse
@@ -49,6 +51,7 @@ parser.add_argument("--masks", action="store_true", help="mask-space GP (BASELIN
 parser.add_argument("--n-train", default=8192, type=int)
 parser.add_argument("--n-candidates", default=8192, type=int)
 parser.add_argument("--rounds", default=20, type=int)
+parser.add_argument("--acq-batch", default=1, type=int, help="masks acquired per round with --masks (Kriging believer)")
 parser.add_argument("--mask-seed", default=0, type=int)
 parser.add_argument("--gt-bbox", default=None, type=int, nargs=4, metavar=("X", "Y", "W", "H"),
                     help="ground-truth box of the image (the reference reads it from the ImageNet annotation, :454)")
@@ -148,7 +151,7 @@ def main():
         train, cand = bits[:args.n_train], bits[args.n_train:]
         y = eng.score_masks(train)["target_prob"].cpu().numpy()
         Z, yy, hist = bayesian_optimisation_masks(args.rounds, lambda b: eng.score_masks(b)["target_prob"].cpu().numpy(),
-                                                  train, y, cand, length_scale=3.0)
+                                                  train, y, cand, length_scale=3.0, batch_size=args.acq_batch)
         for h in hist:
             print(h)
     print("time duration is: ", time.time() - start_time)

@@ -28,8 +28,9 @@
 extern "C" {
 #endif
 
-#define NIB_ABI_VERSION 3   /* 2: + tie policy, device-side batch size, NCCL score all-gather, threshold/bbox helpers
-                               3: + Kronecker-structured SKI (nib_ski_kron_*, nib_ski_band_*) */
+#define NIB_ABI_VERSION 4   /* 2: + tie policy, device-side batch size, NCCL score all-gather, threshold/bbox helpers
+                               3: + Kronecker-structured SKI (nib_ski_kron_*, nib_ski_band_*)
+                               4: + Kriging-believer batch acquisition (nib_gp_kb_select) */
 
 enum nib_status {
   NIB_OK = 0,
@@ -347,6 +348,24 @@ int nib_gp_gemv_t(const double* d_V, int n, int m, int ldv, const double* d_x, d
 int nib_gp_colsumsq(const double* d_V, int n, int m, int ldv, double* d_out, void* stream);
 int nib_gp_append_row(const double* d_ks, const double* d_dot, double d, double* d_vrow, double* d_ssq, int m,
                       void* stream);
+
+/* Batch acquisition on the same resident state: q picks by greedy Kriging believer, all on the device.  The fantasy
+ * observation at a pick is its posterior mean, which leaves every other mean unchanged, so with the mean d_mu [m] fixed
+ * (computed once at the current y-normalisation) each pick only adds one row to L and V.  For k = 0 .. q-1:
+ *   sigma_x = y_std * sqrt(max(0, 1 - ssq_x)), NaN where !alive_x;   EI_x as nib_gp_ei with incumbent b
+ *   j = arg-max of the non-NaN EI (lowest index on ties); none -> stop (d_picks[k..q) stay -1)
+ *   l = V[0:n+k, j] (= L^-1 k(X, z_j));  d^2 = 1 + alpha - ssq_j;  d^2 <= 0 -> *d_status = k + 1, stop
+ *   L[n+k, 0:n+k] = l;  L[n+k, n+k] = d;  X[n+k] = cand[j];  V[n+k][x] = (k(x, z_j) - sum_t V[t][x] l_t) / d;
+ *   ssq += V[n+k]^2;  alive_j = 0;  b = max(b, mu_j) (min when !greater_is_better);  d_picks[k] = j;  d_ei[k] = EI_j
+ * d_L [>= n+q][ldl] with n rows filled, d_V [>= n+q][ldv] with n rows filled, d_ssq / d_alive (bytes) [m],
+ * d_cand [m][words] and d_X [>= n+q][words] selection bits, kernel exp(-popcount(a ^ b) * 0.5 / length_scale^2) as
+ * nib_gp_gram_binary.  One pass over V per pick and no host synchronisation inside the batch; d_picks [q] (int64),
+ * d_ei [q] and d_status (int) are the only outputs the caller has to read.  Deterministic (no floating-point atomics).
+ * The observed values then enter u = L^-1 y, w = L^-1 1 through rows n .. n+q-1 of L (ActiveMaskGP.set_batch_values). */
+int nib_gp_kb_select(double* d_L, int ldl, double* d_V, int ldv, double* d_ssq, unsigned char* d_alive,
+                     const uint64_t* d_cand, int m, int words, uint64_t* d_X, int n, int q, const double* d_mu,
+                     double y_std, double best, int greater_is_better, double length_scale, double alpha,
+                     long long* d_picks, double* d_ei, int* d_status, void* stream);
 
 /* Expected improvement, BayesianOptimization.py:37-54 (returns +EI; the reference returns -EI):
  *   s = greater_is_better ? 1 : -1;  Z = s*(mu-best)/sigma;  EI = s*(mu-best)*Phi(Z)+sigma*phi(Z)

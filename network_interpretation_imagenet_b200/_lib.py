@@ -13,7 +13,7 @@ PKG_DIR = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(PKG_DIR, "libnib.so")
 
 NIB_OK = 0
-ABI_VERSION = 3
+ABI_VERSION = 4
 MASK_KEEP_MUL, MASK_REMOVE_MINMAX = 0, 1
 F32, BF16 = 0, 1
 NCHW, NHWC = 0, 1
@@ -102,6 +102,8 @@ _PROTOTYPES = {
     "nib_gp_gemv_t": (_i, [_vp, _i, _i, _i, _vp, _vp, _vp]),
     "nib_gp_colsumsq": (_i, [_vp, _i, _i, _i, _vp, _vp]),
     "nib_gp_append_row": (_i, [_vp, _vp, _d, _vp, _vp, _i, _vp]),
+    "nib_gp_kb_select": (_i, [_vp, _i, _vp, _i, _vp, _vp, _vp, _i, _i, _vp, _i, _i, _vp, _d, _d, _i, _d, _d, _vp, _vp,
+                              _vp, _vp]),
     "nib_heatmap": (_i, [_vp, _i, _i, _i, _i, _vp, _i, _vp, _i, _vp, _vp]),
     "nib_heatmap_pixels": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp]),
     "nib_ski_accumulate": (_i, [_vp, _vp, _i, _d, _d, _i, _d, _vp, _vp, _vp]),

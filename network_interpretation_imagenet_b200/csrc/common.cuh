@@ -53,7 +53,7 @@ int num_sms();
 // Per-(use, device, stream) library scratch of at least `bytes` (allocated with max(bytes, min_bytes) when it has to
 // grow).  Never shared between streams; see api.cu.
 enum ScratchSlot { SCRATCH_GP_DINV = 0, SCRATCH_GP_TRSV, SCRATCH_GP_COLREDUCE, SCRATCH_GP_SCALARS, SCRATCH_HEAT_WSEG,
-                   SCRATCH_TIES, SCRATCH_BBOX };
+                   SCRATCH_TIES, SCRATCH_BBOX, SCRATCH_GP_KB };
 int stream_scratch(int slot, cudaStream_t st, size_t bytes, size_t min_bytes, void** out);
 
 template <typename T> struct Elem;

@@ -1301,16 +1301,19 @@ __global__ void sum_kernel(const double* __restrict__ v, int n, double* __restri
 }
 
 // ---- Expected improvement ----------------------------------------------------------------------
+// shared by ei_kernel and the Kriging-believer selection so that both produce the same bits
+__device__ __forceinline__ double ei_value(double mu, double s, double best, double sf) {
+  const double d = sf * (mu - best);
+  const double Z = d / s;  // sigma == 0 -> inf/NaN, as the reference (np.errstate(divide='ignore'))
+  const double Phi = 0.5 * erfc(-Z * 0.70710678118654752440);
+  const double phi = exp(-0.5 * Z * Z) * 0.39894228040143267794;
+  return d * Phi + s * phi;
+}
 __global__ void ei_kernel(const double* __restrict__ mu, const double* __restrict__ sigma, int m, double best, double sf,
                           double* __restrict__ ei) {
   const int q = blockIdx.x * blockDim.x + threadIdx.x;
   if (q >= m) return;
-  const double s = sigma[q];
-  const double d = sf * (mu[q] - best);
-  const double Z = d / s;  // sigma == 0 -> inf/NaN, as the reference (np.errstate(divide='ignore'))
-  const double Phi = 0.5 * erfc(-Z * 0.70710678118654752440);
-  const double phi = exp(-0.5 * Z * Z) * 0.39894228040143267794;
-  ei[q] = d * Phi + s * phi;
+  ei[q] = ei_value(mu[q], sigma[q], best, sf);
 }
 __global__ void argmax_kernel(const double* __restrict__ v, int m, long long* __restrict__ out) {
   __shared__ double sv[32];
@@ -1334,6 +1337,174 @@ __global__ void argmax_kernel(const double* __restrict__ v, int m, long long* __
     }
     out[0] = bi;
   }
+}
+
+// ---- Kriging-believer batch selection (nib_gp_kb_select) ---------------------------------------------------------------
+// Greedy q-pick acquisition on the resident rank-one state of ActiveMaskGP.  The fantasy observation at a pick equals its
+// posterior mean, which leaves every other mean unchanged, so a pick only shrinks variances: one new row of V per pick.
+// Per pick two launches, with the pick index passed through device memory so the host never waits inside a batch:
+//   kb_colreduce_kernel  dot[x] = sum_t V[t][x] * l_t over row slices, l = V[:, j] (= the new row of L, written too)
+//   kb_finalize_kernel   fixed-order slice sum, V[n+k][x] = (k(x, z_j) - dot[x]) / d, ssq update, sigma, EI, block
+//                        arg-max; the last block to finish (atomic counter, no spinning) publishes the next pick.
+// No floating-point atomics: picks and V are bitwise reproducible.
+static constexpr int KB_THREADS = 256, KB_COLS = 2, KB_TILE = KB_THREADS * KB_COLS, KB_UNROLL = 8;
+
+struct KbCtrl {
+  long long pick;       // index of the pick whose row is being added; -1 once selection has stopped
+  double d;             // its new diagonal entry of L
+  double best;          // incumbent after the picks so far (Kriging believer: the picked means count as observed)
+  unsigned int done;    // finalize blocks finished (reset by the last one)
+};
+
+struct KbArgs {
+  double* L; int ldl; double* V; long long ldv; double* ssq; unsigned char* alive;
+  const uint64_t* cand; int m; int words; uint64_t* X; int n;
+  const double* mu; double var_scale; double alpha; double inv_l2_half; double sf; double best0;
+  long long* picks; double* ei; int* status;
+  KbCtrl* ctrl; const double* partial; double* bval; long long* bidx;
+};
+
+// (v, i) beats (bv, bi): larger non-NaN value, lower index on ties (argmax_kernel's rule); a total order, so any
+// reduction tree gives the same winner
+__device__ __forceinline__ void kb_better(double& bv, long long& bi, double v, long long i) {
+  if (i >= 0 && (bi < 0 || v > bv || (v == bv && i < bi))) { bv = v; bi = i; }
+}
+__device__ __forceinline__ void kb_block_argmax(double& bv, long long& bi, double* sv, long long* si) {
+  for (int o = 16; o > 0; o >>= 1) {
+    const double ov = __shfl_xor_sync(0xffffffffu, bv, o);
+    const long long oi = __shfl_xor_sync(0xffffffffu, bi, o);
+    kb_better(bv, bi, ov, oi);
+  }
+  if ((threadIdx.x & 31) == 0) { sv[threadIdx.x >> 5] = bv; si[threadIdx.x >> 5] = bi; }
+  __syncthreads();
+  if (threadIdx.x == 0)
+    for (int w = 1; w < KB_THREADS / 32; ++w) kb_better(bv, bi, sv[w], si[w]);
+}
+
+// partial[s][x] = sum_{t in slice s} V[t][x] * V[t][j]   (t < nk).  Each thread owns KB_COLS columns 256 apart and keeps
+// KB_UNROLL * KB_COLS independent loads in flight; l is staged through shared memory 256 rows at a time.
+__global__ void __launch_bounds__(KB_THREADS)
+kb_colreduce_kernel(const double* __restrict__ V, long long ldv, int nk, int m, int rows, double* __restrict__ Lrow,
+                    const KbCtrl* __restrict__ ctrl, double* __restrict__ partial) {
+  const long long j = ctrl->pick;
+  if (j < 0) return;
+  __shared__ double ls[KB_THREADS];
+  const int t0 = blockIdx.y * rows, t1 = min(nk, t0 + rows);
+  const int x0 = blockIdx.x * KB_TILE + threadIdx.x;
+  double acc[KB_COLS];
+#pragma unroll
+  for (int c = 0; c < KB_COLS; ++c) acc[c] = 0.0;
+  for (int c0 = t0; c0 < t1; c0 += KB_THREADS) {
+    const int cn = min(KB_THREADS, t1 - c0);
+    __syncthreads();
+    if (threadIdx.x < cn) {
+      const double l = V[(size_t)(c0 + threadIdx.x) * ldv + j];
+      ls[threadIdx.x] = l;
+      if (blockIdx.x == 0) Lrow[c0 + threadIdx.x] = l;
+    }
+    __syncthreads();
+    for (int u0 = 0; u0 < cn; u0 += KB_UNROLL) {
+      double v[KB_UNROLL][KB_COLS];
+#pragma unroll
+      for (int u = 0; u < KB_UNROLL; ++u)
+#pragma unroll
+        for (int c = 0; c < KB_COLS; ++c) {
+          const int x = x0 + c * KB_THREADS;
+          v[u][c] = (u0 + u < cn && x < m) ? __ldcs(V + (size_t)(c0 + u0 + u) * ldv + x) : 0.0;
+        }
+#pragma unroll
+      for (int u = 0; u < KB_UNROLL; ++u) {
+        const double l = u0 + u < cn ? ls[u0 + u] : 0.0;
+#pragma unroll
+        for (int c = 0; c < KB_COLS; ++c) acc[c] = fma(v[u][c], l, acc[c]);
+      }
+    }
+  }
+#pragma unroll
+  for (int c = 0; c < KB_COLS; ++c) {
+    const int x = x0 + c * KB_THREADS;
+    if (x < m) partial[(size_t)blockIdx.y * m + x] = acc[c];
+  }
+}
+
+// kpub: index of the pick this launch publishes (q: none).  add_row: first append row n + kpub - 1 for the current pick
+// from the `slices` partial sums.  Dynamic shared memory: the (64 * words + 1)-entry Hamming LUT of gram_binary_kernel.
+__global__ void __launch_bounds__(KB_THREADS)
+kb_finalize_kernel(KbArgs a, int kpub, int q, int add_row, int slices) {
+  extern __shared__ double lut[];
+  __shared__ double sv[KB_THREADS / 32];
+  __shared__ long long si[KB_THREADS / 32];
+  __shared__ int last;
+  KbCtrl* c = a.ctrl;
+  const long long jc = add_row ? c->pick : 0;
+  if (jc < 0) return;
+  const int x = blockIdx.x * KB_THREADS + threadIdx.x;
+  double s2 = x < a.m ? a.ssq[x] : 0.0;
+  if (add_row) {
+    const int nl = 64 * a.words + 1;
+    for (int h = threadIdx.x; h < nl; h += KB_THREADS) lut[h] = exp(-(double)h * a.inv_l2_half);
+    __syncthreads();
+    if (x < a.m) {
+      double dot = 0.0;
+      for (int s = 0; s < slices; ++s) dot += a.partial[(size_t)s * a.m + x];
+      int h = 0;
+      for (int w = 0; w < a.words; ++w) h += __popcll(a.cand[(size_t)x * a.words + w] ^ a.cand[(size_t)jc * a.words + w]);
+      const double v = (lut[h] - dot) / c->d;
+      a.V[(size_t)(a.n + kpub - 1) * a.ldv + x] = v;
+      s2 = fma(v, v, s2);
+      a.ssq[x] = s2;
+      __threadfence();   // the last block reads ssq[j] of the new pick
+    }
+  }
+  if (kpub >= q) return;
+  const double best = add_row ? c->best : a.best0;
+  double bv = NAN;
+  long long bi = -1;
+  if (x < a.m && a.alive[x]) {
+    double r = 1.0 - s2;   // ActiveMaskGP.posterior(): var = clamp(1 - ssq, 0) * ystd^2, sd = sqrt(var)
+    if (r < 0.0) r = 0.0;
+    const double e = ei_value(a.mu[x], sqrt(r * a.var_scale), best, a.sf);
+    if (e == e) { bv = e; bi = x; }
+  }
+  kb_block_argmax(bv, bi, sv, si);
+  if (threadIdx.x == 0) {
+    a.bval[blockIdx.x] = bv;
+    a.bidx[blockIdx.x] = bi;
+    __threadfence();
+    last = atomicAdd(&c->done, 1u) == gridDim.x - 1;
+  }
+  __syncthreads();
+  if (!last) return;
+  __threadfence();
+  bv = NAN;
+  bi = -1;
+  for (int b = threadIdx.x; b < (int)gridDim.x; b += KB_THREADS) kb_better(bv, bi, __ldcg(a.bval + b), __ldcg(a.bidx + b));
+  __syncthreads();
+  kb_block_argmax(bv, bi, sv, si);
+  if (threadIdx.x != 0) return;
+  c->done = 0;
+  if (bi < 0) { c->pick = -1; return; }                       // no candidate with a defined EI left
+  const double d2 = 1.0 + a.alpha - __ldcg(a.ssq + bi);
+  if (!(d2 > 0.0)) { *a.status = kpub + 1; c->pick = -1; return; }
+  const double d = sqrt(d2);
+  const int row = a.n + kpub;
+  a.picks[kpub] = bi;
+  a.ei[kpub] = bv;
+  c->pick = bi;
+  c->d = d;
+  const double mj = a.mu[bi];
+  c->best = a.sf > 0.0 ? (mj > best ? mj : best) : (mj < best ? mj : best);
+  a.alive[bi] = 0;
+  a.L[(size_t)row * a.ldl + row] = d;
+  for (int w = 0; w < a.words; ++w) a.X[(size_t)row * a.words + w] = a.cand[(size_t)bi * a.words + w];
+}
+
+// rows per colreduce slice for nk rows: enough slices that the grid covers every SM about four times, at least 64 rows each
+static void kb_slices(int nk, int m, int* slices, int* rows) {
+  const int tiles = ceil_div(m, KB_TILE);
+  const int s = max(1, min(ceil_div(nk, 64), ceil_div(4 * num_sms(), tiles)));
+  *rows = ceil_div(nk, s);
+  *slices = ceil_div(nk, *rows);
 }
 
 // small device scratch for scalar reductions (per stream, common.cuh)
@@ -1528,6 +1699,61 @@ int nib_gp_append_row(const double* d_ks, const double* d_dot, double d, double*
   NIB_REQUIRE(d_ks && d_dot && d_vrow && d_ssq && m > 0 && d > 0.0, "nib_gp_append_row: bad arguments");
   append_row_kernel<<<ceil_div(m, 256), 256, 0, (cudaStream_t)stream>>>(d_ks, d_dot, d, d_vrow, d_ssq, m);
   NIB_LAUNCH_CHECK();
+  return NIB_OK;
+}
+
+int nib_gp_kb_select(double* d_L, int ldl, double* d_V, int ldv, double* d_ssq, unsigned char* d_alive,
+                     const uint64_t* d_cand, int m, int words, uint64_t* d_X, int n, int q, const double* d_mu,
+                     double y_std, double best, int greater_is_better, double length_scale, double alpha,
+                     long long* d_picks, double* d_ei, int* d_status, void* stream) {
+  NIB_DEVICE_OR_FAIL();
+  NIB_REQUIRE(d_L && d_V && d_ssq && d_alive && d_cand && d_X && d_mu && d_picks && d_ei && d_status,
+              "nib_gp_kb_select: null pointer");
+  NIB_REQUIRE(n > 0 && q > 0 && m > 0 && words > 0 && words <= 64 && ldl >= n + q && ldv >= m,
+              "nib_gp_kb_select: bad shape");
+  NIB_REQUIRE(length_scale > 0.0 && alpha >= 0.0 && y_std > 0.0, "nib_gp_kb_select: bad hyper-parameters");
+  cudaStream_t st = (cudaStream_t)stream;
+  const int nblk = ceil_div(m, KB_THREADS);
+  // ceil(nk / ceil(nk / s)) is not monotone in nk (m = 1792 on 148 SMs: 148 slices for nk = 9458 .. 9472, 146 at
+  // nk = 9473), so the partials buffer is sized for the largest count any pick of this batch launches
+  int max_slices = 0, rows = 0;
+  for (int k = 0; k < q; ++k) {
+    int slices = 0;
+    kb_slices(n + k, m, &slices, &rows);
+    max_slices = max(max_slices, slices);
+  }
+  // scratch: control block | per-block arg-max values | indices | colreduce partial sums [slices][m]
+  const size_t head = 64, bytes = head + (size_t)nblk * 16 + (size_t)max_slices * m * sizeof(double);
+  unsigned char* scratch = nullptr;
+  int rc = stream_scratch(SCRATCH_GP_KB, st, bytes, bytes, reinterpret_cast<void**>(&scratch));
+  if (rc != NIB_OK) return rc;
+  KbArgs a;
+  a.L = d_L; a.ldl = ldl; a.V = d_V; a.ldv = ldv; a.ssq = d_ssq; a.alive = d_alive;
+  a.cand = d_cand; a.m = m; a.words = words; a.X = d_X; a.n = n;
+  a.mu = d_mu; a.var_scale = y_std * y_std; a.alpha = alpha; a.inv_l2_half = 0.5 / (length_scale * length_scale);
+  a.sf = greater_is_better ? 1.0 : -1.0; a.best0 = best;
+  a.picks = d_picks; a.ei = d_ei; a.status = d_status;
+  a.ctrl = reinterpret_cast<KbCtrl*>(scratch);
+  a.bval = reinterpret_cast<double*>(scratch + head);
+  a.bidx = reinterpret_cast<long long*>(scratch + head + (size_t)nblk * 8);
+  double* partial = reinterpret_cast<double*>(scratch + head + (size_t)nblk * 16);
+  a.partial = partial;
+  NIB_CUDA(cudaMemsetAsync(scratch, 0, head, st));
+  NIB_CUDA(cudaMemsetAsync(d_picks, 0xff, (size_t)q * sizeof(long long), st));   // -1: not picked
+  NIB_CUDA(cudaMemsetAsync(d_status, 0, sizeof(int), st));
+  const size_t lut = sizeof(double) * (64 * words + 1);
+  kb_finalize_kernel<<<nblk, KB_THREADS, 0, st>>>(a, 0, q, 0, 0);   // pick 0 from the current state
+  NIB_LAUNCH_CHECK();
+  for (int k = 0; k < q; ++k) {
+    int slices = 0;
+    kb_slices(n + k, m, &slices, &rows);
+    dim3 grid(ceil_div(m, KB_TILE), slices);
+    kb_colreduce_kernel<<<grid, KB_THREADS, 0, st>>>(d_V, ldv, n + k, m, rows, d_L + (size_t)(n + k) * ldl, a.ctrl,
+                                                     partial);
+    NIB_LAUNCH_CHECK();
+    kb_finalize_kernel<<<nblk, KB_THREADS, lut, st>>>(a, k + 1, q, 1, slices);   // row n + k, then pick k + 1
+    NIB_LAUNCH_CHECK();
+  }
   return NIB_OK;
 }
 

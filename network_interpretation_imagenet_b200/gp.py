@@ -236,7 +236,12 @@ class ActiveMaskGP:
 
     and   mu = ybar + V^T (u - ybar w),   var = ystd^2 max(0, 1 - ssq)   (u = L^-1 y, w = L^-1 1: y-normalisation,
     _gpr.py:276-280, changes every round but stays an O(n) correction).  O(n^2 + m n) per round; same posterior as a
-    refit up to rounding (tests/test_gpu_gp.py compares the two and the scikit-learn oracle)."""
+    refit up to rounding (tests/test_gpu_gp.py compares the two and the scikit-learn oracle).
+
+    `select_batch(q)` picks q candidates at once by greedy Kriging believer (nib_gp_kb_select): each pick is fantasised
+    at its posterior mean, which leaves every other mean unchanged and only shrinks variances, so the q picks cost q new
+    rows of L and V and no host round trip.  `set_batch_values(scores)` then puts the measured values in place of the
+    fantasies."""
 
     def __init__(self, candidate_bits, alpha: float = 1e-5, length_scale: float = 1.0, normalize_y: bool = True,
                  capacity: int = 64, device="cuda"):
@@ -248,6 +253,8 @@ class ActiveMaskGP:
         self.cand_host = cand
         self.cand_d = torch.from_numpy(cand.view(np.int64)).to(self.device)
         self.alive = torch.ones(self.m, dtype=torch.bool, device=self.device)
+        self._pending = None     # the last select_batch() while its values are outstanding
+        self.stats = {}
 
     def _gram(self, A, na, B, nb, jitter, out, ld):
         _lib.check(self.lib.nib_gp_gram_binary(A.data_ptr(), na, B.data_ptr(), nb, self.words, self.ell, jitter,
@@ -278,6 +285,7 @@ class ActiveMaskGP:
         for r in range(2):
             _lib.check(self.lib.nib_gp_trsm(self.L.data_ptr(), n, cap, self.uw[r].data_ptr(), 1, 1, 0, st), "nib_gp_trsm")
         self._tmp = torch.empty(3, max(m, cap), dtype=torch.float64, device=dev)
+        self._pending = None
         return self
 
     def _ystats(self):
@@ -289,7 +297,15 @@ class ActiveMaskGP:
 
     def posterior(self):
         """(mu, var, std) over the whole candidate pool, fp64 on the device; candidates already used carry std = NaN so
-        that Expected Improvement skips them (the reference's duplicate guard, BayesianOptimization.py:178-180)."""
+        that Expected Improvement skips them (the reference's duplicate guard, BayesianOptimization.py:178-180).
+        While a batch awaits set_batch_values() this is the posterior given its fantasies: the mean the batch was
+        selected with and the variances after its rows, both at the y-normalisation of that moment."""
+        if self._pending is not None:
+            ystd = self._pending["ystats"][1]
+            var = (1.0 - self.ssq).clamp_(min=0.0) * (ystd * ystd)
+            sd = var.sqrt()
+            sd[~self.alive] = float("nan")
+            return self._pending["mu"].clone(), var, sd
         n, m, st = self.n, self.m, _lib.stream_handle()
         ybar, ystd = self._ystats()
         z = self._tmp[0, :n]
@@ -304,6 +320,8 @@ class ActiveMaskGP:
 
     def append(self, index: int, y_new: float):
         """Candidate `index` has been evaluated: it joins the training set (and leaves the pool)."""
+        if self._pending is not None:
+            raise RuntimeError("ActiveMaskGP: the last select_batch() awaits set_batch_values()")
         if self.n >= self.cap:
             raise RuntimeError("ActiveMaskGP capacity exhausted: construct with a larger `capacity`")
         n, m, cap, st = self.n, self.m, self.cap, _lib.stream_handle()
@@ -328,6 +346,73 @@ class ActiveMaskGP:
         self.y_host.append(float(y_new))
         self.alive[index] = False
         self.n = n + 1
+
+    def select_batch(self, q: int, greater_is_better: bool = True):
+        """Up to q candidates to evaluate next, by greedy Kriging believer on the device: pick the EI arg-max, condition on
+        a fantasy observation equal to its posterior mean (the incumbent becomes max(incumbent, that mean)), repeat.
+        The mean is computed once, at the current y-normalisation.  Returns (picks int64, EI at each pick); fewer than q
+        when no candidate with a defined EI is left.  The picks join the training set with their fantasies until
+        set_batch_values() supplies the measured values."""
+        q = int(q)
+        if q < 1:
+            raise ValueError("select_batch: q must be >= 1")
+        if self._pending is not None:
+            raise RuntimeError("ActiveMaskGP: the last select_batch() awaits set_batch_values()")
+        if self.n + q > self.cap:
+            raise RuntimeError("ActiveMaskGP capacity exhausted: construct with a larger `capacity`")
+        mu, _, _ = self.posterior()
+        ystats = self._ystats()
+        y = np.asarray(self.y_host)
+        best = float(y.max() if greater_is_better else y.min())
+        ssq0, alive0 = self.ssq.clone(), self.alive.clone()
+        dev, n = self.device, self.n
+        picks = torch.empty(q, dtype=torch.int64, device=dev)
+        ei = torch.empty(q, dtype=torch.float64, device=dev)
+        status = torch.empty(1, dtype=torch.int32, device=dev)
+        ev = [torch.cuda.Event(enable_timing=True) for _ in range(2)]
+        ev[0].record()
+        _lib.check(self.lib.nib_gp_kb_select(self.L.data_ptr(), self.cap, self.V.data_ptr(), self.m, self.ssq.data_ptr(),
+                                             self.alive.data_ptr(), self.cand_d.data_ptr(), self.m, self.words,
+                                             self.X_d.data_ptr(), n, q, mu.data_ptr(), ystats[1], best,
+                                             int(greater_is_better), self.ell, self.alpha, picks.data_ptr(),
+                                             ei.data_ptr(), status.data_ptr(), _lib.stream_handle()), "nib_gp_kb_select")
+        ev[1].record()
+        ev[1].synchronize()
+        self.stats["select_ms"] = ev[0].elapsed_time(ev[1])       # the q picks' kernels, device time
+        picks, ei, status = picks.cpu().numpy(), ei.cpu().numpy(), int(status.item())
+        if status != 0:
+            self.ssq.copy_(ssq0)
+            self.alive.copy_(alive0)
+            raise np.linalg.LinAlgError(f"Kriging-believer pick {status - 1} lost positive definiteness "
+                                        "(duplicate mask with alpha too small?)")
+        p = int(np.count_nonzero(picks >= 0))
+        if p:
+            self.n = n + p
+            self._pending = {"n0": n, "mu": mu, "ystats": ystats}
+        return picks[:p].astype(np.int64), ei[:p].copy()
+
+    def set_batch_values(self, scores):
+        """The measured values of the last select_batch(), in pick order: they replace the fantasies in u = L^-1 y and
+        w = L^-1 1 (rows n0 .. n0+p-1 of L solve L_bb u_b = y_b - L_ba u_a) and join y.  Afterwards posterior() equals a
+        fit from scratch on the grown training set."""
+        if self._pending is None:
+            raise RuntimeError("ActiveMaskGP.set_batch_values: no batch is pending")
+        n0, n = self._pending["n0"], self.n
+        p = n - n0
+        s = np.asarray(scores, dtype=np.float64).reshape(-1)
+        if s.shape[0] != p:
+            raise ValueError(f"set_batch_values: {p} values expected, got {s.shape[0]}")
+        dev, cap = self.device, self.cap
+        rhs = torch.empty(p, 2, dtype=torch.float64, device=dev)
+        rhs[:, 0] = torch.from_numpy(s).to(dev)
+        rhs[:, 1] = 1.0
+        rhs -= self.L[n0:n, :n0] @ self.uw[:, :n0].t()                                 # (y_b, 1) - L_ba (u_a, w_a)
+        Lbb = self.L[n0:, n0:]
+        _lib.check(self.lib.nib_gp_trsm(Lbb.data_ptr(), p, cap, rhs.data_ptr(), 2, 2, 0, _lib.stream_handle()),
+                   "nib_gp_trsm")
+        self.uw[:, n0:n] = rhs.t()
+        self.y_host.extend(float(v) for v in s)
+        self._pending = None
 
 
 def expected_improvement_device(mu: torch.Tensor, sigma: torch.Tensor, best: float, greater_is_better: bool = False):
