@@ -2281,6 +2281,10 @@ template <int BLOCK_N, int STAGES, bool HAS_RES, bool BRES = false, bool SPLIT =
 static int launch_tc3(const TcConvPlan* plan, const TcKernelParams& kp, cudaStream_t st) {
   using SM = Tc3Smem<BLOCK_N, STAGES, HAS_RES, BRES, SPLIT>;
   static_assert(SM::TOTAL <= 232448, "exceeds the 227 KB per-CTA shared memory limit");
+  if (kp.xf_scale != nullptr && (BRES || SPLIT)) {   // no transform warps in these instantiations: never drop the BN-ReLU
+    set_error("tc_dispatch: a pre-activation conv reached a CTA-pair instantiation without the transform role");
+    return NIB_EINVAL;
+  }
   static bool attr_set = false;
   if (!attr_set) {
     NIB_CUDA(cudaFuncSetAttribute(conv_tc3_kernel<BLOCK_N, STAGES, HAS_RES, BRES, SPLIT>,
@@ -2327,9 +2331,15 @@ static int tc_dispatch(const TcConvPlan* plan, const TcKernelParams& kp, int til
     if (plan->im2col == 5 && plan->block_n == 128) return launch_tc3<128, 6, false, true>(plan, kp, st);   // raw rows, 128 out
     if (plan->block_n == 256) return res ? launch_tc3<256, 5, true>(plan, kp, st) : launch_tc3<256, 6, false>(plan, kp, st);
     if (plan->block_n == 128) return res ? launch_tc3<128, 6, true>(plan, kp, st) : launch_tc3<128, 8, false>(plan, kp, st);
-    if (plan->block_n == 64 && !res && kp.n_tiles == 1 && kp.num_k_blocks <= TC3_BRES_KBLOCKS)
-      return launch_tc3<64, 9, false, true>(plan, kp, st);   // resident weights: stem, 56x56 64-channel layers
+    // resident weights: stem, 56x56 64-channel layers.  Not for a pre-activated conv: the BRES instantiation has no
+    // transform warps, so a 64-output BN-ReLU-conv (DenseNet-BC with bn_size * growth == 64) stays on the streamed one
+    if (plan->block_n == 64 && !res && kp.n_tiles == 1 && kp.num_k_blocks <= TC3_BRES_KBLOCKS && kp.xf_scale == nullptr)
+      return launch_tc3<64, 9, false, true>(plan, kp, st);
     if (plan->block_n == 64) return res ? launch_tc3<64, 9, true>(plan, kp, st) : launch_tc3<64, 9, false>(plan, kp, st);
+  }
+  if (kp.xf_scale != nullptr) {
+    set_error("tc_dispatch: a pre-activation conv reached the one-CTA kernel, which has no transform role");
+    return NIB_EINVAL;
   }
   switch (plan->block_n) {
     case 32:  return launch_tc<32, 4>(plan, kp, tiles, st);

@@ -432,8 +432,13 @@ def test_densenet121_bf16(nib):
     x = x * torch.rand(4, 1, 1, 1, generator=torch.Generator().manual_seed(1))
     net, got, want = _check_net(nib, m, x, "bf16", TOL_BF16)
     total, tc = net.launch_counts()
-    # stem + 58 bottleneck 1x1 (BN-ReLU packed into a scratch tensor first) + 58 3x3 + 3 transitions
+    # stem + 58 bottleneck 1x1 (BN-ReLU applied to the A tiles inside the pair kernel) + 58 3x3 + 3 transitions
     assert tc >= 118, f"only {tc} tcgen05 launches for DenseNet-121 (expected 120 convs on the tensor path)"
+    # from the op list: input staging + one launch per op that is not a tcgen05 conv.  A pre-activated conv that fell
+    # back to the pack pass would add one launch of its own
+    kinds = [k for _, k, _, _ in net.profile(4)]
+    assert tc == sum(k == 1 for k in kinds)
+    assert total - tc == 1 + sum(k not in (1, 4) for k in kinds), f"{total - tc} non-tcgen05 launches: a pack pass ran"
 
 
 def test_densenet_cifar_fp32(nib):
