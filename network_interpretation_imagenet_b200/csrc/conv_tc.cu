@@ -10,11 +10,11 @@
 // Both land as a 128 x 64 bf16, 128B-swizzled, K-major tile = one tcgen05.mma operand.
 // Weights are KRSC ([Cout][R*S*Cin], BN folded) and arrive through a second tiled map.
 // Round 2 added three ways of NOT fetching one box per tap (the L2 -> SM port, ~43 B/clk/SM, was the bound of the
-// layers concerned), all in conv_tc3_kernel and selected by TcKernelParams::im2col:
-//   * mode 4: 3x3 stride-1 pad-1 convs with 64 -> 64, 64 -> 32 or 128 -> 32 channels read ONE resident input patch per
+// layers concerned), all in conv_tc3_kernel and selected by TcKernelParams::a_mode:
+//   * TC_A_HALO: 3x3 stride-1 pad-1 convs with 64 -> 64, 64 -> 32 or 128 -> 32 channels read ONE resident input patch per
 //     tile (whole image rows in the raster of the padded width); tap (dy, dx) is the same swizzled operand started
 //     (dy * Wp + dx) rows further on (descriptor base offset 0: the swizzle phase is address-based);
-//   * mode 5: the 7x7 stride-2 stem reads the raw padded input rows through an UNSWIZZLED descriptor whose rows
+//   * TC_A_RAW: the 7x7 stride-2 stem reads the raw padded input rows through an UNSWIZZLED descriptor whose rows
 //     overlap (row pitch 16 B = the stride-2 window over 8-byte pixels); a 3x3 stride-1 first conv on 16-byte pixels
 //     (VGG's conv1_1) reads its three rows the same way (row pitch 16 B = one pixel);
 //   * pre-activation 1x1 convs (DenseNet): four extra warps apply relu(x * scale + shift) to every A tile in shared
@@ -39,6 +39,7 @@
 #include <cuda.h>
 #include <string.h>
 #include <stdlib.h>
+#include <memory>
 
 namespace nib {
 
@@ -46,6 +47,16 @@ static constexpr int TC_BLOCK_M = 128;
 static constexpr int TC_BLOCK_K = 64;   // 64 bf16 = 128 B = one swizzle row
 static constexpr int TC_UMMA_K = 16;
 static constexpr int TC_THREADS = 192;
+
+// How the A operand (the activations) reaches shared memory: TcKernelParams::a_mode.
+enum TcAMode : int {
+  TC_A_DENSE = 0,    // tiled 2D map over the NHWC activation matrix (1x1 stride-1 convs, the GEMM self-test)
+  TC_A_IM2COL = 1,   // TMA im2col 4D map, one box per filter tap
+  TC_A_STEM8 = 2,    // stem rows: overlapping-window 4D tiled map over 8-channel pixels, one filter row per K block
+  TC_A_STEM4 = 3,    // stem row PAIRS over 4-channel pixels (CTA-pair kernel only)
+  TC_A_HALO = 4,     // one resident input patch per tile (3x3 stride 1)
+  TC_A_RAW = 5,      // raw padded input rows through an unswizzled descriptor with overlapping rows
+};
 
 struct TcKernelParams {
   const float* bias;
@@ -60,8 +71,7 @@ struct TcKernelParams {
   int num_k_blocks;
   int cblocks;      // Cin / 64
   int S;            // filter width (tap -> (r, s))
-  int im2col;       // 0: tiled 2D A map, 1: im2col 4D A map, 2: stem rows (overlapping-window 4D tiled map, 8-channel
-                    // pixels, one filter row per K block), 3: stem row PAIRS (5D map, 4-channel pixels, v3 only)
+  int a_mode;       // TcAMode
   int tile_rows;    // valid output rows per M tile (128; Q for the stem mode: one output row per tile)
   int a_bytes;      // bytes the A load delivers per stage (tile_rows * 128)
   int P, Q, stride, pad;
@@ -77,7 +87,7 @@ struct TcKernelParams {
   int lo_off_res;            // ... and in the residual tensor
   const int* dyn_n;          // split mode: optional device-side live image count (the tie policy's re-score batch); tiles
                              // beyond live * P * Q rows are not computed
-  // im2col == 4 (3x3 stride-1 pad-1, 64 -> 64 channels): an M tile is halo_r whole image rows in the raster of the PADDED
+  // TC_A_HALO (3x3 stride-1 pad-1, 64 -> 64 channels): an M tile is halo_r whole image rows in the raster of the PADDED
   // width halo_wp = Q + 2; the (halo_r + 2) x halo_wp input patch is loaded once and all nine taps read it at shifted
   // start addresses
   int halo_wp, halo_r, halo_tpi;   // padded width, image rows per tile, tiles per image
@@ -88,8 +98,8 @@ struct TcKernelParams {
   // channels past Cin become exact zeros whatever the concat buffer holds there)
   const float* xf_scale;
   const float* xf_shift;
-  int halo_swap;                   // im2col == 5 diagnostics: swap the LBO / SBO roles of the unswizzled descriptor
-  // im2col == 5 (raw input rows): filter rows per tile (7: the 7x7/2 stem, 3: a 3x3/1 first conv) and column tiles per
+  int halo_swap;                   // TC_A_RAW diagnostics: swap the LBO / SBO roles of the unswizzled descriptor
+  // TC_A_RAW (raw input rows): filter rows per tile (7: the 7x7/2 stem, 3: a 3x3/1 first conv) and column tiles per
   // output row (1 unless the row is wider than the 128-row M tile).  Pair tile mp holds output rows 2 (mp / col_tiles) and
   // 2 (mp / col_tiles) + 1 (one per CTA) in the SAME column tile mp % col_tiles, so both CTAs' A operands start at the same
   // shared-memory offset: the leader's descriptor addresses both.
@@ -201,7 +211,7 @@ __device__ __forceinline__ uint64_t make_smem_desc_sw128(uint32_t smem_addr) {
 
 // K-major, unswizzled: core matrices of 8 rows x 16 B (128 contiguous bytes); lbo = distance between core matrices along K,
 // sbo = between 8-row groups.  With lbo = 16 and sbo = 128 row r starts 16 r bytes into the buffer and its K run simply
-// continues: overlapping rows, which is exactly a stride-2 window over 8-byte pixels (the stem, im2col mode 5).
+// continues: overlapping rows, which is exactly a stride-2 window over 8-byte pixels (the stem, TC_A_RAW).
 __device__ __forceinline__ uint64_t make_smem_desc_nosw(uint32_t smem_addr, uint32_t lbo, uint32_t sbo) {
   uint64_t d = 0;
   d |= (uint64_t)((smem_addr >> 4) & 0x3FFF);
@@ -285,14 +295,14 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     if (lane == 0) {
       // ===== TMA producer =====
       int w0 = 0, h0 = 0, img = 0;
-      if (p.im2col == 1) {
+      if (p.a_mode == TC_A_IM2COL) {
         const int pq = p.P * p.Q;
         img = m0 / pq;
         const int rem = m0 - img * pq;
         const int pp = rem / p.Q, qq = rem - pp * p.Q;
         w0 = qq * p.stride - p.pad;
         h0 = pp * p.stride - p.pad;
-      } else if (p.im2col == 2) {   // one output row (img, pp) per tile; input rows pp*stride + r of the haloed image
+      } else if (p.a_mode == TC_A_STEM8) {   // one output row (img, pp) per tile; input rows pp*stride + r of the haloed image
         img = m_tile / p.P;
         h0 = (m_tile - img * p.P) * p.stride;
       }
@@ -305,10 +315,10 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         mbar_arrive_expect_tx(full_bar(stage), (uint32_t)(p.a_bytes + SM::B_BYTES));
         const int tap = kb / p.cblocks;
         const int c0 = (kb - tap * p.cblocks) * TC_BLOCK_K + p.in_coff;
-        if (p.im2col == 1) {
+        if (p.a_mode == TC_A_IM2COL) {
           const int r = tap / p.S, s = tap - r * p.S;
           tma_load_im2col_4d(a_dst, &tmA, full_bar(stage), c0, w0, h0, img, (uint16_t)s, (uint16_t)r);
-        } else if (p.im2col == 2) {
+        } else if (p.a_mode == TC_A_STEM8) {
           tma_load_4d(a_dst, &tmA, full_bar(stage), 0, 0, h0 + kb, img);   // k-block kb = filter row r
         } else {
           tma_load_2d(a_dst, &tmA, full_bar(stage), c0, m0);
@@ -694,7 +704,7 @@ conv_tc3_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
     asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tmem_slot), "r"(TMEM_COLS) : "memory");
     asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
   }
-  if (p.im2col == 5 && p.stride == 1) {
+  if (p.a_mode == TC_A_RAW && p.stride == 1) {
     // 3x3 raw rows: the last output pixel's zero-weight filler tap reads the 16 bytes just past the third row, which no
     // TMA load ever writes.  Zero the ring once so that 0 * (whatever the SM held before) cannot inject a NaN.
     for (uint32_t off = 16u * threadIdx.x; off < (uint32_t)(STAGES * SM::STAGE_BYTES); off += 16u * blockDim.x)
@@ -722,7 +732,7 @@ conv_tc3_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
     int it = 0;
     const uint32_t lbar0 = mapa_shared(full_bar(0), 0);   // leader CTA's full barriers
     const uint32_t tx_bytes = (uint32_t)(2 * ((xform ? 0 : p.a_bytes) + (BRES ? 0 : SM::BH_BYTES)));
-    const int b_row0 = (int)rank * ((BRES && p.im2col == 4 ? p.halo_n : BLOCK_N) / 2);
+    const int b_row0 = (int)rank * ((BRES && p.a_mode == TC_A_HALO ? p.halo_n : BLOCK_N) / 2);
     // residual boxes of the previous tile still to be requested: they are issued opportunistically while this
     // tile's operands stream (a box frees up when the epilogue's store of the tile before has drained), so a
     // busy epilogue never stalls the operand ring
@@ -751,11 +761,11 @@ conv_tc3_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
     if (BRES) {   // both CTAs fetch their half of every K block of the weights once
       if (elect_one()) {
         const uint32_t lb = mapa_shared(bres_full_bar, 0);
-        const uint32_t bhb = p.im2col == 4 ? (uint32_t)(p.halo_n * 64) : (uint32_t)SM::BH_BYTES;   // halo_n / 2 rows x 128 B
+        const uint32_t bhb = p.a_mode == TC_A_HALO ? (uint32_t)(p.halo_n * 64) : (uint32_t)SM::BH_BYTES;   // halo_n / 2 rows x 128 B
         if (rank == 0) mbar_arrive_expect_tx(bres_full_bar, (uint32_t)(2 * p.num_k_blocks) * bhb);
         for (int kb = 0; kb < p.num_k_blocks; ++kb) {
           const uint32_t dst = smem_base + SM::BRES_OFFSET + kb * bhb;
-          if (p.im2col == 3 || p.im2col == 5) {   // 64B-swizzled: the K block is two 32-element atoms
+          if (p.a_mode == TC_A_STEM4 || p.a_mode == TC_A_RAW) {   // 64B-swizzled: the K block is two 32-element atoms
             tma2_load_2d(dst, &tmB, lb, kb * TC_BLOCK_K, b_row0);
             tma2_load_2d(dst + SM::BH_BYTES / 2, &tmB, lb, kb * TC_BLOCK_K + 32, b_row0);
           } else {
@@ -769,22 +779,22 @@ conv_tc3_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
       const int n_tile = tile % p.n_tiles;
       const int mp = tile / p.n_tiles;
       // raw rows: m_tile is the output row (image-major); the tile covers column tile mp % col_tiles of it
-      const int m_tile = p.im2col == 5 ? (mp / p.col_tiles) * 2 + (int)rank : mp * 2 + (int)rank;
-      const int m0 = p.im2col == 5 ? (m_tile * p.col_tiles + mp % p.col_tiles) * p.tile_rows : m_tile * p.tile_rows;
+      const int m_tile = p.a_mode == TC_A_RAW ? (mp / p.col_tiles) * 2 + (int)rank : mp * 2 + (int)rank;
+      const int m0 = p.a_mode == TC_A_RAW ? (m_tile * p.col_tiles + mp % p.col_tiles) * p.tile_rows : m_tile * p.tile_rows;
       const int n0 = n_tile * BLOCK_N;
       int w0 = 0, h0 = 0, img = 0;
-      if (p.im2col == 1) {
+      if (p.a_mode == TC_A_IM2COL) {
         const int pq = p.P * p.Q;
         img = m0 / pq;
         const int rem = m0 - img * pq;
         const int pp = rem / p.Q, qq = rem - pp * p.Q;
         w0 = qq * p.stride - p.pad;
         h0 = pp * p.stride - p.pad;
-      } else if (p.im2col >= 2) {
+      } else if (p.a_mode >= TC_A_STEM8) {
         img = m_tile / p.P;
         h0 = (m_tile - img * p.P) * p.stride;
       }
-      if (BRES && !HAS_RES && p.im2col == 4) {
+      if (BRES && !HAS_RES && p.a_mode == TC_A_HALO) {
         // halo patch: ONE 4D tiled load per tile (rows y0-1 .. y0+halo_r, columns -1 .. Q; out-of-range coordinates are
         // zero-filled = the convolution's padding) into one of four 32 KB buffers (ring stages 0, 2, 4, 6)
         // (two 32 KB blocks per buffer and two buffers when Cin = 128)
@@ -801,7 +811,7 @@ conv_tc3_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
         __syncwarp();
         continue;
       }
-      if (BRES && !HAS_RES && p.im2col == 5) {
+      if (BRES && !HAS_RES && p.a_mode == TC_A_RAW) {
         // the padded input rows under one output row (7 for the stem, 3 for a 3x3 conv), raw, one ring stage per tile
         TC3_TIMED(0, mbar_wait(empty_bar(stage), phase ^ 1u, p.err_flag, 1));
         if (elect_one()) {
@@ -822,11 +832,11 @@ conv_tc3_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
           if (rank == 0) mbar_arrive_expect_tx(full_bar(stage), tx_bytes);
           const int ca = SPLIT ? (cb >= p.a_wrap ? cb - p.a_wrap : cb) : cb;   // split mode: hi, lo, hi again
           const int c0 = ca * TC_BLOCK_K + p.in_coff;
-          if (p.im2col == 1) {
+          if (p.a_mode == TC_A_IM2COL) {
             tma2_load_im2col_4d(a_dst, &tmA, lbar, c0, w0, h0, img, (uint16_t)tap_s, (uint16_t)tap_r);
-          } else if (p.im2col == 2) {
+          } else if (p.a_mode == TC_A_STEM8) {
             tma2_load_4d(a_dst, &tmA, lbar, 0, 0, h0 + kb, img);
-          } else if (p.im2col == 3) {
+          } else if (p.a_mode == TC_A_STEM4) {
             // K block kb = filter rows 2kb, 2kb+1: two 64B-swizzled K atoms of [Q rows x 32 elements]
             tma2_load_4d(a_dst, &tmA, lbar, 0, 0, h0 + 2 * kb, img);
             tma2_load_4d(a_dst + SM::A_BYTES / 2, &tmA, lbar, 0, 0, h0 + 2 * kb + 1, img);
@@ -873,7 +883,7 @@ conv_tc3_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
         TC3_TIMED(1, mbar_wait(tmem_empty_bar(ab), (uint32_t)(((it >> 1) & 1) ^ 1), p.err_flag, 5));
         tc_fence_after();
         const uint32_t d_tmem = tmem_base + (uint32_t)(ab * BLOCK_N);
-        if (BRES && !HAS_RES && p.im2col == 4) {
+        if (BRES && !HAS_RES && p.a_mode == TC_A_HALO) {
           // nine taps out of one resident patch: tap (dy, dx) is the same 128-row operand started (dy * Wp + dx) pixels
           // = that many 128 B swizzle rows further on.  The tensor core derives the swizzle phase from the absolute
           // shared-memory address, like the copy engine that wrote the patch, so a start that is not a multiple of 8 rows
@@ -904,7 +914,7 @@ conv_tc3_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
           __syncwarp();
           continue;
         }
-        if (BRES && !HAS_RES && p.im2col == 5) {
+        if (BRES && !HAS_RES && p.a_mode == TC_A_RAW) {
           // stem on raw input rows: output pixel q of filter row r reads 32 elements (8 taps x 4 channels) starting at
           // pixel 2q of input row 2p + r, i.e. 16 q bytes into that row - an unswizzled K-major operand whose rows
           // OVERLAP (row pitch 16 B, K chunk pitch 16 B).  Each input byte crosses L2 -> SM once per output row instead
@@ -943,7 +953,7 @@ conv_tc3_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
           if (elect_one()) {
             const uint32_t a_addr = smem_base + stage * SM::STAGE_BYTES;
             const uint32_t b_addr = BRES ? smem_base + SM::BRES_OFFSET + kb * SM::BH_BYTES : a_addr + SM::A_BYTES;
-            if (BRES && p.im2col == 3) {
+            if (BRES && p.a_mode == TC_A_STEM4) {
               // 64B-swizzled operands: K atom a (32 elements) at +a * half the tile, 16-element step inside it = +32 B
 #pragma unroll
               for (int k = 0; k < TC_BLOCK_K / TC_UMMA_K; ++k) {
@@ -1036,7 +1046,7 @@ conv_tc3_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
     // With ~225 KB of the SM carved out as shared memory there is no L1 to speak of: the tile's bias slice is fetched
     // one tile ahead into a register, parked in smem and read back as broadcast LDS.128.
     // halo mode: TMEM lane i is raster position i of the padded-width tile; its dense output row (junk columns dropped)
-    const bool halo = BRES && !HAS_RES && !SPLIT && p.im2col == 4;
+    const bool halo = BRES && !HAS_RES && !SPLIT && p.a_mode == TC_A_HALO;
     bool halo_valid = false;
     uint32_t halo_base = 0, halo_sw = 0;
     if (halo) {
@@ -1053,14 +1063,14 @@ conv_tc3_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
       }
     }
     float bias_pre = 0.f;
-    const int bias_cols = (BRES && p.im2col == 4) ? p.halo_n : SM::CW;   // the resident-patch mode may have only 32 outputs
+    const int bias_cols = (BRES && p.a_mode == TC_A_HALO) ? p.halo_n : SM::CW;   // the resident-patch mode may have only 32 outputs
     if (has_bias && wt < bias_cols && tile < total_tiles) bias_pre = __ldg(p.bias + (tile % p.n_tiles) * BLOCK_N + colbase + wt);
     if (dbg_on) t_loop0 = clock64();
     for (; tile < total_tiles; tile += step, it += (SM::SPLIT_COLS ? 1 : 2), ++lt) {
       const int n_tile = tile % p.n_tiles;
       const int mp = tile / p.n_tiles;
-      const int m_tile = p.im2col == 5 ? (mp / p.col_tiles) * 2 + (int)rank : mp * 2 + (int)rank;
-      const int m0 = p.im2col == 5 ? (m_tile * p.col_tiles + mp % p.col_tiles) * p.tile_rows : m_tile * p.tile_rows;
+      const int m_tile = p.a_mode == TC_A_RAW ? (mp / p.col_tiles) * 2 + (int)rank : mp * 2 + (int)rank;
+      const int m0 = p.a_mode == TC_A_RAW ? (m_tile * p.col_tiles + mp % p.col_tiles) * p.tile_rows : m_tile * p.tile_rows;
       const int n0 = n_tile * BLOCK_N;
       const int ab = it & 1;
       TC3_TIMED(0, mbar_wait(tmem_full_bar(ab), (uint32_t)((it >> 1) & 1), p.err_flag, 3));
@@ -1667,20 +1677,29 @@ typedef CUresult (*PFN_encodeIm2col)(CUtensorMap*, CUtensorMapDataType, cuuint32
                                      CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 static PFN_encodeTiled g_encodeTiled = nullptr;
 static PFN_encodeIm2col g_encodeIm2col = nullptr;
+static unsigned int* g_err_flag = nullptr;
 
-static int load_driver_fns() {
-  if (g_encodeTiled && g_encodeIm2col) return NIB_OK;
-  cudaDriverEntryPointQueryResult q;
-  void* fn = nullptr;
-  NIB_CUDA(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &q));
-  if (q != cudaDriverEntryPointSuccess || !fn) { set_error("cuTensorMapEncodeTiled not available"); return NIB_ECUDA; }
-  g_encodeTiled = (PFN_encodeTiled)fn;
-  fn = nullptr;
-  NIB_CUDA(cudaGetDriverEntryPoint("cuTensorMapEncodeIm2col", &fn, cudaEnableDefault, &q));
-  if (q != cudaDriverEntryPointSuccess || !fn) { set_error("cuTensorMapEncodeIm2col not available"); return NIB_ECUDA; }
-  g_encodeIm2col = (PFN_encodeIm2col)fn;
+// driver entry points for the tensor maps and the kernels' shared error flag
+static int init_tc() {
+  if (!g_encodeTiled || !g_encodeIm2col) {
+    cudaDriverEntryPointQueryResult q;
+    void* fn = nullptr;
+    NIB_CUDA(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &q));
+    if (q != cudaDriverEntryPointSuccess || !fn) { set_error("cuTensorMapEncodeTiled not available"); return NIB_ECUDA; }
+    g_encodeTiled = (PFN_encodeTiled)fn;
+    fn = nullptr;
+    NIB_CUDA(cudaGetDriverEntryPoint("cuTensorMapEncodeIm2col", &fn, cudaEnableDefault, &q));
+    if (q != cudaDriverEntryPointSuccess || !fn) { set_error("cuTensorMapEncodeIm2col not available"); return NIB_ECUDA; }
+    g_encodeIm2col = (PFN_encodeIm2col)fn;
+  }
+  if (!g_err_flag) {
+    NIB_CUDA(cudaMalloc(&g_err_flag, sizeof(unsigned int)));
+    NIB_CUDA(cudaMemset(g_err_flag, 0, sizeof(unsigned int)));
+  }
   return NIB_OK;
 }
+
+typedef int (*TcLauncher)(const TcConvPlan* plan, const TcKernelParams& kp, cudaStream_t st);
 
 struct TcConvPlan {
   CUtensorMap tmA, tmB, tmOut, tmRes;
@@ -1688,44 +1707,61 @@ struct TcConvPlan {
   CUtensorMap tmOut32, tmOutTail;   // pair kernel: per-warp 32-row output boxes (+ the short last box of a 112-row stem tile)
   int v3;             // 1: the CTA-pair kernel serves this layer; 0: the one-CTA kernel (Cout = 32, NIB_TC_V1)
   int split;          // split-bf16 tensors: K = 3 x Cin per tap, both halves of the result are stored
-  int block_n, stages;
-  int im2col;
-  int tile_rows;
-  int num_k_blocks, cblocks;
-  int halo_wp, halo_r, halo_tpi, halo_cb, halo_n;   // im2col == 4
-  int raw_rows, col_tiles;                          // im2col == 5
-  unsigned int* err_flag;
+  int block_n;
+  TcKernelParams kp;  // every launch parameter except the batch-dependent M, m_tiles and dyn_n (tc_conv_launch)
+  TcLauncher launch;  // the kernel instance (pick_instance)
 };
 
-static unsigned int* g_err_flag = nullptr;
-
-static int encode_2d_bf16(CUtensorMap* tm, const void* ptr, uint64_t inner, uint64_t outer, uint64_t row_bytes,
-                          uint32_t box_inner, uint32_t box_outer) {
-  cuuint64_t dims[2] = {inner, outer};
-  cuuint64_t strides[1] = {row_bytes};
-  cuuint32_t box[2] = {box_inner, box_outer};
-  cuuint32_t es[2] = {1, 1};
-  CUresult r = g_encodeTiled(tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(ptr), dims, strides, box, es,
-                             CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-                             CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+static int encode_tiled_bf16(CUtensorMap* tm, const void* ptr, int rank, const cuuint64_t* dims, const cuuint64_t* strides,
+                             const cuuint32_t* box, CUtensorMapSwizzle swizzle) {
+  const cuuint32_t es[4] = {1, 1, 1, 1};
+  CUresult r = g_encodeTiled(tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, rank, const_cast<void*>(ptr), dims, strides, box, es,
+                             CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) {
-    set_error("cuTensorMapEncodeTiled failed (%d): dims=(%llu,%llu) row_bytes=%llu box=(%u,%u) ptr=%p", (int)r,
-              (unsigned long long)inner, (unsigned long long)outer, (unsigned long long)row_bytes, box_inner,
-              box_outer, ptr);
+    set_error("cuTensorMapEncodeTiled failed (%d): rank %d dims=(%llu,%llu,...) box=(%u,%u,...) swizzle %d ptr=%p", (int)r,
+              rank, (unsigned long long)dims[0], (unsigned long long)dims[1], box[0], box[1], (int)swizzle, ptr);
     return NIB_ECUDA;
   }
   return NIB_OK;
+}
+
+static int encode_2d_bf16(CUtensorMap* tm, const void* ptr, uint64_t inner, uint64_t outer, uint64_t row_bytes,
+                          uint32_t box_inner, uint32_t box_outer, CUtensorMapSwizzle swizzle = CU_TENSOR_MAP_SWIZZLE_128B) {
+  const cuuint64_t dims[2] = {inner, outer};
+  const cuuint64_t strides[1] = {row_bytes};
+  const cuuint32_t box[2] = {box_inner, box_outer};
+  return encode_tiled_bf16(tm, ptr, 2, dims, strides, box, swizzle);
+}
+
+// dims {inner, ..., outer}; strides in bytes of dims 1..3
+static int encode_4d_bf16(CUtensorMap* tm, const void* ptr, const cuuint64_t (&dims)[4], const cuuint64_t (&strides)[3],
+                          const cuuint32_t (&box)[4], CUtensorMapSwizzle swizzle) {
+  return encode_tiled_bf16(tm, ptr, 4, dims, strides, box, swizzle);
+}
+
+RawRowLayout tc_raw_row_layout(int R, int S, int stride, int pad, int Cin, int in_cstride, int in_halo) {
+  if (R == 7 && S == 7 && stride == 2 && pad == 3 && in_halo == 3) {
+    if (in_cstride == 8 && Cin <= 8) return {7, 8, 8};   // stem on 8-channel pixels: a K block is one filter row
+    if (in_cstride == 4 && Cin <= 4) return {8, 8, 4};   // on 4-channel pixels: two filter rows per K block, row 7 zero
+  }
+  if (R == 3 && S == 3 && stride == 1 && pad == 1 && in_halo == 1 && in_cstride == 8 && Cin <= 8)
+    return {4, 4, 8};                                   // 3x3 first conv: a 32-element K atom per filter row, row 3 zero
+  return {0, 0, 0};
+}
+
+static RawRowLayout raw_row_layout(const ConvParams& p) {
+  return tc_raw_row_layout(p.R, p.S, p.stride, p.pad, p.Cin, p.in_cstride, p.in_halo);
 }
 
 // 7x7 stride-2 pad-3 stem on a haloed, 8-channel-padded NHWC input (torchvision conv1): for filter row r the 7 taps x 8
 // channels of output pixel q are 56 contiguous elements starting at pixel 2q of input row 2p+r, so a tiled map whose
 // pixel dimension advances 2 pixels (32 B) per index delivers a [Q x 64] K-major tile per filter row (8 zero-weight
 // filler elements).  K = 7 x 64.
-bool tc_conv_is_stem(const ConvParams& p) {
-  return p.R == 7 && p.S == 7 && p.stride == 2 && p.pad == 3 && p.Cin <= 8 && p.in_cstride == 8 && p.in_coff == 0 &&
-         p.in_halo == 3 && p.Cout % 32 == 0 && p.Q <= TC_BLOCK_M && p.out_halo == 0 && p.out_cstride % 8 == 0 &&
-         p.out_coff % 8 == 0 && p.pre_scale == nullptr && p.res == nullptr && p.w_alt != nullptr &&
-         (p.Win + 2 * p.in_halo) >= 2 * (p.Q - 1) + 8;
+static bool tc_conv_is_stem(const ConvParams& p) {
+  return raw_row_layout(p).rows == 7 && p.in_coff == 0 && p.Cout % 32 == 0 && p.Q <= TC_BLOCK_M && p.out_halo == 0 &&
+         p.out_cstride % 8 == 0 && p.out_coff % 8 == 0 && p.pre_scale == nullptr && p.res == nullptr &&
+         p.w_alt != nullptr && (p.Win + 2 * p.in_halo) >= 2 * (p.Q - 1) + 8;
 }
 
 // Same stem on 4-channel-padded pixels (8 B): a K block is TWO filter rows x (7 taps + 1 filler) x 4 channels.  Each
@@ -1733,9 +1769,8 @@ bool tc_conv_is_stem(const ConvParams& p) {
 // padded to 128 B rows by the copy engine, measured with tools/stem_diag.py, hence SWIZZLE_64B + matching UMMA
 // descriptors).  K = 4 x 64 instead of 7 x 64: 43 % fewer activation bytes through the TMA and 43 % fewer MMAs.
 // CTA-pair kernel with resident weights only.
-bool tc_conv_is_stem4(const ConvParams& p) {
-  return p.R == 7 && p.S == 7 && p.stride == 2 && p.pad == 3 && p.Cin <= 4 && p.in_cstride == 4 &&
-         p.in_coff == 0 && p.in_halo == 3 && p.Cout % 64 == 0 && p.Q <= TC_BLOCK_M && p.out_halo == 0 &&
+static bool tc_conv_is_stem4(const ConvParams& p) {
+  return raw_row_layout(p).rows == 8 && p.in_coff == 0 && p.Cout % 64 == 0 && p.Q <= TC_BLOCK_M && p.out_halo == 0 &&
          p.out_cstride % 8 == 0 && p.out_coff % 8 == 0 && p.pre_scale == nullptr && p.res == nullptr &&
          p.w_alt != nullptr && (p.Win + 2 * p.in_halo) % 2 == 0 && (p.Win + 2 * p.in_halo) >= 2 * (p.Q - 1) + 8 &&
          (p.Hin + 2 * p.in_halo) >= 2 * (p.P - 1) + 8;
@@ -1758,17 +1793,15 @@ static int raw3x3_col_tiles(int Q) {
   return 0;
 }
 
-// 3x3 stride-1 pad-1 first conv (VGG conv1_1) on 8-channel-padded pixels (16 B) inside a 1-pixel zero halo, im2col mode 5:
+// 3x3 stride-1 pad-1 first conv (VGG conv1_1) on 8-channel-padded pixels (16 B) inside a 1-pixel zero halo, TC_A_RAW:
 // output pixel q of filter row r reads 3 taps x 8 channels starting at pixel q of padded row p + r, so each filter row is
 // one 32-element K atom (3 taps + a zero-weight filler tap) of the overlapping-row operand the stem uses; K = 3 x 32, six
 // MMAs per tile.  Weights [Cout][4][32] (row 3 zero), resident; Cout 64 or 128 (the resident-weight pair kernel holds one
 // N tile).  The three rows of one image row (plus the filler's 16 B) must fit one 16 KB ring stage.
-bool tc_conv_is_raw3x3(const ConvParams& p) {
+static bool tc_conv_is_raw3x3(const ConvParams& p) {
   static const bool off = getenv("NIB_TC_NO_HALO") != nullptr;
   if (off || p.split) return false;
-  if (!(p.R == 3 && p.S == 3 && p.stride == 1 && p.pad == 1 && p.Cin <= 8 && p.in_cstride == 8 && p.in_coff == 0 &&
-        p.in_halo == 1))
-    return false;
+  if (raw_row_layout(p).rows != 4 || p.in_coff != 0) return false;
   if (!(p.Cout == 64 || p.Cout == 128) || p.out_halo != 0 || p.out_cstride % 8 != 0 || p.out_coff % 8 != 0) return false;
   if (p.pre_scale != nullptr || p.res != nullptr || p.w_alt == nullptr || p.P != p.Hin || p.Q != p.Win) return false;
   const int t = raw3x3_col_tiles(p.Q);
@@ -1791,7 +1824,7 @@ static int halo_rows_per_tile(int H, int Wp) {
     if (H % r == 0) return r;
   return 0;
 }
-bool tc_conv_is_halo3x3(const ConvParams& p) {
+static bool tc_conv_is_halo3x3(const ConvParams& p) {
   static const bool off = getenv("NIB_TC_NO_HALO") != nullptr;
   if (off || p.split) return false;
   if (!(p.R == 3 && p.S == 3 && p.stride == 1 && p.pad == 1)) return false;
@@ -1842,6 +1875,7 @@ static int pick_block_n(int Cout) {
   return 32;
 }
 
+// the CTA-pair kernel's output, residual and half-width weight maps; leaves v3 = 0 (one-CTA kernel) where it does not apply
 static int finish_plan(TcConvPlan* plan, const ConvParams& p, int max_batch, const void* w_ptr, int K) {
   plan->v3 = 0;
   static const bool v1_only = getenv("NIB_TC_V1") != nullptr;   // debugging aid: everything on the one-CTA kernel
@@ -1849,8 +1883,9 @@ static int finish_plan(TcConvPlan* plan, const ConvParams& p, int max_batch, con
   const bool bn_ok = plan->block_n == 64 || plan->block_n == 128 || plan->block_n == 256;
   if (!bn_ok || p.Cout % plan->block_n != 0) return NIB_OK;
   const uint64_t rows = (uint64_t)max_batch * p.P * p.Q;
+  const int tile_rows = plan->kp.tile_rows;
   int rc = encode_2d_bf16(&plan->tmOut, p.out, (uint64_t)p.out_cstride, rows, (uint64_t)p.out_cstride * 2, 64,
-                          (uint32_t)plan->tile_rows);
+                          (uint32_t)tile_rows);
   if (rc != NIB_OK) return rc;
   if (p.res != nullptr) {
     rc = encode_2d_bf16(&plan->tmRes, p.res, (uint64_t)p.res_cstride, rows, (uint64_t)p.res_cstride * 2, 64, TC_BLOCK_M);
@@ -1863,7 +1898,7 @@ static int finish_plan(TcConvPlan* plan, const ConvParams& p, int max_batch, con
   if (rc != NIB_OK) return rc;
   rc = encode_2d_bf16(&plan->tmOut32, p.out, (uint64_t)p.out_cstride, rows, (uint64_t)p.out_cstride * 2, 64, 32);
   if (rc != NIB_OK) return rc;
-  const int tail = plan->tile_rows % 32;
+  const int tail = tile_rows % 32;
   rc = encode_2d_bf16(&plan->tmOutTail, p.out, (uint64_t)p.out_cstride, rows, (uint64_t)p.out_cstride * 2, 64,
                       (uint32_t)(tail ? tail : 32));
   if (rc != NIB_OK) return rc;
@@ -1871,219 +1906,133 @@ static int finish_plan(TcConvPlan* plan, const ConvParams& p, int max_batch, con
   return NIB_OK;
 }
 
-int tc_conv_plan_create(const ConvParams& p, int max_batch, TcConvPlan** out) {
-  int rc = load_driver_fns();
-  if (rc != NIB_OK) return rc;
-  if (!g_err_flag) {
-    NIB_CUDA(cudaMalloc(&g_err_flag, sizeof(unsigned int)));
-    NIB_CUDA(cudaMemset(g_err_flag, 0, sizeof(unsigned int)));
-  }
-  TcConvPlan* plan = new TcConvPlan();
-  memset(plan, 0, sizeof(*plan));
-  plan->err_flag = g_err_flag;
-  plan->block_n = pick_block_n(p.Cout);
-  plan->tile_rows = TC_BLOCK_M;
+// resident raw-row weights [Cout][K] as 64B-swizzled K atoms of 32 elements, BLOCK_N/2 rows per CTA, for both kernels
+// (replaces finish_plan's map)
+static int encode_raw_row_weights(TcConvPlan* plan, const ConvParams& p, int K) {
+  int rc = encode_2d_bf16(&plan->tmBh, p.w_alt, (uint64_t)K, (uint64_t)p.Cout, (uint64_t)K * 2, 32,
+                          (uint32_t)(plan->block_n / 2), CU_TENSOR_MAP_SWIZZLE_64B);
+  plan->tmB = plan->tmBh;
+  return rc;
+}
+
+// The A operand's tensor map and the mode's tile geometry (kp.a_mode, cblocks, num_k_blocks, tile_rows, a_bytes and the
+// resident-patch / raw-row fields), then the weight and output maps.
+static int build_maps(TcConvPlan* plan, const ConvParams& p, int max_batch) {
+  TcKernelParams& kp = plan->kp;
+  int rc;
   if (tc_conv_is_stem4(p)) {
-    plan->im2col = 3;
-    plan->cblocks = 1;
-    plan->num_k_blocks = 4;
-    plan->tile_rows = p.Q;
+    const int K = raw_row_layout(p).k();
+    kp.a_mode = TC_A_STEM4;
+    kp.cblocks = 1;
+    kp.num_k_blocks = K / TC_BLOCK_K;
+    kp.tile_rows = p.Q;
+    kp.a_bytes = kp.tile_rows * TC_BLOCK_K * 2;
     const int Hp = p.Hin + 6, Wp = p.Win + 6;
-    // raw-row mode (5): the padded row (Wp pixels x 4 channels) as inner x outer with a TMA-legal inner extent
+    // raw-row mode: the padded row (Wp pixels x 4 channels) as inner x outer with a TMA-legal inner extent
     int inner = 0;
     {
       static const bool off = getenv("NIB_TC_NO_HALO") != nullptr;
       if (!off && 6 * Wp * 8 + 16 * 127 + 64 <= 16384) inner = raw_row_inner(Wp * 4);
     }
     if (inner > 0) {
-      plan->im2col = 5;
-      plan->raw_rows = 7;
-      plan->col_tiles = 1;
-      plan->halo_wp = Wp * 8;
-      cuuint64_t dims[4] = {(cuuint64_t)inner, (cuuint64_t)(Wp * 4 / inner), (cuuint64_t)Hp, (cuuint64_t)max_batch};
-      cuuint64_t strides[3] = {(cuuint64_t)inner * 2, (cuuint64_t)Wp * 8, (cuuint64_t)Hp * Wp * 8};
-      cuuint32_t box[4] = {(cuuint32_t)inner, (cuuint32_t)(Wp * 4 / inner), 7, 1};
-      cuuint32_t es[4] = {1, 1, 1, 1};
-      CUresult r = g_encodeTiled(&plan->tmA, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(p.in), dims, strides,
-                                 box, es, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
-                                 CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-      if (r != CUDA_SUCCESS) {
-        set_error("cuTensorMapEncodeTiled (stem, raw rows) failed (%d)", (int)r);
-        delete plan;
-        return NIB_ECUDA;
-      }
+      kp.a_mode = TC_A_RAW;
+      kp.raw_rows = 7;
+      kp.col_tiles = 1;
+      kp.halo_wp = Wp * 8;
+      kp.a_bytes = kp.raw_rows * kp.halo_wp;
+      rc = encode_4d_bf16(&plan->tmA, p.in, {(cuuint64_t)inner, (cuuint64_t)(Wp * 4 / inner), (cuuint64_t)Hp, (cuuint64_t)max_batch},
+                          {(cuuint64_t)inner * 2, (cuuint64_t)Wp * 8, (cuuint64_t)Hp * Wp * 8},
+                          {(cuuint32_t)inner, (cuuint32_t)(Wp * 4 / inner), 7, 1}, CU_TENSOR_MAP_SWIZZLE_NONE);
     } else {
       // one filter row of one output row: {window element (8 pixels x 4 ch), output pixel q (+2 pixels), input row, image}
-      cuuint64_t dims[4] = {32, (cuuint64_t)p.Q, (cuuint64_t)Hp, (cuuint64_t)max_batch};
-      cuuint64_t strides[3] = {16, (cuuint64_t)Wp * 8, (cuuint64_t)Hp * Wp * 8};
-      cuuint32_t box[4] = {32, (cuuint32_t)p.Q, 1, 1};
-      cuuint32_t es[4] = {1, 1, 1, 1};
-      CUresult r = g_encodeTiled(&plan->tmA, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(p.in), dims, strides,
-                                 box, es, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B,
-                                 CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-      if (r != CUDA_SUCCESS) {
-        set_error("cuTensorMapEncodeTiled (stem, 4-channel rows, 64B swizzle) failed (%d)", (int)r);
-        delete plan;
-        return NIB_ECUDA;
-      }
+      rc = encode_4d_bf16(&plan->tmA, p.in, {32, (cuuint64_t)p.Q, (cuuint64_t)Hp, (cuuint64_t)max_batch},
+                          {16, (cuuint64_t)Wp * 8, (cuuint64_t)Hp * Wp * 8}, {32, (cuuint32_t)p.Q, 1, 1},
+                          CU_TENSOR_MAP_SWIZZLE_64B);
     }
-    rc = finish_plan(plan, p, max_batch, p.w_alt, 4 * 64);
-    if (rc != NIB_OK) { delete plan; return rc; }
-    {
-      // weights [Cout][256] as 64B-swizzled K atoms of 32 elements, BLOCK_N/2 rows per CTA (overrides finish_plan's map)
-      cuuint64_t dims[2] = {256, (cuuint64_t)p.Cout};
-      cuuint64_t strides[1] = {256 * 2};
-      cuuint32_t box[2] = {32, (cuuint32_t)(plan->block_n / 2)};
-      cuuint32_t es[2] = {1, 1};
-      CUresult r = g_encodeTiled(&plan->tmBh, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(p.w_alt), dims, strides,
-                                 box, es, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B,
-                                 CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-      if (r != CUDA_SUCCESS) {
-        set_error("cuTensorMapEncodeTiled (stem weights, 64B swizzle) failed (%d)", (int)r);
-        delete plan;
-        return NIB_ECUDA;
-      }
-    }
-    plan->tmB = plan->tmBh;
-    *out = plan;
-    return NIB_OK;
+    if (rc != NIB_OK) return rc;
+    if ((rc = finish_plan(plan, p, max_batch, p.w_alt, K)) != NIB_OK) return rc;
+    return encode_raw_row_weights(plan, p, K);
   }
   if (tc_conv_is_raw3x3(p)) {
+    const int K = raw_row_layout(p).k();
     const int Hp = p.Hin + 2, Wp = p.Win + 2, row_el = Wp * 8, inner = raw_row_inner(row_el);
-    plan->im2col = 5;
-    plan->raw_rows = 3;
-    plan->col_tiles = raw3x3_col_tiles(p.Q);
-    plan->cblocks = 1;
-    plan->num_k_blocks = 2;                 // resident weights: filter rows (0, 1) and (2, zero row)
-    plan->tile_rows = p.Q / plan->col_tiles;
-    plan->halo_wp = Wp * 16;
-    {
-      // three padded rows of one image as {inner, chunk, row, image}
-      cuuint64_t dims[4] = {(cuuint64_t)inner, (cuuint64_t)(row_el / inner), (cuuint64_t)Hp, (cuuint64_t)max_batch};
-      cuuint64_t strides[3] = {(cuuint64_t)inner * 2, (cuuint64_t)Wp * 16, (cuuint64_t)Hp * Wp * 16};
-      cuuint32_t box[4] = {(cuuint32_t)inner, (cuuint32_t)(row_el / inner), 3, 1};
-      cuuint32_t es[4] = {1, 1, 1, 1};
-      CUresult r = g_encodeTiled(&plan->tmA, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(p.in), dims, strides,
-                                 box, es, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
-                                 CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-      if (r != CUDA_SUCCESS) {
-        set_error("cuTensorMapEncodeTiled (3x3, raw rows) failed (%d)", (int)r);
-        delete plan;
-        return NIB_ECUDA;
-      }
-    }
-    rc = finish_plan(plan, p, max_batch, p.w_alt, 2 * 64);
-    if (rc != NIB_OK) { delete plan; return rc; }
-    if (!plan->v3) { set_error("tc_conv_plan_create: the 3x3 raw-row mode needs the CTA-pair kernel"); delete plan; return NIB_EINVAL; }
-    {
-      // weights [Cout][128] as 64B-swizzled K atoms of 32 elements, BLOCK_N/2 rows per CTA (overrides finish_plan's map)
-      cuuint64_t dims[2] = {128, (cuuint64_t)p.Cout};
-      cuuint64_t strides[1] = {128 * 2};
-      cuuint32_t box[2] = {32, (cuuint32_t)(plan->block_n / 2)};
-      cuuint32_t es[2] = {1, 1};
-      CUresult r = g_encodeTiled(&plan->tmBh, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(p.w_alt), dims, strides,
-                                 box, es, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B,
-                                 CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-      if (r != CUDA_SUCCESS) {
-        set_error("cuTensorMapEncodeTiled (3x3 raw-row weights, 64B swizzle) failed (%d)", (int)r);
-        delete plan;
-        return NIB_ECUDA;
-      }
-    }
-    plan->tmB = plan->tmBh;
-    *out = plan;
-    return NIB_OK;
+    kp.a_mode = TC_A_RAW;
+    kp.raw_rows = 3;
+    kp.col_tiles = raw3x3_col_tiles(p.Q);
+    kp.cblocks = 1;
+    kp.num_k_blocks = K / TC_BLOCK_K;       // resident weights: filter rows (0, 1) and (2, zero row)
+    kp.tile_rows = p.Q / kp.col_tiles;
+    kp.halo_wp = Wp * 16;
+    kp.a_bytes = kp.raw_rows * kp.halo_wp;
+    // three padded rows of one image as {inner, chunk, row, image}
+    rc = encode_4d_bf16(&plan->tmA, p.in, {(cuuint64_t)inner, (cuuint64_t)(row_el / inner), (cuuint64_t)Hp, (cuuint64_t)max_batch},
+                        {(cuuint64_t)inner * 2, (cuuint64_t)Wp * 16, (cuuint64_t)Hp * Wp * 16},
+                        {(cuuint32_t)inner, (cuuint32_t)(row_el / inner), 3, 1}, CU_TENSOR_MAP_SWIZZLE_NONE);
+    if (rc != NIB_OK) return rc;
+    if ((rc = finish_plan(plan, p, max_batch, p.w_alt, K)) != NIB_OK) return rc;
+    return encode_raw_row_weights(plan, p, K);
   }
   if (tc_conv_is_stem(p)) {
-    plan->im2col = 2;
-    plan->cblocks = 1;
-    plan->num_k_blocks = 7;
-    plan->tile_rows = p.Q;
-    rc = encode_2d_bf16(&plan->tmB, p.w_alt, 7 * 64, (uint64_t)p.Cout, 7 * 64 * 2, TC_BLOCK_K, plan->block_n);
-    if (rc != NIB_OK) { delete plan; return rc; }
+    const int K = raw_row_layout(p).k();
+    kp.a_mode = TC_A_STEM8;
+    kp.cblocks = 1;
+    kp.num_k_blocks = K / TC_BLOCK_K;
+    kp.tile_rows = p.Q;
+    kp.a_bytes = kp.tile_rows * TC_BLOCK_K * 2;
+    rc = encode_2d_bf16(&plan->tmB, p.w_alt, (uint64_t)K, (uint64_t)p.Cout, (uint64_t)K * 2, TC_BLOCK_K, plan->block_n);
+    if (rc != NIB_OK) return rc;
     const int Hp = p.Hin + 6, Wp = p.Win + 6;
-    cuuint64_t dims[4] = {64, (cuuint64_t)p.Q, (cuuint64_t)Hp, (cuuint64_t)max_batch};
-    cuuint64_t strides[3] = {32, (cuuint64_t)Wp * 16, (cuuint64_t)Hp * Wp * 16};   // 2 pixels, one row, one image
-    cuuint32_t box[4] = {64, (cuuint32_t)p.Q, 1, 1};
-    cuuint32_t es[4] = {1, 1, 1, 1};
-    CUresult r = g_encodeTiled(&plan->tmA, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(p.in), dims, strides,
-                               box, es, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-                               CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) {
-      set_error("cuTensorMapEncodeTiled (stem, overlapping windows) failed (%d)", (int)r);
-      delete plan;
-      return NIB_ECUDA;
-    }
-    rc = finish_plan(plan, p, max_batch, p.w_alt, 7 * 64);
-    if (rc != NIB_OK) { delete plan; return rc; }
-    *out = plan;
-    return NIB_OK;
+    // {window element, output pixel q (+2 pixels), input row, image}
+    rc = encode_4d_bf16(&plan->tmA, p.in, {64, (cuuint64_t)p.Q, (cuuint64_t)Hp, (cuuint64_t)max_batch},
+                        {32, (cuuint64_t)Wp * 16, (cuuint64_t)Hp * Wp * 16}, {64, (cuuint32_t)p.Q, 1, 1},
+                        CU_TENSOR_MAP_SWIZZLE_128B);
+    if (rc != NIB_OK) return rc;
+    return finish_plan(plan, p, max_batch, p.w_alt, K);
   }
   if (tc_conv_is_halo3x3(p)) {
     const int Wp = p.Win + 2, R = halo_rows_per_tile(p.Hin, Wp);
-    plan->im2col = 4;
-    plan->cblocks = p.Cin / 64;
-    plan->num_k_blocks = 9 * plan->cblocks;
-    plan->tile_rows = R * p.Win;
-    plan->halo_wp = Wp; plan->halo_r = R; plan->halo_tpi = p.Hin / R;
-    plan->halo_cb = plan->cblocks; plan->halo_n = p.Cout;
+    kp.a_mode = TC_A_HALO;
+    kp.cblocks = p.Cin / 64;
+    kp.num_k_blocks = 9 * kp.cblocks;
+    kp.tile_rows = R * p.Win;
+    kp.halo_wp = Wp; kp.halo_r = R; kp.halo_tpi = p.Hin / R;
+    kp.halo_cb = kp.cblocks; kp.halo_n = p.Cout;
+    kp.a_bytes = (R + 2) * Wp * 128;
     plan->block_n = 64;                               // the kernel instance; the MMA's N is halo_n
     const int Kh = 9 * p.Cin;
     rc = encode_2d_bf16(&plan->tmB, p.w, (uint64_t)Kh, (uint64_t)p.Cout, (uint64_t)Kh * 2, TC_BLOCK_K, (uint32_t)p.Cout);
-    if (rc != NIB_OK) { delete plan; return rc; }
-    {
-      // the dense NHWC input as {channel, column, row, image}; the box is the whole patch of one tile
-      cuuint64_t dims[4] = {(cuuint64_t)p.in_cstride, (cuuint64_t)p.Win, (cuuint64_t)p.Hin, (cuuint64_t)max_batch};
-      cuuint64_t strides[3] = {(cuuint64_t)p.in_cstride * 2, (cuuint64_t)p.Win * p.in_cstride * 2,
-                               (cuuint64_t)p.Hin * p.Win * p.in_cstride * 2};
-      cuuint32_t box[4] = {64, (cuuint32_t)Wp, (cuuint32_t)(R + 2), 1};
-      cuuint32_t es[4] = {1, 1, 1, 1};
-      CUresult r = g_encodeTiled(&plan->tmA, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(p.in), dims, strides,
-                                 box, es, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-                                 CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-      if (r != CUDA_SUCCESS) {
-        set_error("cuTensorMapEncodeTiled (3x3 halo patch) failed (%d)", (int)r);
-        delete plan;
-        return NIB_ECUDA;
-      }
-    }
+    if (rc != NIB_OK) return rc;
+    // the dense NHWC input as {channel, column, row, image}; the box is the whole patch of one tile
+    rc = encode_4d_bf16(&plan->tmA, p.in, {(cuuint64_t)p.in_cstride, (cuuint64_t)p.Win, (cuuint64_t)p.Hin, (cuuint64_t)max_batch},
+                        {(cuuint64_t)p.in_cstride * 2, (cuuint64_t)p.Win * p.in_cstride * 2,
+                         (cuuint64_t)p.Hin * p.Win * p.in_cstride * 2},
+                        {64, (cuuint32_t)Wp, (cuuint32_t)(R + 2), 1}, CU_TENSOR_MAP_SWIZZLE_128B);
+    if (rc != NIB_OK) return rc;
     // each CTA of the pair holds Cout / 2 weight rows per K block; the kernel's "tail" slot carries the whole-tile output
     // box (Cout channels: 64 B rows under the 64B swizzle when Cout = 32); the other output / residual maps are unused
     rc = encode_2d_bf16(&plan->tmBh, p.w, (uint64_t)Kh, (uint64_t)p.Cout, (uint64_t)Kh * 2, TC_BLOCK_K, (uint32_t)(p.Cout / 2));
-    if (rc != NIB_OK) { delete plan; return rc; }
-    {
-      const uint64_t rows = (uint64_t)max_batch * p.P * p.Q;
-      cuuint64_t dims[2] = {(cuuint64_t)p.out_cstride, rows};
-      cuuint64_t strides[1] = {(cuuint64_t)p.out_cstride * 2};
-      cuuint32_t box[2] = {(cuuint32_t)p.Cout, (cuuint32_t)plan->tile_rows};
-      cuuint32_t es[2] = {1, 1};
-      CUresult r = g_encodeTiled(&plan->tmOutTail, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, p.out, dims, strides, box, es,
-                                 CU_TENSOR_MAP_INTERLEAVE_NONE, p.Cout == 32 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_128B,
-                                 CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-      if (r != CUDA_SUCCESS) {
-        set_error("cuTensorMapEncodeTiled (3x3 halo output box) failed (%d)", (int)r);
-        delete plan;
-        return NIB_ECUDA;
-      }
-    }
+    if (rc != NIB_OK) return rc;
+    rc = encode_2d_bf16(&plan->tmOutTail, p.out, (uint64_t)p.out_cstride, (uint64_t)max_batch * p.P * p.Q,
+                        (uint64_t)p.out_cstride * 2, (uint32_t)p.Cout, (uint32_t)kp.tile_rows,
+                        p.Cout == 32 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_128B);
+    if (rc != NIB_OK) return rc;
     plan->tmOut = plan->tmOut32 = plan->tmRes = plan->tmOutTail;
     plan->v3 = 1;
-    *out = plan;
     return NIB_OK;
   }
-  plan->split = p.split;
-  plan->cblocks = (p.split ? 3 : 1) * p.Cin / TC_BLOCK_K;
-  plan->num_k_blocks = p.R * p.S * plan->cblocks;
-  plan->im2col = !(p.R == 1 && p.S == 1 && p.stride == 1 && p.pad == 0);
+  kp.cblocks = (p.split ? 3 : 1) * p.Cin / TC_BLOCK_K;
+  kp.num_k_blocks = p.R * p.S * kp.cblocks;
+  kp.a_mode = (p.R == 1 && p.S == 1 && p.stride == 1 && p.pad == 0) ? TC_A_DENSE : TC_A_IM2COL;
+  kp.a_bytes = kp.tile_rows * TC_BLOCK_K * 2;
   const int K = p.R * p.S * p.Cin * (p.split ? 3 : 1);
   // B: weights [Cout][K]
   rc = encode_2d_bf16(&plan->tmB, p.w, (uint64_t)K, (uint64_t)p.Cout, (uint64_t)K * 2, TC_BLOCK_K, plan->block_n);
-  if (rc != NIB_OK) { delete plan; return rc; }
-  if (!plan->im2col) {
+  if (rc != NIB_OK) return rc;
+  if (kp.a_mode == TC_A_DENSE) {
     const uint64_t rows = (uint64_t)max_batch * p.Hin * p.Win;
     rc = encode_2d_bf16(&plan->tmA, p.in, (uint64_t)p.in_cstride, rows, (uint64_t)p.in_cstride * 2, TC_BLOCK_K,
                         TC_BLOCK_M);
-    if (rc != NIB_OK) { delete plan; return rc; }
+    if (rc != NIB_OK) return rc;
   } else {
     cuuint64_t dims[4] = {(cuuint64_t)p.in_cstride, (cuuint64_t)p.Win, (cuuint64_t)p.Hin, (cuuint64_t)max_batch};
     cuuint64_t strides[3] = {(cuuint64_t)p.in_cstride * 2, (cuuint64_t)p.Win * p.in_cstride * 2,
@@ -2098,7 +2047,6 @@ int tc_conv_plan_create(const ConvParams& p, int max_batch, TcConvPlan** out) {
     if (r != CUDA_SUCCESS) {
       set_error("cuTensorMapEncodeIm2col failed (%d): C=%d W=%d H=%d N=%d R=%d stride=%d pad=%d", (int)r,
                 p.in_cstride, p.Win, p.Hin, max_batch, p.R, p.stride, p.pad);
-      delete plan;
       return NIB_ECUDA;
     }
     // Driver quirk mirrored from CUTLASS (cute/atom/copy_traits_sm90_im2col.hpp): for tensors smaller
@@ -2108,13 +2056,152 @@ int tc_conv_plan_create(const ConvParams& p, int max_batch, TcConvPlan** out) {
     const uint64_t bytes = (uint64_t)max_batch * p.Hin * p.Win * p.in_cstride * 2;
     if (drv <= 13010 && bytes < 131072) reinterpret_cast<uint64_t*>(&plan->tmA)[1] &= ~(1ull << 21);
   }
-  rc = finish_plan(plan, p, max_batch, p.w, K);
-  if (rc != NIB_OK) { delete plan; return rc; }
-  *out = plan;
+  return finish_plan(plan, p, max_batch, p.w, K);
+}
+
+template <int BLOCK_N, int STAGES>
+static int launch_tc(const TcConvPlan* plan, const TcKernelParams& kp, cudaStream_t st) {
+  using SM = TcSmem<BLOCK_N, STAGES>;
+  static bool attr_set = false;
+  if (!attr_set) {
+    NIB_CUDA(cudaFuncSetAttribute(conv_tc_kernel<BLOCK_N, STAGES>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                  SM::TOTAL));
+    attr_set = true;
+  }
+  conv_tc_kernel<BLOCK_N, STAGES><<<kp.m_tiles * kp.n_tiles, TC_THREADS, SM::TOTAL, st>>>(plan->tmA, plan->tmB, kp);
+  NIB_LAUNCH_CHECK();
+  return NIB_OK;
+}
+
+template <int BLOCK_N, int STAGES, bool HAS_RES, bool BRES = false, bool SPLIT = false>
+static int launch_tc3(const TcConvPlan* plan, const TcKernelParams& kp, cudaStream_t st) {
+  using SM = Tc3Smem<BLOCK_N, STAGES, HAS_RES, BRES, SPLIT>;
+  static_assert(SM::TOTAL <= 232448, "exceeds the 227 KB per-CTA shared memory limit");
+  static bool attr_set = false;
+  if (!attr_set) {
+    NIB_CUDA(cudaFuncSetAttribute(conv_tc3_kernel<BLOCK_N, STAGES, HAS_RES, BRES, SPLIT>,
+                                  cudaFuncAttributeMaxDynamicSharedMemorySize, SM::TOTAL));
+    attr_set = true;
+  }
+  const int pair_tiles = ((kp.m_tiles + 1) / 2) * kp.n_tiles;
+  const int max_pairs = num_sms() / 2;
+  const int pairs = pair_tiles < max_pairs ? pair_tiles : max_pairs;
+  // launched with programmatic stream serialization: the CTAs become resident (and run their prologue) as the SMs of
+  // the previous kernel free up, then block in griddepcontrol.wait until that kernel has completed
+  static const bool pdl = getenv("NIB_TC_NO_PDL") == nullptr;
+  cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+  cudaStreamIsCapturing(st, &cap);
+  cudaLaunchConfig_t cfg;
+  memset(&cfg, 0, sizeof(cfg));
+  cfg.gridDim = dim3(2 * pairs);
+  cfg.blockDim = dim3((!BRES && !SPLIT && kp.xf_scale != nullptr) ? TC3_THREADS_XF : TC3_THREADS);
+  cfg.dynamicSmemBytes = SM::TOTAL;
+  cfg.stream = st;
+  cudaLaunchAttribute attr[1];
+  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  attr[0].val.programmaticStreamSerializationAllowed = 1;
+  cfg.attrs = attr;
+  cfg.numAttrs = (pdl && cap == cudaStreamCaptureStatusNone && kp.dbg == nullptr) ? 1 : 0;
+  NIB_CUDA(cudaLaunchKernelEx(&cfg, conv_tc3_kernel<BLOCK_N, STAGES, HAS_RES, BRES, SPLIT>, plan->tmA, plan->tmBh, plan->tmOut32,
+                              plan->tmOutTail, plan->tmRes, kp));
+  return NIB_OK;
+}
+
+// The kernel instance of a plan whose kp is filled in.  CTA-pair stage counts fill the 227 KB of each SM (ring +
+// output / residual boxes).  Only the streamed-weight CTA-pair instances have the transform warps a pre-activated conv
+// needs; a plan that would land elsewhere is refused here rather than run without its BN-ReLU.
+static int pick_instance(TcConvPlan* plan) {
+  const TcKernelParams& kp = plan->kp;
+  const bool res = kp.res != nullptr;
+  bool xf_role = false;
+  TcLauncher L = nullptr;
+  if (plan->split) {
+    // split-bf16 tensors: twice the residual / staging boxes, so shallower operand rings where a residual is added
+    if (!plan->v3) { set_error("tc_conv_plan_create: split mode needs the CTA-pair kernel"); return NIB_EINVAL; }
+    if (plan->block_n == 256) L = res ? &launch_tc3<256, 3, true, false, true> : &launch_tc3<256, 6, false, false, true>;
+    else if (plan->block_n == 128) L = res ? &launch_tc3<128, 4, true, false, true> : &launch_tc3<128, 8, false, false, true>;
+    else L = res ? &launch_tc3<64, 8, true, false, true> : &launch_tc3<64, 9, false, false, true>;
+  } else if (plan->v3 && !kp.out_f32) {
+    xf_role = true;
+    if (kp.a_mode == TC_A_HALO) {                                   // resident patch + resident weights
+      L = &launch_tc3<64, 9, false, true>;
+      xf_role = false;
+    } else if (kp.a_mode == TC_A_RAW && plan->block_n == 128) {     // raw rows, 128 outputs
+      L = &launch_tc3<128, 6, false, true>;
+      xf_role = false;
+    } else if (plan->block_n == 256) {
+      L = res ? &launch_tc3<256, 5, true> : &launch_tc3<256, 6, false>;
+    } else if (plan->block_n == 128) {
+      L = res ? &launch_tc3<128, 6, true> : &launch_tc3<128, 8, false>;
+    } else if (!res && kp.n_tiles == 1 && kp.num_k_blocks <= TC3_BRES_KBLOCKS && kp.xf_scale == nullptr) {
+      // resident weights: stem, 56x56 64-channel layers.  Not for a pre-activated conv (DenseNet-BC with
+      // bn_size * growth == 64): it stays on the streamed instance, which has the transform warps
+      L = &launch_tc3<64, 9, false, true>;
+      xf_role = false;
+    } else {
+      L = res ? &launch_tc3<64, 9, true> : &launch_tc3<64, 9, false>;
+    }
+  } else {
+    if (kp.a_mode > TC_A_STEM8) {   // the one-CTA kernel has no row-pair, resident-patch or raw-row operand
+      set_error("tc_conv_plan_create: A-operand mode %d needs the CTA-pair kernel", kp.a_mode);
+      return NIB_EINVAL;
+    }
+    switch (plan->block_n) {
+      case 32:  L = &launch_tc<32, 4>; break;
+      case 64:  L = &launch_tc<64, 4>; break;
+      case 128: L = &launch_tc<128, 3>; break;
+      default:  L = &launch_tc<256, 4>; break;
+    }
+  }
+  if (kp.xf_scale != nullptr && !xf_role) {
+    set_error("tc_conv_plan_create: no kernel instance with the BN-ReLU transform warps serves this pre-activation conv "
+              "(Cout=%d, block_n=%d, CTA pair %d)", kp.Cout, plan->block_n, plan->v3);
+    return NIB_EINVAL;
+  }
+  plan->launch = L;
+  return NIB_OK;
+}
+
+int tc_conv_plan_create(const ConvParams& p, int max_batch, TcConvPlan** out) {
+  int rc = init_tc();
+  if (rc != NIB_OK) return rc;
+  std::unique_ptr<TcConvPlan> plan(new TcConvPlan());
+  TcKernelParams& kp = plan->kp;
+  plan->split = p.split;
+  plan->block_n = pick_block_n(p.Cout);
+  kp.tile_rows = TC_BLOCK_M;
+  if ((rc = build_maps(plan.get(), p, max_batch)) != NIB_OK) return rc;
+  kp.bias = p.bias;
+  kp.res = reinterpret_cast<const __nv_bfloat16*>(p.res);
+  kp.out = p.out;
+  kp.Cout = p.Cout;
+  kp.out_cstride = p.out_cstride;
+  kp.out_coff = p.out_coff;
+  kp.res_cstride = p.res_cstride;
+  kp.res_coff = p.res_coff;
+  kp.relu = p.relu;
+  kp.S = p.S;
+  kp.P = p.P;
+  kp.Q = p.Q;
+  kp.stride = p.stride;
+  kp.pad = p.pad;
+  kp.in_coff = p.in_coff;
+  kp.n_tiles = kp.a_mode == TC_A_HALO ? 1 : ceil_div(p.Cout, plan->block_n);
+  kp.err_flag = g_err_flag;
+  kp.a_wrap = plan->split ? 2 * p.Cin / TC_BLOCK_K : kp.cblocks;
+  kp.lo_off_out = p.out_lo_off;
+  kp.lo_off_res = p.res_lo_off;
+  kp.xf_scale = p.pre_scale;
+  kp.xf_shift = p.pre_shift;
+  static const bool swap = getenv("NIB_TC_STEM_SWAP") != nullptr;
+  kp.halo_swap = kp.a_mode == TC_A_RAW && swap ? 1 : 0;
+  if ((rc = pick_instance(plan.get())) != NIB_OK) return rc;
+  *out = plan.release();
   return NIB_OK;
 }
 
 void tc_conv_plan_destroy(TcConvPlan* plan) { delete plan; }
+int tc_conv_plan_block_n(const TcConvPlan* plan) { return plan->block_n; }
 
 // ---- fused expansion + next reduction (conv_fused_ca_kernel) ------------------------------------------------
 struct TcFusedPlan {
@@ -2152,14 +2239,9 @@ bool tc_fuse_supported(const ConvParams& c, const ConvParams& a) {
 }
 
 int tc_fused_plan_create(const ConvParams& c, const ConvParams& a, int max_batch, TcFusedPlan** out) {
-  int rc = load_driver_fns();
+  int rc = init_tc();
   if (rc != NIB_OK) return rc;
-  if (!g_err_flag) {
-    NIB_CUDA(cudaMalloc(&g_err_flag, sizeof(unsigned int)));
-    NIB_CUDA(cudaMemset(g_err_flag, 0, sizeof(unsigned int)));
-  }
-  TcFusedPlan* plan = new TcFusedPlan();
-  memset(plan, 0, sizeof(*plan));
+  std::unique_ptr<TcFusedPlan> plan(new TcFusedPlan());
   plan->err_flag = g_err_flag;
   plan->n2 = a.Cout;
   const uint64_t rows = (uint64_t)max_batch * c.P * c.Q;
@@ -2170,8 +2252,8 @@ int tc_fused_plan_create(const ConvParams& c, const ConvParams& a, int max_batch
   if (rc == NIB_OK) rc = encode_2d_bf16(&plan->tmY, c.out, N1, rows, N1 * 2, 64, 32);
   if (rc == NIB_OK) rc = encode_2d_bf16(&plan->tmB2, a.w, N1, N2, N1 * 2, TC_BLOCK_K, (uint32_t)(N2 / 2));
   if (rc == NIB_OK) rc = encode_2d_bf16(&plan->tmOut2, a.out, N2, rows, N2 * 2, 64, 32);
-  if (rc != NIB_OK) { delete plan; return rc; }
-  *out = plan;
+  if (rc != NIB_OK) return rc;
+  *out = plan.release();
   return NIB_OK;
 }
 
@@ -2261,99 +2343,9 @@ int tc_fused_launch(const TcFusedPlan* plan, const ConvParams& c, const ConvPara
   set_error("tc_fused_launch: unsupported N2=%d", plan->n2);
   return NIB_EINVAL;
 }
-int tc_conv_plan_block_n(const TcConvPlan* plan) { return plan->block_n; }
-
-template <int BLOCK_N, int STAGES>
-static int launch_tc(const TcConvPlan* plan, const TcKernelParams& kp, int tiles, cudaStream_t st) {
-  using SM = TcSmem<BLOCK_N, STAGES>;
-  static bool attr_set = false;
-  if (!attr_set) {
-    NIB_CUDA(cudaFuncSetAttribute(conv_tc_kernel<BLOCK_N, STAGES>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                  SM::TOTAL));
-    attr_set = true;
-  }
-  conv_tc_kernel<BLOCK_N, STAGES><<<tiles, TC_THREADS, SM::TOTAL, st>>>(plan->tmA, plan->tmB, kp);
-  NIB_LAUNCH_CHECK();
-  return NIB_OK;
-}
-
-template <int BLOCK_N, int STAGES, bool HAS_RES, bool BRES = false, bool SPLIT = false>
-static int launch_tc3(const TcConvPlan* plan, const TcKernelParams& kp, cudaStream_t st) {
-  using SM = Tc3Smem<BLOCK_N, STAGES, HAS_RES, BRES, SPLIT>;
-  static_assert(SM::TOTAL <= 232448, "exceeds the 227 KB per-CTA shared memory limit");
-  if (kp.xf_scale != nullptr && (BRES || SPLIT)) {   // no transform warps in these instantiations: never drop the BN-ReLU
-    set_error("tc_dispatch: a pre-activation conv reached a CTA-pair instantiation without the transform role");
-    return NIB_EINVAL;
-  }
-  static bool attr_set = false;
-  if (!attr_set) {
-    NIB_CUDA(cudaFuncSetAttribute(conv_tc3_kernel<BLOCK_N, STAGES, HAS_RES, BRES, SPLIT>,
-                                  cudaFuncAttributeMaxDynamicSharedMemorySize, SM::TOTAL));
-    attr_set = true;
-  }
-  const int pair_tiles = ((kp.m_tiles + 1) / 2) * kp.n_tiles;
-  const int max_pairs = num_sms() / 2;
-  const int pairs = pair_tiles < max_pairs ? pair_tiles : max_pairs;
-  // launched with programmatic stream serialization: the CTAs become resident (and run their prologue) as the SMs of
-  // the previous kernel free up, then block in griddepcontrol.wait until that kernel has completed
-  static const bool pdl = getenv("NIB_TC_NO_PDL") == nullptr;
-  cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-  cudaStreamIsCapturing(st, &cap);
-  cudaLaunchConfig_t cfg;
-  memset(&cfg, 0, sizeof(cfg));
-  cfg.gridDim = dim3(2 * pairs);
-  cfg.blockDim = dim3((!BRES && !SPLIT && kp.xf_scale != nullptr) ? TC3_THREADS_XF : TC3_THREADS);
-  cfg.dynamicSmemBytes = SM::TOTAL;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = (pdl && cap == cudaStreamCaptureStatusNone && kp.dbg == nullptr) ? 1 : 0;
-  NIB_CUDA(cudaLaunchKernelEx(&cfg, conv_tc3_kernel<BLOCK_N, STAGES, HAS_RES, BRES, SPLIT>, plan->tmA, plan->tmBh, plan->tmOut32,
-                              plan->tmOutTail, plan->tmRes, kp));
-  return NIB_OK;
-}
-
-static int tc_dispatch(const TcConvPlan* plan, const TcKernelParams& kp, int tiles, cudaStream_t st) {
-  if (plan->split) {
-    // split-bf16 tensors: twice the residual / staging boxes, so shallower operand rings where a residual is added
-    const bool res = kp.res != nullptr;
-    if (!plan->v3 || kp.out_f32) { set_error("tc_dispatch: split mode needs the CTA-pair kernel"); return NIB_EINVAL; }
-    if (plan->block_n == 256) return res ? launch_tc3<256, 3, true, false, true>(plan, kp, st) : launch_tc3<256, 6, false, false, true>(plan, kp, st);
-    if (plan->block_n == 128) return res ? launch_tc3<128, 4, true, false, true>(plan, kp, st) : launch_tc3<128, 8, false, false, true>(plan, kp, st);
-    return res ? launch_tc3<64, 8, true, false, true>(plan, kp, st) : launch_tc3<64, 9, false, false, true>(plan, kp, st);
-  }
-  if (plan->v3 && !kp.out_f32) {
-    // CTA-pair kernel; stage counts fill the 227 KB of each SM (ring + output/residual boxes)
-    const bool res = kp.res != nullptr;
-    if (plan->im2col == 4) return launch_tc3<64, 9, false, true>(plan, kp, st);   // resident patch + resident weights
-    if (plan->im2col == 5 && plan->block_n == 128) return launch_tc3<128, 6, false, true>(plan, kp, st);   // raw rows, 128 out
-    if (plan->block_n == 256) return res ? launch_tc3<256, 5, true>(plan, kp, st) : launch_tc3<256, 6, false>(plan, kp, st);
-    if (plan->block_n == 128) return res ? launch_tc3<128, 6, true>(plan, kp, st) : launch_tc3<128, 8, false>(plan, kp, st);
-    // resident weights: stem, 56x56 64-channel layers.  Not for a pre-activated conv: the BRES instantiation has no
-    // transform warps, so a 64-output BN-ReLU-conv (DenseNet-BC with bn_size * growth == 64) stays on the streamed one
-    if (plan->block_n == 64 && !res && kp.n_tiles == 1 && kp.num_k_blocks <= TC3_BRES_KBLOCKS && kp.xf_scale == nullptr)
-      return launch_tc3<64, 9, false, true>(plan, kp, st);
-    if (plan->block_n == 64) return res ? launch_tc3<64, 9, true>(plan, kp, st) : launch_tc3<64, 9, false>(plan, kp, st);
-  }
-  if (kp.xf_scale != nullptr) {
-    set_error("tc_dispatch: a pre-activation conv reached the one-CTA kernel, which has no transform role");
-    return NIB_EINVAL;
-  }
-  switch (plan->block_n) {
-    case 32:  return launch_tc<32, 4>(plan, kp, tiles, st);
-    case 64:  return launch_tc<64, 4>(plan, kp, tiles, st);
-    case 128: return launch_tc<128, 3>(plan, kp, tiles, st);
-    case 256: return launch_tc<256, 4>(plan, kp, tiles, st);
-  }
-  set_error("tc_dispatch: bad block_n %d", plan->block_n);
-  return NIB_EINVAL;
-}
-
 // NIB_TC_DBG=1: run the launch with the role timers on, synchronise and print where each warp role of the CTA-pair
 // kernel spent its time (average over CTAs, microseconds at the SM clock).  Diagnostic only.
-static int tc_launch_debug(const TcConvPlan* plan, TcKernelParams kp, const ConvParams& p, int tiles, cudaStream_t st) {
+static int tc_launch_debug(const TcConvPlan* plan, TcKernelParams kp, const ConvParams& p, cudaStream_t st) {
   static unsigned long long* d_dbg = nullptr;
   const int nslots = 160 * 16;
   if (!d_dbg) NIB_CUDA(cudaMalloc(&d_dbg, nslots * sizeof(unsigned long long)));
@@ -2362,7 +2354,7 @@ static int tc_launch_debug(const TcConvPlan* plan, TcKernelParams kp, const Conv
   cudaEvent_t e0, e1;
   cudaEventCreate(&e0); cudaEventCreate(&e1);
   cudaEventRecord(e0, st);
-  int rc = tc_dispatch(plan, kp, tiles, st);
+  int rc = plan->launch(plan, kp, st);
   cudaEventRecord(e1, st);
   if (rc != NIB_OK) return rc;
   NIB_CUDA(cudaStreamSynchronize(st));
@@ -2405,66 +2397,15 @@ static int tc_launch_debug(const TcConvPlan* plan, TcKernelParams kp, const Conv
 }
 
 int tc_conv_launch(const TcConvPlan* plan, const ConvParams& p, cudaStream_t st) {
-  TcKernelParams kp;
-  memset(&kp, 0, sizeof(kp));
-  kp.bias = p.bias;
-  kp.res = reinterpret_cast<const __nv_bfloat16*>(p.res);
-  kp.out = p.out;
+  TcKernelParams kp = plan->kp;
   kp.M = p.M;
-  kp.Cout = p.Cout;
-  kp.out_cstride = p.out_cstride;
-  kp.out_coff = p.out_coff;
-  kp.res_cstride = p.res_cstride;
-  kp.res_coff = p.res_coff;
-  kp.relu = p.relu;
-  kp.out_f32 = 0;
-  kp.num_k_blocks = plan->num_k_blocks;
-  kp.cblocks = plan->cblocks;
-  kp.S = p.S;
-  kp.im2col = plan->im2col;
-  kp.P = p.P;
-  kp.Q = p.Q;
-  kp.stride = p.stride;
-  kp.pad = p.pad;
-  kp.in_coff = p.in_coff;
-  kp.n_tiles = ceil_div(p.Cout, plan->block_n);
-  kp.err_flag = plan->err_flag;
-  kp.tile_rows = plan->tile_rows;
-  kp.a_bytes = plan->tile_rows * TC_BLOCK_K * 2;
-  kp.m_tiles = ceil_div(p.M, plan->tile_rows);
-  kp.a_wrap = plan->split ? 2 * p.Cin / TC_BLOCK_K : plan->cblocks;
-  kp.lo_off_out = p.out_lo_off;
-  kp.lo_off_res = p.res_lo_off;
+  // raw rows: pair tiles = output-row pairs x column tiles (an odd last row pairs with a row past the batch, as any odd
+  // tile count)
+  kp.m_tiles = kp.a_mode == TC_A_RAW ? (p.M / p.Q + 1) / 2 * 2 * kp.col_tiles : ceil_div(p.M, kp.tile_rows);
   kp.dyn_n = plan->split ? p.dyn_n : nullptr;
-  if (p.pre_scale != nullptr) {
-    if (!(p.pre_padded && plan->im2col == 0 && plan->v3 && !plan->split)) {
-      set_error("tc_conv_launch: a pre-activation conv reached a tensor path without the transform role");
-      return NIB_EINVAL;
-    }
-    kp.xf_scale = p.pre_scale;
-    kp.xf_shift = p.pre_shift;
-  }
-  if (plan->im2col == 4) {
-    kp.n_tiles = 1;
-    kp.halo_cb = plan->halo_cb; kp.halo_n = plan->halo_n;
-    kp.halo_wp = plan->halo_wp; kp.halo_r = plan->halo_r; kp.halo_tpi = plan->halo_tpi;
-    kp.a_bytes = (plan->halo_r + 2) * plan->halo_wp * 128;
-  }
-  if (plan->im2col == 5) {
-    static const bool swap = getenv("NIB_TC_STEM_SWAP") != nullptr;
-    kp.halo_wp = plan->halo_wp;          // bytes of one padded input row
-    kp.halo_swap = swap ? 1 : 0;
-    kp.raw_rows = plan->raw_rows;
-    kp.col_tiles = plan->col_tiles;
-    kp.a_bytes = plan->raw_rows * plan->halo_wp;
-    // pair tiles = output-row pairs x column tiles (an odd last row pairs with a row past the batch, as any odd tile count)
-    const int rows = p.M / p.Q;
-    kp.m_tiles = (rows + 1) / 2 * 2 * plan->col_tiles;
-  }
-  const int tiles = kp.m_tiles * kp.n_tiles;
   static const bool dbg = getenv("NIB_TC_DBG") != nullptr;
-  if (dbg && plan->v3) return tc_launch_debug(plan, kp, p, tiles, st);
-  return tc_dispatch(plan, kp, tiles, st);
+  if (dbg && plan->v3) return tc_launch_debug(plan, kp, p, st);
+  return plan->launch(plan, kp, st);
 }
 
 }  // namespace nib
@@ -2476,38 +2417,29 @@ extern "C" int nib_tc_gemm_bf16(const void* d_A, const void* d_B, float* d_C, in
   using namespace nib;
   NIB_REQUIRE(d_A && d_B && d_C, "nib_tc_gemm_bf16: null pointer");
   NIB_REQUIRE(M > 0 && N > 0 && K > 0 && K % 64 == 0 && N % 32 == 0, "nib_tc_gemm_bf16: need K%%64==0, N%%32==0");
-  int rc = load_driver_fns();
+  int rc = init_tc();
   if (rc != NIB_OK) return rc;
-  if (!g_err_flag) {
-    NIB_CUDA(cudaMalloc(&g_err_flag, sizeof(unsigned int)));
-    NIB_CUDA(cudaMemset(g_err_flag, 0, sizeof(unsigned int)));
-  }
-  TcConvPlan plan;
-  memset(&plan, 0, sizeof(plan));
-  plan.err_flag = g_err_flag;
+  TcConvPlan plan = {};
   plan.block_n = pick_block_n(N);
-  plan.cblocks = K / TC_BLOCK_K;
-  plan.num_k_blocks = plan.cblocks;
-  plan.im2col = 0;
-  rc = encode_2d_bf16(&plan.tmB, d_B, (uint64_t)K, (uint64_t)N, (uint64_t)K * 2, TC_BLOCK_K, plan.block_n);
-  if (rc != NIB_OK) return rc;
-  rc = encode_2d_bf16(&plan.tmA, d_A, (uint64_t)K, (uint64_t)M, (uint64_t)K * 2, TC_BLOCK_K, TC_BLOCK_M);
-  if (rc != NIB_OK) return rc;
-  TcKernelParams kp;
-  memset(&kp, 0, sizeof(kp));
+  TcKernelParams& kp = plan.kp;
+  kp.a_mode = TC_A_DENSE;
+  kp.cblocks = K / TC_BLOCK_K;
+  kp.num_k_blocks = kp.cblocks;
   kp.out = d_C;
   kp.M = M;
   kp.Cout = N;
   kp.out_cstride = N;
   kp.out_f32 = 1;
-  kp.num_k_blocks = plan.num_k_blocks;
-  kp.cblocks = plan.cblocks;
   kp.S = 1;
   kp.n_tiles = ceil_div(N, plan.block_n);
   kp.tile_rows = TC_BLOCK_M;
   kp.a_bytes = TC_BLOCK_M * TC_BLOCK_K * 2;
   kp.m_tiles = ceil_div(M, TC_BLOCK_M);
   kp.err_flag = g_err_flag;
-  const int tiles = ceil_div(M, TC_BLOCK_M) * kp.n_tiles;
-  return tc_dispatch(&plan, kp, tiles, (cudaStream_t)stream);
+  rc = encode_2d_bf16(&plan.tmB, d_B, (uint64_t)K, (uint64_t)N, (uint64_t)K * 2, TC_BLOCK_K, plan.block_n);
+  if (rc != NIB_OK) return rc;
+  rc = encode_2d_bf16(&plan.tmA, d_A, (uint64_t)K, (uint64_t)M, (uint64_t)K * 2, TC_BLOCK_K, TC_BLOCK_M);
+  if (rc != NIB_OK) return rc;
+  if ((rc = pick_instance(&plan)) != NIB_OK) return rc;
+  return plan.launch(&plan, kp, (cudaStream_t)stream);
 }

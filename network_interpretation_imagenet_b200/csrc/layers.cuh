@@ -7,7 +7,7 @@ namespace nib {
 struct ConvParams {
   const void* in;       // NHWC activations (T)
   const void* w;        // KRSC weights (T)
-  const void* w_alt;    // stem only: bf16 [Cout][7][8][8] (filter row, 7 taps + 1 filler, 8 padded channels) or null
+  const void* w_alt;    // raw-row modes only (tc_raw_row_layout): bf16 [Cout][rows][taps][ch], or null
   const float* bias;    // [Cout] fp32 or null
   const void* res;      // residual NHWC (T) or null
   void* out;
@@ -65,6 +65,14 @@ int mask_synth_impl(const nib_mask_args* a, cudaStream_t st, bool skip_halo, con
 
 // ---- tcgen05 implicit-GEMM convolution (conv_tc.cu) ---------------------------------------------
 struct TcConvPlan;  // opaque: tensor maps + tile configuration for one conv layer
+
+// Weights of the tcgen05 modes that read raw input rows (the 7x7 stride-2 stem, a 3x3 stride-1 first conv): bf16
+// [Cout][rows][taps][ch], zero past the filter's R x S x Cin, uploaded as ConvParams::w_alt.  rows == 0: no such mode.
+struct RawRowLayout {
+  int rows, taps, ch;
+  int k() const { return rows * taps * ch; }
+};
+RawRowLayout tc_raw_row_layout(int R, int S, int stride, int pad, int Cin, int in_cstride, int in_halo);
 
 // true when the layer geometry is covered by the tcgen05 kernel
 bool tc_conv_supported(const ConvParams& p);

@@ -27,11 +27,26 @@ struct NetBuffer {
   size_t esize() const { return kind == BUF_F32 ? 4 : 2; }
 };
 
+enum OpKind { OP_CONV, OP_POOL, OP_FC, OP_CONVERT };   // OP_CONVERT: fp32 <-> split
+
+// How a conv runs, resolved once by nib_net_finalize.
+enum ConvPath {
+  PATH_TC,           // tcgen05 plan on the conv's own operands
+  PATH_TC_XFORM,     // tcgen05 on the raw channel slice, BN-ReLU applied to the A tiles by the pair kernel's transform warps
+  PATH_TC_PACK,      // relu(bn(x)) packed into pack_scratch by a separate pass, then tcgen05 on it
+  PATH_FUSED_HEAD,   // a 1x1 expansion that also computes the next op (the following bottleneck's 1x1 reduction)
+  PATH_FUSED_TAIL,   // computed by the previous op's fused launch
+  PATH_X3,           // split-bf16 tensor-core products on fp32 activations (conv_x3.cu)
+  PATH_SIMT,         // CUDA cores
+};
+
+static bool on_tcgen05(ConvPath p) { return p != PATH_X3 && p != PATH_SIMT; }
+
 struct NetOp {
-  int kind;  // 0 conv, 1 pool, 2 fc, 3 convert (fp32 <-> split)
+  OpKind kind;
   nib_conv_desc cd;
   void* d_w;          // conv: KRSC in net dtype; fc: fp32 [Cout][Cin]
-  void* d_w_alt;      // 7x7/2 stem in bf16 nets: [Cout][7][8][8] packing for the tcgen05 row-window path
+  void* d_w_alt;      // bf16 nets, raw-row tcgen05 modes: the weights in tc_raw_row_layout
   float* d_bias;
   float* d_pre_scale;
   float* d_pre_shift;
@@ -39,17 +54,12 @@ struct NetOp {
   int pack_cin;       // that padded Cin (0: no packed tensor-core path for this op)
   float* d_pre_scale_pad;   // scale / shift zero-padded to pack_cin (the pair kernel's in-kernel transform)
   float* d_pre_shift_pad;
-  int xform;          // 1: the conv reads the raw channel slice and transforms its A tiles itself (no pack pass)
-  void* d_w_hi;       // NIB_PREC_X3: bf16 split of the fp32 KRSC weights, w = hi + lo (conv_x3.cu)
+  void* d_w_hi;       // NIB_PREC_X3 convs and bf16 nets' fc: bf16 split of the fp32 weights, w = hi + lo (conv_x3.cu)
   void* d_w_lo;
+  ConvPath path;        // with the tensor cores on
+  ConvPath cuda_path;   // after nib_net_set_tensor_core(0): PATH_X3 or PATH_SIMT
   TcConvPlan* plan;
-  // 1x1 expansion fused with the next op (the following bottleneck's 1x1 reduction): this op launches both, the next op
-  // carries fused_skip.  next_* is a copy of what the launch needs from that op (the profiler runs ops one at a time).
-  TcFusedPlan* fplan;
-  bool fused_skip;
-  nib_conv_desc next_cd;
-  void* next_w;
-  float* next_bias;
+  TcFusedPlan* fplan;   // PATH_FUSED_HEAD
   // pool
   int pool_kind, k, stride, pad, C, in_buf, in_coff, out_buf, out_coff;
   // fc
@@ -64,6 +74,7 @@ struct nib_net {
   bool split;                 // NIB_PREC_SPLIT: body tensors are BUF_SPLIT, convs run on the tcgen05 pair kernel in split mode
   std::vector<NetBuffer> bufs;
   std::vector<NetOp> ops;
+  std::vector<void*> allocs;  // every device allocation (upload), freed by nib_net_destroy
   void* pack_scratch;        // [max_batch * H * W][pack_cin] bf16: relu(bn(x)) of the conv being run (largest such layer)
   size_t pack_scratch_bytes;
   int input_buf;
@@ -72,7 +83,7 @@ struct nib_net {
   bool use_tc;
   bool use_graph;
   const int* dyn_n;           // device-side live batch size for the CUDA-core kernels (fp32 nets), or null
-  long long launches, tc_launches, x3_launches;
+  long long launches, tc_launches;
   // CUDA graphs of the op list, one per batch size: the graph reads the net's own input buffer and writes the net's own
   // logits buffer (staging the caller's input and copying the logits out happen outside it), so caller pointers are not
   // part of the key and the cache is bounded by the number of distinct batch sizes (at most kMaxGraphs, then flushed).
@@ -82,14 +93,24 @@ struct nib_net {
   float* graph_logits;
 };
 
-static size_t elem_size(const nib_net* n) { return n->bf16 ? 2 : 4; }
+// Every device allocation of the net: bytes + 256 B of slack (TMA boxes never read past the tensor-map extent, but SIMT
+// vector loads on the last element may touch up to 16 B beyond it), copied from h or zeroed when h is null.  Recorded
+// before anything else can fail, so nib_net_destroy frees it even when the op or buffer it was for is never added.
+static int upload(nib_net* net, const void* h, size_t bytes, void** d) {
+  NIB_CUDA(cudaMalloc(d, bytes + 256));
+  net->allocs.push_back(*d);
+  if (h) NIB_CUDA(cudaMemcpy(*d, h, bytes, cudaMemcpyHostToDevice));
+  else NIB_CUDA(cudaMemset(*d, 0, bytes + 256));
+  return NIB_OK;
+}
 
-static int upload_floats(const float* h, size_t n, float** d) {
+static int upload_floats(nib_net* net, const float* h, size_t n, float** d) {
   *d = nullptr;
   if (!h || n == 0) return NIB_OK;
-  NIB_CUDA(cudaMalloc(d, n * sizeof(float)));
-  NIB_CUDA(cudaMemcpy(*d, h, n * sizeof(float), cudaMemcpyHostToDevice));
-  return NIB_OK;
+  void* p = nullptr;
+  int rc = upload(net, h, n * sizeof(float), &p);
+  *d = (float*)p;
+  return rc;
 }
 
 static inline uint16_t f32_to_bf16_rn(float f) {
@@ -98,6 +119,33 @@ static inline uint16_t f32_to_bf16_rn(float f) {
   if ((u & 0x7fffffffu) > 0x7f800000u) return (uint16_t)((u >> 16) | 0x40);  // NaN
   u += 0x7fffu + ((u >> 16) & 1u);
   return (uint16_t)(u >> 16);
+}
+
+// w = hi + lo with hi = bf16(w), lo = bf16(w - hi)
+static inline void bf16_hi_lo(float w, uint16_t* hi, uint16_t* lo) {
+  *hi = f32_to_bf16_rn(w);
+  const uint32_t u = (uint32_t)*hi << 16;
+  float hf;
+  memcpy(&hf, &u, 4);
+  *lo = f32_to_bf16_rn(w - hf);
+}
+
+static std::vector<uint16_t> to_bf16(const std::vector<float>& v) {
+  std::vector<uint16_t> out(v.size());
+  for (size_t i = 0; i < v.size(); ++i) out[i] = f32_to_bf16_rn(v[i]);
+  return out;
+}
+
+// [Cout][Cin][R][S] -> [Cout][Rp][Sp][Cp], zero past the filter's R x S x Cin: KRSC (Rp, Sp, Cp = R, S, Cin), KRSC with
+// Cin padded to the K block, and the raw-row layouts of conv_tc.cu
+static std::vector<float> to_krsc(const float* w, const nib_conv_desc& d, int Rp, int Sp, int Cp) {
+  std::vector<float> out((size_t)d.Cout * Rp * Sp * Cp, 0.f);
+  for (int co = 0; co < d.Cout; ++co)
+    for (int c = 0; c < d.Cin; ++c)
+      for (int r = 0; r < d.R; ++r)
+        for (int s = 0; s < d.S; ++s)
+          out[(((size_t)co * Rp + r) * Sp + s) * Cp + c] = w[(((size_t)co * d.Cin + c) * d.R + r) * d.S + s];
+  return out;
 }
 
 extern "C" {
@@ -123,7 +171,7 @@ int nib_net_create(int precision, int max_batch, nib_net** out) {
   n->use_graph = false;
   n->dyn_n = nullptr;
   n->graph_logits = nullptr;
-  n->launches = n->tc_launches = n->x3_launches = 0;
+  n->launches = n->tc_launches = 0;
   *out = n;
   return NIB_OK;
 }
@@ -131,21 +179,8 @@ int nib_net_create(int precision, int max_batch, nib_net** out) {
 int nib_net_destroy(nib_net* net) {
   if (!net) return NIB_OK;
   for (auto& g : net->graphs) cudaGraphExecDestroy(g.second.exec);
-  for (auto& b : net->bufs)
-    if (b.ptr) cudaFree(b.ptr);
-  if (net->pack_scratch) cudaFree(net->pack_scratch);
-  if (net->graph_logits) cudaFree(net->graph_logits);
+  for (void* p : net->allocs) cudaFree(p);
   for (auto& o : net->ops) {
-    if (o.d_w) cudaFree(o.d_w);
-    if (o.d_w_pack) cudaFree(o.d_w_pack);
-    if (o.d_w_alt) cudaFree(o.d_w_alt);
-    if (o.d_w_hi) cudaFree(o.d_w_hi);
-    if (o.d_w_lo) cudaFree(o.d_w_lo);
-    if (o.d_bias) cudaFree(o.d_bias);
-    if (o.d_pre_scale) cudaFree(o.d_pre_scale);
-    if (o.d_pre_scale_pad) cudaFree(o.d_pre_scale_pad);
-    if (o.d_pre_shift_pad) cudaFree(o.d_pre_shift_pad);
-    if (o.d_pre_shift) cudaFree(o.d_pre_shift);
     if (o.plan) tc_conv_plan_destroy(o.plan);
     if (o.fplan) tc_fused_plan_destroy(o.fplan);
   }
@@ -160,11 +195,8 @@ static int add_buffer_kind(nib_net* net, int H, int W, int C, int pad, int kind)
   b.H = H; b.W = W; b.C = C; b.pad = pad;
   b.kind = kind;
   b.elems_per_image = (size_t)(H + 2 * pad) * (W + 2 * pad) * b.phys_c();
-  size_t bytes = b.elems_per_image * net->max_batch * b.esize();
-  // one extra tile row block of slack: TMA boxes never read past the tensor-map extent, but SIMT
-  // vector loads on the last pixel may touch up to 16 B beyond the last channel group.
-  NIB_CUDA(cudaMalloc(&b.ptr, bytes + 256));
-  NIB_CUDA(cudaMemset(b.ptr, 0, bytes + 256));
+  int rc = upload(net, nullptr, b.elems_per_image * net->max_batch * b.esize(), &b.ptr);
+  if (rc != NIB_OK) return rc;
   net->bufs.push_back(b);
   return (int)net->bufs.size() - 1;
 }
@@ -189,9 +221,8 @@ int nib_net_add_convert(nib_net* net, int in_buf, int out_buf) {
   NIB_REQUIRE(bi.H == bo.H && bi.W == bo.W && bi.C == bo.C && bi.pad == 0 && bo.pad == 0, "nib_net_add_convert: geometry mismatch");
   NIB_REQUIRE((bi.kind == BUF_F32 && bo.kind == BUF_SPLIT) || (bi.kind == BUF_SPLIT && bo.kind == BUF_F32),
               "nib_net_add_convert: one side must be fp32, the other split");
-  NetOp op;
-  memset(&op, 0, sizeof(op));
-  op.kind = 3;
+  NetOp op = {};
+  op.kind = OP_CONVERT;
   op.in_buf = in_buf;
   op.out_buf = out_buf;
   net->ops.push_back(op);
@@ -220,132 +251,69 @@ int nib_net_add_conv(nib_net* net, const nib_conv_desc* d, const float* h_weight
   }
   if (d->flags & NIB_CONV_PRE_BNRELU) NIB_REQUIRE(h_pre_scale && h_pre_shift, "nib_net_add_conv: PRE_BNRELU needs scale/shift");
 
-  NetOp op;
-  memset(&op, 0, sizeof(op));
-  op.kind = 0;
+  NetOp op = {};
+  op.kind = OP_CONV;
   op.cd = *d;
   NIB_REQUIRE(bi.kind == bo.kind, "nib_net_add_conv: input and output buffers must have the same kind (use nib_net_add_convert)");
   if (d->res_buf >= 0) NIB_REQUIRE(net->bufs[d->res_buf].kind == bo.kind, "nib_net_add_conv: residual buffer kind mismatch");
-  const bool split_op = bi.kind == BUF_SPLIT;
   const size_t K = (size_t)d->R * d->S * d->Cin;
-  const size_t nel = K * d->Cout;
-  // [Cout][Cin][R][S] -> [Cout][R][S][Cin]
-  std::vector<float> krsc(nel);
-  for (int co = 0; co < d->Cout; ++co)
-    for (int c = 0; c < d->Cin; ++c)
-      for (int r = 0; r < d->R; ++r)
-        for (int s = 0; s < d->S; ++s)
-          krsc[(((size_t)co * d->R + r) * d->S + s) * d->Cin + c] =
-              h_weight[(((size_t)co * d->Cin + c) * d->R + r) * d->S + s];
-  if (split_op) {
+  const std::vector<float> krsc = to_krsc(h_weight, *d, d->R, d->S, d->Cin);
+  const size_t nel = krsc.size();
+  int rc;
+  if (bi.kind == BUF_SPLIT) {
     // [Cout][tap][Wh(Cin) | Wh(Cin) | Wl(Cin)]: against activations walked as hi, lo, hi (conv_tc.cu split mode)
-    const size_t taps = (size_t)d->R * d->S;
     std::vector<uint16_t> hb(nel * 3);
-    for (int co = 0; co < d->Cout; ++co)
-      for (size_t t = 0; t < taps; ++t)
-        for (int c = 0; c < d->Cin; ++c) {
-          const float w = krsc[((size_t)co * taps + t) * d->Cin + c];
-          const uint16_t hi = f32_to_bf16_rn(w);
-          uint32_t u = (uint32_t)hi << 16;
-          float hf;
-          memcpy(&hf, &u, 4);
-          const uint16_t lo = f32_to_bf16_rn(w - hf);
-          const size_t base = ((size_t)co * taps + t) * 3 * d->Cin;
-          hb[base + c] = hi;
-          hb[base + d->Cin + c] = hi;
-          hb[base + 2 * (size_t)d->Cin + c] = lo;
-        }
-    NIB_CUDA(cudaMalloc(&op.d_w, hb.size() * 2 + 256));
-    NIB_CUDA(cudaMemcpy(op.d_w, hb.data(), hb.size() * 2, cudaMemcpyHostToDevice));
+    for (size_t i = 0; i < nel; ++i) {
+      uint16_t hi, lo;
+      bf16_hi_lo(krsc[i], &hi, &lo);
+      const size_t base = i / d->Cin * 3 * d->Cin, c = i % d->Cin;
+      hb[base + c] = hi;
+      hb[base + d->Cin + c] = hi;
+      hb[base + 2 * (size_t)d->Cin + c] = lo;
+    }
+    rc = upload(net, hb.data(), hb.size() * 2, &op.d_w);
   } else if (net->bf16) {
-    std::vector<uint16_t> hb(nel);
-    for (size_t i = 0; i < nel; ++i) hb[i] = f32_to_bf16_rn(krsc[i]);
-    NIB_CUDA(cudaMalloc(&op.d_w, nel * 2 + 256));
-    NIB_CUDA(cudaMemcpy(op.d_w, hb.data(), nel * 2, cudaMemcpyHostToDevice));
+    rc = upload(net, to_bf16(krsc).data(), nel * 2, &op.d_w);
   } else {
-    NIB_CUDA(cudaMalloc(&op.d_w, nel * 4 + 256));
-    NIB_CUDA(cudaMemcpy(op.d_w, krsc.data(), nel * 4, cudaMemcpyHostToDevice));
-    // w = hi + lo with hi = bf16(w), lo = bf16(w - hi).  Not for reductions longer than NIB_X3_MAX_K: the tensor cores'
-    // fp32 accumulation drifts with K (VGG's fc6, K = 25088, measured 1.6e-4 .. 1.9e-4 of the logits' scale against 1e-4
-    // for fp32 grade), so those run on the CUDA cores
-    if (net->x3 && d->Cin % 16 == 0 && K <= NIB_X3_MAX_K) {
+    rc = upload(net, krsc.data(), nel * 4, &op.d_w);
+    // Not for reductions longer than NIB_X3_MAX_K: the tensor cores' fp32 accumulation drifts with K (VGG's fc6,
+    // K = 25088, measured 1.6e-4 .. 1.9e-4 of the logits' scale against 1e-4 for fp32 grade), so those run on the CUDA cores
+    if (rc == NIB_OK && net->x3 && d->Cin % 16 == 0 && K <= NIB_X3_MAX_K) {
       std::vector<uint16_t> hi(nel), lo(nel);
-      for (size_t i = 0; i < nel; ++i) {
-        hi[i] = f32_to_bf16_rn(krsc[i]);
-        uint32_t u = (uint32_t)hi[i] << 16;
-        float hf;
-        memcpy(&hf, &u, 4);
-        lo[i] = f32_to_bf16_rn(krsc[i] - hf);
-      }
-      NIB_CUDA(cudaMalloc(&op.d_w_hi, nel * 2 + 256));
-      NIB_CUDA(cudaMalloc(&op.d_w_lo, nel * 2 + 256));
-      NIB_CUDA(cudaMemcpy(op.d_w_hi, hi.data(), nel * 2, cudaMemcpyHostToDevice));
-      NIB_CUDA(cudaMemcpy(op.d_w_lo, lo.data(), nel * 2, cudaMemcpyHostToDevice));
+      for (size_t i = 0; i < nel; ++i) bf16_hi_lo(krsc[i], &hi[i], &lo[i]);
+      rc = upload(net, hi.data(), nel * 2, &op.d_w_hi);
+      if (rc == NIB_OK) rc = upload(net, lo.data(), nel * 2, &op.d_w_lo);
     }
   }
-  if (net->bf16 && d->R == 7 && d->S == 7 && d->stride == 2 && d->pad == 3 && d->Cin <= 4 && bi.C == 4 && bi.pad == 3) {
-    // 4-channel pixels: K block kb = filter rows (2kb, 2kb+1), each (7 taps + 1 filler) x 4 channels; row 7 is zero
-    std::vector<uint16_t> hb((size_t)d->Cout * 4 * 64, 0);
-    for (int co = 0; co < d->Cout; ++co)
-      for (int r = 0; r < 7; ++r)
-        for (int s = 0; s < 7; ++s)
-          for (int c = 0; c < d->Cin; ++c)
-            hb[((size_t)co * 8 + r) * 32 + s * 4 + c] =
-                f32_to_bf16_rn(h_weight[(((size_t)co * d->Cin + c) * 7 + r) * 7 + s]);
-    NIB_CUDA(cudaMalloc(&op.d_w_alt, hb.size() * 2 + 256));
-    NIB_CUDA(cudaMemcpy(op.d_w_alt, hb.data(), hb.size() * 2, cudaMemcpyHostToDevice));
-  }
-  if (net->bf16 && d->R == 7 && d->S == 7 && d->stride == 2 && d->pad == 3 && d->Cin <= 8 && bi.C == 8 && bi.pad == 3) {
-    std::vector<uint16_t> hb((size_t)d->Cout * 7 * 64, 0);
-    for (int co = 0; co < d->Cout; ++co)
-      for (int r = 0; r < 7; ++r)
-        for (int s = 0; s < 7; ++s)
-          for (int c = 0; c < d->Cin; ++c)
-            hb[(((size_t)co * 7 + r) * 8 + s) * 8 + c] =
-                f32_to_bf16_rn(h_weight[(((size_t)co * d->Cin + c) * 7 + r) * 7 + s]);
-    NIB_CUDA(cudaMalloc(&op.d_w_alt, hb.size() * 2 + 256));
-    NIB_CUDA(cudaMemcpy(op.d_w_alt, hb.data(), hb.size() * 2, cudaMemcpyHostToDevice));
-  }
-  if (net->bf16 && d->R == 3 && d->S == 3 && d->stride == 1 && d->pad == 1 && d->Cin <= 8 && bi.C == 8 && bi.pad == 1) {
-    // 3x3 first conv on raw input rows (conv_tc.cu tc_conv_is_raw3x3): filter row r = one 32-element K atom of
-    // 3 taps x 8 channels + a zero filler tap; row 3 is zero so the weights are two whole 64-element K blocks
-    std::vector<uint16_t> hb((size_t)d->Cout * 4 * 32, 0);
-    for (int co = 0; co < d->Cout; ++co)
-      for (int r = 0; r < 3; ++r)
-        for (int s = 0; s < 3; ++s)
-          for (int c = 0; c < d->Cin; ++c)
-            hb[((size_t)co * 4 + r) * 32 + s * 8 + c] =
-                f32_to_bf16_rn(h_weight[(((size_t)co * d->Cin + c) * 3 + r) * 3 + s]);
-    NIB_CUDA(cudaMalloc(&op.d_w_alt, hb.size() * 2 + 256));
-    NIB_CUDA(cudaMemcpy(op.d_w_alt, hb.data(), hb.size() * 2, cudaMemcpyHostToDevice));
+  if (rc != NIB_OK) return rc;
+  const RawRowLayout raw = tc_raw_row_layout(d->R, d->S, d->stride, d->pad, d->Cin, bi.phys_c(), bi.pad);
+  if (net->bf16 && raw.rows > 0) {
+    rc = upload(net, to_bf16(to_krsc(h_weight, *d, raw.rows, raw.taps, raw.ch)).data(), (size_t)d->Cout * raw.k() * 2,
+                &op.d_w_alt);
+    if (rc != NIB_OK) return rc;
   }
   // BN-ReLU-conv (DenseNet) on the tensor-core path: the conv reads relu(bn(x)) from a packed scratch tensor whose
   // channel count is rounded up to the 64-channel K block, so the weights get the same zero padding along Cin.
   if (net->bf16 && (d->flags & NIB_CONV_PRE_BNRELU) && d->Cin % 8 == 0 && d->in_coff % 8 == 0 && bi.C % 8 == 0 &&
       bi.pad == 0 && d->Cout % 32 == 0) {
     const int cpad = (d->Cin + 63) / 64 * 64;
-    const size_t npad = (size_t)d->Cout * d->R * d->S * cpad;
-    std::vector<uint16_t> hb(npad, 0);
-    for (int co = 0; co < d->Cout; ++co)
-      for (int rs = 0; rs < d->R * d->S; ++rs)
-        for (int c = 0; c < d->Cin; ++c)
-          hb[((size_t)co * d->R * d->S + rs) * cpad + c] = f32_to_bf16_rn(krsc[((size_t)co * d->R * d->S + rs) * d->Cin + c]);
-    NIB_CUDA(cudaMalloc(&op.d_w_pack, npad * 2 + 256));
-    NIB_CUDA(cudaMemcpy(op.d_w_pack, hb.data(), npad * 2, cudaMemcpyHostToDevice));
+    rc = upload(net, to_bf16(to_krsc(h_weight, *d, d->R, d->S, cpad)).data(), (size_t)d->Cout * d->R * d->S * cpad * 2,
+                &op.d_w_pack);
+    if (rc != NIB_OK) return rc;
     op.pack_cin = cpad;
   }
-  int rc = upload_floats(h_bias, d->Cout, &op.d_bias);
+  rc = upload_floats(net, h_bias, d->Cout, &op.d_bias);
   if (rc != NIB_OK) return rc;
   if (d->flags & NIB_CONV_PRE_BNRELU) {
-    rc = upload_floats(h_pre_scale, d->Cin, &op.d_pre_scale);
+    rc = upload_floats(net, h_pre_scale, d->Cin, &op.d_pre_scale);
     if (rc != NIB_OK) return rc;
-    rc = upload_floats(h_pre_shift, d->Cin, &op.d_pre_shift);
+    rc = upload_floats(net, h_pre_shift, d->Cin, &op.d_pre_shift);
     if (rc != NIB_OK) return rc;
     if (op.pack_cin) {
       std::vector<float> sp(op.pack_cin, 0.f), hp(op.pack_cin, 0.f);
       for (int c = 0; c < d->Cin; ++c) { sp[c] = h_pre_scale[c]; hp[c] = h_pre_shift[c]; }
-      if ((rc = upload_floats(sp.data(), sp.size(), &op.d_pre_scale_pad)) != NIB_OK) return rc;
-      if ((rc = upload_floats(hp.data(), hp.size(), &op.d_pre_shift_pad)) != NIB_OK) return rc;
+      if ((rc = upload_floats(net, sp.data(), sp.size(), &op.d_pre_scale_pad)) != NIB_OK) return rc;
+      if ((rc = upload_floats(net, hp.data(), hp.size(), &op.d_pre_shift_pad)) != NIB_OK) return rc;
     }
   }
   net->ops.push_back(op);
@@ -365,14 +333,13 @@ int nib_net_add_pool(nib_net* net, int kind, int in_buf, int in_coff, int C, int
   NIB_REQUIRE(in_coff + C <= bi.C && out_coff + C <= bo.C, "nib_net_add_pool: channel slice out of range");
   const int P = (bi.H + 2 * pad - k) / stride + 1, Q = (bi.W + 2 * pad - k) / stride + 1;
   NIB_REQUIRE(P == bo.H && Q == bo.W, "nib_net_add_pool: output buffer is %dx%d but pool produces %dx%d", bo.H, bo.W, P, Q);
-  NetOp op;
-  memset(&op, 0, sizeof(op));
-  op.kind = 1;
+  NetOp op = {};
+  op.kind = OP_POOL;
   op.pool_kind = kind; op.k = k; op.stride = stride; op.pad = pad; op.C = C;
   op.in_buf = in_buf; op.in_coff = in_coff; op.out_buf = out_buf; op.out_coff = out_coff;
-  int rc = upload_floats(h_pre_scale, C, &op.d_pre_scale);
+  int rc = upload_floats(net, h_pre_scale, C, &op.d_pre_scale);
   if (rc != NIB_OK) return rc;
-  rc = upload_floats(h_pre_shift, C, &op.d_pre_shift);
+  rc = upload_floats(net, h_pre_shift, C, &op.d_pre_shift);
   if (rc != NIB_OK) return rc;
   net->ops.push_back(op);
   return NIB_OK;
@@ -384,30 +351,22 @@ int nib_net_add_fc(nib_net* net, int in_buf, int Cin, int Cout, const float* h_w
   const NetBuffer& bi = net->bufs[in_buf];
   NIB_REQUIRE(bi.H == 1 && bi.W == 1 && bi.C >= Cin, "nib_net_add_fc: input must be a 1x1xC feature buffer");
   NIB_REQUIRE(bi.kind != BUF_SPLIT, "nib_net_add_fc: the feature buffer must be fp32 or bf16");
-  NetOp op;
-  memset(&op, 0, sizeof(op));
-  op.kind = 2;
+  NetOp op = {};
+  op.kind = OP_FC;
   op.fc_in = in_buf; op.fc_cin = Cin; op.fc_cout = Cout;
   float* w = nullptr;
-  int rc = upload_floats(h_weight, (size_t)Cin * Cout, &w);
+  int rc = upload_floats(net, h_weight, (size_t)Cin * Cout, &w);
   if (rc != NIB_OK) return rc;
   op.d_w = w;
-  rc = upload_floats(h_bias, Cout, &op.d_bias);
+  rc = upload_floats(net, h_bias, Cout, &op.d_bias);
   if (rc != NIB_OK) return rc;
   if (bi.kind == BUF_BF16 && fc_x2_supported(Cin, bi.C)) {   // bf16 features: tensor-core fc on W = hi + lo (conv_x3.cu)
     const size_t nel = (size_t)Cin * Cout;
     std::vector<uint16_t> hi(nel), lo(nel);
-    for (size_t i = 0; i < nel; ++i) {
-      hi[i] = f32_to_bf16_rn(h_weight[i]);
-      uint32_t u = (uint32_t)hi[i] << 16;
-      float hf;
-      memcpy(&hf, &u, 4);
-      lo[i] = f32_to_bf16_rn(h_weight[i] - hf);
-    }
-    NIB_CUDA(cudaMalloc(&op.d_w_hi, nel * 2 + 256));
-    NIB_CUDA(cudaMalloc(&op.d_w_lo, nel * 2 + 256));
-    NIB_CUDA(cudaMemcpy(op.d_w_hi, hi.data(), nel * 2, cudaMemcpyHostToDevice));
-    NIB_CUDA(cudaMemcpy(op.d_w_lo, lo.data(), nel * 2, cudaMemcpyHostToDevice));
+    for (size_t i = 0; i < nel; ++i) bf16_hi_lo(h_weight[i], &hi[i], &lo[i]);
+    rc = upload(net, hi.data(), nel * 2, &op.d_w_hi);
+    if (rc == NIB_OK) rc = upload(net, lo.data(), nel * 2, &op.d_w_lo);
+    if (rc != NIB_OK) return rc;
   }
   net->ops.push_back(op);
   net->num_classes = Cout;
@@ -420,7 +379,8 @@ int nib_net_set_input(nib_net* net, int buf) {
   return NIB_OK;
 }
 
-static void fill_conv_params(const nib_net* net, const NetOp& op, int N, ConvParams* p) {
+// The conv's kernel parameters for N images on the given path
+static void fill_conv_params(const nib_net* net, const NetOp& op, ConvPath path, int N, ConvParams* p) {
   const nib_conv_desc& d = op.cd;
   const NetBuffer& bi = net->bufs[d.in_buf];
   const NetBuffer& bo = net->bufs[d.out_buf];
@@ -447,181 +407,176 @@ static void fill_conv_params(const nib_net* net, const NetOp& op, int N, ConvPar
   p->R = d.R; p->S = d.S; p->stride = d.stride; p->pad = d.pad;
   p->relu = (d.flags & NIB_CONV_RELU) ? 1 : 0;
   p->dyn_n = net->dyn_n;
+  if (path == PATH_TC_XFORM) {
+    // the raw channel slice: padded channel count, padded weights, padded scale / shift (channels past Cin come out as
+    // exact zeros)
+    p->w = op.d_w_pack;
+    p->pre_scale = op.d_pre_scale_pad;
+    p->pre_shift = op.d_pre_shift_pad;
+    p->pre_padded = 1;
+    p->Cin = op.pack_cin;
+  } else if (path == PATH_TC_PACK) {
+    // the packed relu(bn(x)) scratch tensor instead of the raw channel slice
+    p->in = net->pack_scratch;
+    p->w = op.d_w_pack;
+    p->pre_scale = nullptr;
+    p->pre_shift = nullptr;
+    p->Cin = op.pack_cin;
+    p->in_cstride = op.pack_cin;
+    p->in_coff = 0;
+  }
 }
 
-// the same conv on the raw channel slice, BN-ReLU applied to the A tiles inside the pair kernel: padded channel count,
-// padded weights, padded scale / shift (channels past Cin come out as exact zeros)
-static void fill_xform_conv_params(const nib_net* net, const NetOp& op, int N, ConvParams* p) {
-  fill_conv_params(net, op, N, p);
-  p->w = op.d_w_pack;
-  p->pre_scale = op.d_pre_scale_pad;
-  p->pre_shift = op.d_pre_shift_pad;
-  p->pre_padded = 1;
-  p->Cin = op.pack_cin;
-}
-
-// the same conv, reading the packed relu(bn(x)) scratch tensor instead of the raw channel slice
-static void fill_packed_conv_params(const nib_net* net, const NetOp& op, int N, ConvParams* p) {
-  fill_conv_params(net, op, N, p);
-  p->in = net->pack_scratch;
-  p->w = op.d_w_pack;
-  p->pre_scale = nullptr;
-  p->pre_shift = nullptr;
-  p->Cin = op.pack_cin;
-  p->in_cstride = op.pack_cin;
-  p->in_coff = 0;
+// The conv's paths, in order of preference.  Only tc_conv_supported is consulted: the plans are built afterwards.
+static int resolve_paths(const nib_net* net, NetOp& op) {
+  static const bool no_xform = getenv("NIB_TC_NO_XFORM") != nullptr;   // A/B: the separate pack pass
+  ConvParams p, pt;
+  fill_conv_params(net, op, PATH_TC, net->max_batch, &p);
+  op.cuda_path = net->x3 && op.d_w_hi && conv_x3_supported(p) ? PATH_X3 : PATH_SIMT;
+  op.path = op.cuda_path;
+  if (p.split) {
+    NIB_REQUIRE(tc_conv_supported(p), "nib_net_finalize: a conv on split tensors needs Cin %% 64 == 0, Cout %% 64 == 0, whole-buffer channel ranges (Cin=%d Cout=%d)", p.Cin, p.Cout);
+    op.path = PATH_TC;
+  } else if (net->bf16 && op.pack_cin) {
+    fill_conv_params(net, op, PATH_TC_XFORM, net->max_batch, &pt);
+    if (!no_xform && tc_conv_supported(pt)) {
+      op.path = PATH_TC_XFORM;
+    } else {
+      fill_conv_params(net, op, PATH_TC_PACK, net->max_batch, &pt);
+      if (tc_conv_supported(pt)) op.path = PATH_TC_PACK;
+    }
+  } else if (net->bf16 && tc_conv_supported(p)) {
+    op.path = PATH_TC;
+  }
+  return NIB_OK;
 }
 
 int nib_net_finalize(nib_net* net) {
   NIB_REQUIRE(net && !net->finalized, "nib_net_finalize: bad handle/state");
   NIB_REQUIRE(net->input_buf >= 0, "nib_net_finalize: input buffer not set");
-  NIB_REQUIRE(!net->ops.empty() && net->ops.back().kind == 2, "nib_net_finalize: the last op must be the fc layer");
-  if (net->split) {
-    for (auto& op : net->ops) {
-      if (op.kind != 0 || net->bufs[op.cd.in_buf].kind != BUF_SPLIT) continue;
-      ConvParams p;
-      fill_conv_params(net, op, net->max_batch, &p);
-      NIB_REQUIRE(tc_conv_supported(p), "nib_net_finalize: a conv on split tensors needs Cin %% 64 == 0, Cout %% 64 == 0, whole-buffer channel ranges (Cin=%d Cout=%d)", p.Cin, p.Cout);
-      int rc = tc_conv_plan_create(p, net->max_batch, &op.plan);
-      if (rc != NIB_OK) return rc;
-    }
-  }
-  if (net->bf16) {
-    // one scratch tensor serves every packed pre-activation conv (ops run one at a time on the stream)
-    static const bool no_xform = getenv("NIB_TC_NO_XFORM") != nullptr;   // A/B: the separate pack pass
-    for (auto& op : net->ops) {
-      if (op.kind != 0 || op.pack_cin == 0) continue;
-      if (!no_xform && op.d_pre_scale_pad) {
-        ConvParams px;
-        fill_xform_conv_params(net, op, net->max_batch, &px);
-        if (tc_conv_supported(px)) { op.xform = 1; continue; }
-      }
+  NIB_REQUIRE(!net->ops.empty() && net->ops.back().kind == OP_FC, "nib_net_finalize: the last op must be the fc layer");
+  int rc;
+  for (auto& op : net->ops) {
+    if (op.kind != OP_CONV) continue;
+    if ((rc = resolve_paths(net, op)) != NIB_OK) return rc;
+    if (op.path == PATH_TC_PACK) {
       const NetBuffer& bi = net->bufs[op.cd.in_buf];
       const size_t need = (size_t)net->max_batch * bi.H * bi.W * op.pack_cin * 2;
       if (need > net->pack_scratch_bytes) net->pack_scratch_bytes = need;
     }
-    if (net->pack_scratch_bytes) NIB_CUDA(cudaMalloc(&net->pack_scratch, net->pack_scratch_bytes + 256));
-    for (auto& op : net->ops) {
-      if (op.kind != 0) continue;
-      ConvParams p;
-      if (op.xform) {
-        fill_xform_conv_params(net, op, net->max_batch, &p);
-        int rc = tc_conv_plan_create(p, net->max_batch, &op.plan);
-        if (rc != NIB_OK) return rc;
-        continue;
-      }
-      if (op.pack_cin) {
-        fill_packed_conv_params(net, op, net->max_batch, &p);
-        if (tc_conv_supported(p)) {
-          int rc = tc_conv_plan_create(p, net->max_batch, &op.plan);
-          if (rc != NIB_OK) return rc;
-        } else {
-          op.pack_cin = 0;
-        }
-        continue;
-      }
-      fill_conv_params(net, op, net->max_batch, &p);
-      if (tc_conv_supported(p)) {
-        int rc = tc_conv_plan_create(p, net->max_batch, &op.plan);
-        if (rc != NIB_OK) {
-          if (op.d_w_alt == nullptr) return rc;
-          op.plan = nullptr;   // the stem's overlapping-window map is optional: the CUDA-core kernel covers it
-        }
-      }
+  }
+  // one scratch tensor serves every packed pre-activation conv (ops run one at a time on the stream); the plans of those
+  // convs read it, so it exists before they are built
+  if (net->pack_scratch_bytes && (rc = upload(net, nullptr, net->pack_scratch_bytes, &net->pack_scratch)) != NIB_OK) return rc;
+  for (auto& op : net->ops) {
+    if (op.kind != OP_CONV || !on_tcgen05(op.path)) continue;
+    ConvParams p;
+    fill_conv_params(net, op, op.path, net->max_batch, &p);
+    rc = tc_conv_plan_create(p, net->max_batch, &op.plan);
+    if (rc != NIB_OK) {
+      if (op.path != PATH_TC || op.d_w_alt == nullptr) return rc;
+      op.path = op.cuda_path;   // the raw-row modes are optional: the CUDA-core kernel covers the conv
     }
   }
-  if (net->bf16) {
-    for (size_t i = 0; i + 1 < net->ops.size(); ++i) {
-      NetOp& c = net->ops[i];
-      NetOp& a = net->ops[i + 1];
-      if (c.kind != 0 || a.kind != 0 || !c.plan || !a.plan || c.pack_cin || a.pack_cin || c.fused_skip) continue;
-      ConvParams pc, pa;
-      fill_conv_params(net, c, net->max_batch, &pc);
-      fill_conv_params(net, a, net->max_batch, &pa);
-      if (!tc_fuse_supported(pc, pa)) continue;
-      int rc = tc_fused_plan_create(pc, pa, net->max_batch, &c.fplan);
-      if (rc != NIB_OK) return rc;
-      c.next_cd = a.cd;
-      c.next_w = a.d_w;
-      c.next_bias = a.d_bias;
-      a.fused_skip = true;
-    }
+  for (size_t i = 0; i + 1 < net->ops.size(); ++i) {
+    NetOp& c = net->ops[i];
+    NetOp& a = net->ops[i + 1];
+    if (c.kind != OP_CONV || a.kind != OP_CONV || c.path != PATH_TC || a.path != PATH_TC) continue;
+    ConvParams pc, pa;
+    fill_conv_params(net, c, PATH_TC, net->max_batch, &pc);
+    fill_conv_params(net, a, PATH_TC, net->max_batch, &pa);
+    if (!tc_fuse_supported(pc, pa)) continue;
+    if ((rc = tc_fused_plan_create(pc, pa, net->max_batch, &c.fplan)) != NIB_OK) return rc;
+    c.path = PATH_FUSED_HEAD;
+    a.path = PATH_FUSED_TAIL;
   }
   net->finalized = true;
   return NIB_OK;
 }
 
-static int run_ops(nib_net* net, int N, float* d_logits, cudaStream_t st) {
-  for (auto& op : net->ops) {
-    if (op.kind == 0) {
-      if (op.fused_skip && net->use_tc) continue;     // computed by the previous op's fused launch
-      ConvParams p;
-      fill_conv_params(net, op, N, &p);
-      int rc;
-      if (op.fplan && net->use_tc) {
-        NetOp nx = op;                                // the fused partner's geometry, weights and bias
-        nx.cd = op.next_cd;
-        nx.d_w = op.next_w;
-        nx.d_bias = op.next_bias;
-        ConvParams pa;
-        fill_conv_params(net, nx, N, &pa);
-        rc = tc_fused_launch(op.fplan, p, pa, st);
-        net->tc_launches++;
-      } else if (op.plan && net->use_tc && op.xform) {
-        fill_xform_conv_params(net, op, N, &p);
-        rc = tc_conv_launch(op.plan, p, st);
-        net->tc_launches++;
-      } else if (op.plan && net->use_tc && op.pack_cin) {
-        const NetBuffer& bi = net->bufs[op.cd.in_buf];
-        rc = launch_bnrelu_pack(bi.ptr, bi.C, op.cd.in_coff, op.cd.Cin, op.pack_cin, op.d_pre_scale, op.d_pre_shift,
-                                net->pack_scratch, (long long)N * bi.H * bi.W, st);
-        net->launches++;
-        if (rc != NIB_OK) return rc;
-        fill_packed_conv_params(net, op, N, &p);
-        rc = tc_conv_launch(op.plan, p, st);
-        net->tc_launches++;
-      } else if (op.plan && (net->use_tc || net->split)) {
-        rc = tc_conv_launch(op.plan, p, st);
-        net->tc_launches++;
-      } else if (net->x3 && op.d_w_hi && conv_x3_supported(p)) {
-        rc = launch_conv_x3(p, op.d_w_hi, op.d_w_lo, st);
-        net->x3_launches++;
-      } else {
-        rc = launch_conv_simt(p, net->bf16, st);
-      }
-      net->launches++;
-      if (rc != NIB_OK) return rc;
-    } else if (op.kind == 3) {
-      const NetBuffer& bi = net->bufs[op.in_buf];
-      const NetBuffer& bo = net->bufs[op.out_buf];
-      int rc = launch_split_convert(bi.ptr, bo.ptr, (long long)N * bi.H * bi.W, bi.C, bi.kind == BUF_F32, net->dyn_n, bi.H * bi.W, st);
-      net->launches++;
-      if (rc != NIB_OK) return rc;
-    } else if (op.kind == 1) {
-      const NetBuffer& bi = net->bufs[op.in_buf];
-      const NetBuffer& bo = net->bufs[op.out_buf];
-      PoolParams p;
-      memset(&p, 0, sizeof(p));
-      p.in = bi.ptr; p.out = bo.ptr;
-      p.pre_scale = op.d_pre_scale; p.pre_shift = op.d_pre_shift;
-      p.kind = op.pool_kind; p.N = N; p.Hin = bi.H; p.Win = bi.W; p.C = op.C;
-      p.in_cstride = bi.C; p.in_coff = op.in_coff;
-      p.P = bo.H; p.Q = bo.W; p.out_cstride = bo.C; p.out_coff = op.out_coff;
-      p.k = op.k; p.stride = op.stride; p.pad = op.pad;
-      p.dyn_n = net->dyn_n;
-      int rc = launch_pool(p, bi.kind == BUF_BF16, st);
-      net->launches++;
-      if (rc != NIB_OK) return rc;
-    } else {
-      const NetBuffer& bi = net->bufs[op.fc_in];
-      static const bool fc_simt = getenv("NIB_FC_SIMT") != nullptr;   // A/B: the CUDA-core SGEMM
-      int rc = (op.d_w_hi && !fc_simt)
-                   ? launch_fc_x2(bi.ptr, bi.C, op.d_w_hi, op.d_w_lo, op.d_bias, N, op.fc_cin, op.fc_cout, d_logits, net->dyn_n, st)
-                   : launch_fc(bi.ptr, bi.C, bi.kind == BUF_BF16, (const float*)op.d_w, op.d_bias, N, op.fc_cin, op.fc_cout,
-                               d_logits, net->dyn_n, st);
-      net->launches++;
-      if (rc != NIB_OK) return rc;
+static int run_conv(nib_net* net, size_t i, int N, cudaStream_t st) {
+  const NetOp& op = net->ops[i];
+  const ConvPath path = net->use_tc ? op.path : op.cuda_path;
+  if (path == PATH_FUSED_TAIL) return NIB_OK;
+  ConvParams p;
+  fill_conv_params(net, op, path, N, &p);
+  int rc = NIB_OK;
+  switch (path) {
+    case PATH_FUSED_HEAD: {
+      ConvParams pa;
+      fill_conv_params(net, net->ops[i + 1], PATH_FUSED_TAIL, N, &pa);
+      rc = tc_fused_launch(op.fplan, p, pa, st);
+      break;
     }
+    case PATH_TC_PACK: {
+      const NetBuffer& bi = net->bufs[op.cd.in_buf];
+      rc = launch_bnrelu_pack(bi.ptr, bi.C, op.cd.in_coff, op.cd.Cin, op.pack_cin, op.d_pre_scale, op.d_pre_shift,
+                              net->pack_scratch, (long long)N * bi.H * bi.W, st);
+      net->launches++;
+      if (rc != NIB_OK) return rc;
+      rc = tc_conv_launch(op.plan, p, st);
+      break;
+    }
+    case PATH_TC:
+    case PATH_TC_XFORM:
+      rc = tc_conv_launch(op.plan, p, st);
+      break;
+    case PATH_X3:
+      rc = launch_conv_x3(p, op.d_w_hi, op.d_w_lo, st);
+      break;
+    default:
+      rc = launch_conv_simt(p, net->bf16, st);
+      break;
+  }
+  if (on_tcgen05(path)) net->tc_launches++;
+  net->launches++;
+  return rc;
+}
+
+// ops [begin, end) on N images
+static int run_ops(nib_net* net, size_t begin, size_t end, int N, float* d_logits, cudaStream_t st) {
+  for (size_t i = begin; i < end; ++i) {
+    const NetOp& op = net->ops[i];
+    int rc = NIB_OK;
+    switch (op.kind) {
+      case OP_CONV:
+        rc = run_conv(net, i, N, st);
+        break;
+      case OP_CONVERT: {
+        const NetBuffer& bi = net->bufs[op.in_buf];
+        const NetBuffer& bo = net->bufs[op.out_buf];
+        rc = launch_split_convert(bi.ptr, bo.ptr, (long long)N * bi.H * bi.W, bi.C, bi.kind == BUF_F32, net->dyn_n, bi.H * bi.W, st);
+        net->launches++;
+        break;
+      }
+      case OP_POOL: {
+        const NetBuffer& bi = net->bufs[op.in_buf];
+        const NetBuffer& bo = net->bufs[op.out_buf];
+        PoolParams p;
+        memset(&p, 0, sizeof(p));
+        p.in = bi.ptr; p.out = bo.ptr;
+        p.pre_scale = op.d_pre_scale; p.pre_shift = op.d_pre_shift;
+        p.kind = op.pool_kind; p.N = N; p.Hin = bi.H; p.Win = bi.W; p.C = op.C;
+        p.in_cstride = bi.C; p.in_coff = op.in_coff;
+        p.P = bo.H; p.Q = bo.W; p.out_cstride = bo.C; p.out_coff = op.out_coff;
+        p.k = op.k; p.stride = op.stride; p.pad = op.pad;
+        p.dyn_n = net->dyn_n;
+        rc = launch_pool(p, bi.kind == BUF_BF16, st);
+        net->launches++;
+        break;
+      }
+      case OP_FC: {
+        const NetBuffer& bi = net->bufs[op.fc_in];
+        static const bool fc_simt = getenv("NIB_FC_SIMT") != nullptr;   // A/B: the CUDA-core SGEMM
+        rc = (op.d_w_hi && !fc_simt)
+                 ? launch_fc_x2(bi.ptr, bi.C, op.d_w_hi, op.d_w_lo, op.d_bias, N, op.fc_cin, op.fc_cout, d_logits, net->dyn_n, st)
+                 : launch_fc(bi.ptr, bi.C, bi.kind == BUF_BF16, (const float*)op.d_w, op.d_bias, N, op.fc_cin, op.fc_cout,
+                             d_logits, net->dyn_n, st);
+        net->launches++;
+        break;
+      }
+    }
+    if (rc != NIB_OK) return rc;
   }
   return NIB_OK;
 }
@@ -635,13 +590,13 @@ static int stage_input(nib_net* net, const void* d_x, int x_layout, int N, cudaS
     int C = bi.C;
     // real channel count = Cin of the first conv reading this buffer
     for (auto& op : net->ops)
-      if (op.kind == 0 && op.cd.in_buf == net->input_buf) { C = op.cd.Cin; break; }
+      if (op.kind == OP_CONV && op.cd.in_buf == net->input_buf) { C = op.cd.Cin; break; }
     int rc = launch_nchw_to_nhwc((const float*)d_x, N, C, bi.H, bi.W, bi.ptr, bi.C, bi.pad, net->bf16, st);
     net->launches++;
     return rc;
   }
   if (d_x != bi.ptr)
-    NIB_CUDA(cudaMemcpyAsync(bi.ptr, d_x, bi.elems_per_image * N * elem_size(net), cudaMemcpyDeviceToDevice, st));
+    NIB_CUDA(cudaMemcpyAsync(bi.ptr, d_x, bi.elems_per_image * N * bi.esize(), cudaMemcpyDeviceToDevice, st));
   return NIB_OK;
 }
 
@@ -655,12 +610,16 @@ int nib_net_forward(nib_net* net, const void* d_x, int x_layout, int N, float* d
   if (!net->use_graph) {
     int rc = stage_input(net, d_x, x_layout, N, st);
     if (rc != NIB_OK) return rc;
-    return run_ops(net, N, d_logits, st);
+    return run_ops(net, 0, net->ops.size(), N, d_logits, st);
   }
   int rc = stage_input(net, d_x, x_layout, N, st);
   if (rc != NIB_OK) return rc;
-  if (!net->graph_logits)
-    NIB_CUDA(cudaMalloc(&net->graph_logits, sizeof(float) * (size_t)net->max_batch * (net->num_classes > 0 ? net->num_classes : 1)));
+  if (!net->graph_logits) {
+    void* p = nullptr;
+    rc = upload(net, nullptr, sizeof(float) * (size_t)net->max_batch * (net->num_classes > 0 ? net->num_classes : 1), &p);
+    if (rc != NIB_OK) return rc;
+    net->graph_logits = (float*)p;
+  }
   auto it = net->graphs.find(N);
   if (it == net->graphs.end()) {
     if (net->graphs.size() >= nib_net::kMaxGraphs) {
@@ -671,7 +630,7 @@ int nib_net_forward(nib_net* net, const void* d_x, int x_layout, int N, float* d
     NIB_CUDA(cudaStreamCreateWithFlags(&cap, cudaStreamNonBlocking));
     const long long l0 = net->launches, t0 = net->tc_launches;
     NIB_CUDA(cudaStreamBeginCapture(cap, cudaStreamCaptureModeThreadLocal));
-    rc = run_ops(net, N, net->graph_logits, cap);
+    rc = run_ops(net, 0, net->ops.size(), N, net->graph_logits, cap);
     cudaGraph_t graph = nullptr;
     cudaError_t ce = cudaStreamEndCapture(cap, &graph);
     if (rc != NIB_OK || ce != cudaSuccess) {
@@ -709,39 +668,35 @@ int nib_net_profile(nib_net* net, int N, float* h_ms, int* h_kind, double* h_flo
   for (auto& e : ev) NIB_CUDA(cudaEventCreate(&e));
   float* d_logits = nullptr;
   NIB_CUDA(cudaMalloc(&d_logits, sizeof(float) * (size_t)N * (net->num_classes > 0 ? net->num_classes : 1)));
-  // run op by op, reusing run_ops on single-op slices
-  std::vector<NetOp> all;
-  all.swap(net->ops);
   int rc = NIB_OK;
   for (int i = 0; i < nops && rc == NIB_OK; ++i) {
     cudaEventRecord(ev[i], st);
-    net->ops.assign(1, all[i]);
-    rc = run_ops(net, N, d_logits, st);
+    rc = run_ops(net, i, i + 1, N, d_logits, st);
   }
   cudaEventRecord(ev[nops], st);
-  net->ops.swap(all);
   cudaError_t ce = cudaStreamSynchronize(st);
   if (rc == NIB_OK && ce != cudaSuccess) { set_error("nib_net_profile: %s", cudaGetErrorString(ce)); rc = NIB_ECUDA; }
   for (int i = 0; i < nops && rc == NIB_OK; ++i) {
     cudaEventElapsedTime(&h_ms[i], ev[i], ev[i + 1]);
     const NetOp& op = net->ops[i];
-    if (op.kind == 0) {
+    if (op.kind == OP_CONV) {
       const NetBuffer& bo = net->bufs[op.cd.out_buf];
+      const ConvPath path = net->use_tc ? op.path : op.cuda_path;
       // 4: a tcgen05 conv computed by the PREVIOUS op's fused launch (its own slot only holds event overhead)
-      h_kind[i] = (op.fused_skip && net->use_tc) ? 4 : (op.plan && net->use_tc) ? 1 : 0;
+      h_kind[i] = path == PATH_FUSED_TAIL ? 4 : on_tcgen05(path) ? 1 : 0;
       h_flops[i] = 2.0 * N * bo.H * bo.W * (double)op.cd.R * op.cd.S * op.cd.Cin * op.cd.Cout;
       if (h_geom) {
         int* g = h_geom + 8 * i;
         g[0] = bo.H; g[1] = bo.W; g[2] = op.cd.Cin; g[3] = op.cd.Cout; g[4] = op.cd.R; g[5] = op.cd.stride;
         g[6] = op.cd.res_buf >= 0; g[7] = op.plan ? tc_conv_plan_block_n(op.plan) : 0;
       }
-    } else if (op.kind == 1 || op.kind == 3) {
+    } else if (op.kind == OP_POOL || op.kind == OP_CONVERT) {
       h_kind[i] = 2;
       h_flops[i] = 0.0;
       if (h_geom) {
         const NetBuffer& bo = net->bufs[op.out_buf];
         int* g = h_geom + 8 * i;
-        g[0] = bo.H; g[1] = bo.W; g[2] = bo.C; g[3] = bo.C; g[4] = op.kind == 1 ? op.k : 0; g[5] = op.kind == 1 ? op.stride : 1; g[6] = 0; g[7] = 0;
+        g[0] = bo.H; g[1] = bo.W; g[2] = bo.C; g[3] = bo.C; g[4] = op.kind == OP_POOL ? op.k : 0; g[5] = op.kind == OP_POOL ? op.stride : 1; g[6] = 0; g[7] = 0;
       }
     } else {
       h_kind[i] = 3;

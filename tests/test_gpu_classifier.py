@@ -103,7 +103,7 @@ CONV_CASES = [
     (256, 512, 1, 2, 0, 28, 28, False, False),
     (128, 32, 3, 1, 1, 7, 7, False, False),
     (512, 512, 3, 1, 1, 7, 7, True, True),
-    # 3x3 64 -> 64 on the resident input patch (conv_tc.cu im2col mode 4): 2 / 4 / 8 image rows per tile; N = 5 images
+    # 3x3 64 -> 64 on the resident input patch (conv_tc.cu TC_A_HALO): 2 / 4 / 8 image rows per tile; N = 5 images
     # makes the tile count odd, so one CTA of the last pair runs past the batch
     (64, 64, 3, 1, 1, 56, 56, True, False),
     (64, 64, 3, 1, 1, 32, 30, False, False),

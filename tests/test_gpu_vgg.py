@@ -1,6 +1,6 @@
 """GPU: torchvision VGG and AlexNet on the engine.
 
-The 3x3 first conv on raw input rows (conv_tc.cu tc_conv_is_raw3x3, im2col mode 5 over 16-byte pixels), Linear layers
+The 3x3 first conv on raw input rows (conv_tc.cu tc_conv_is_raw3x3, TC_A_RAW over 16-byte pixels), Linear layers
 lowered as convolutions (the first as a valid KxK conv over the final map, the middle ones as 1x1 convs on 1x1 maps),
 whole networks in all four precisions against the torch fp32 CPU forward (oracle.classifier.forward_logits), the bench
 configuration with the tie policy on, and the ImageNet drop-in with `-a vgg16`.  Tolerances as tests/test_gpu_classifier.py:
